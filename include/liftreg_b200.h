@@ -305,6 +305,35 @@ LR_API int lr_diffusion_reg_sum(const float *disp, int B, int D, int H, int W, i
 LR_API int lr_diffusion_reg_backward(const float *disp, int B, int D, int H, int W, int boundary, const float *grad_loss,
                                      float *grad_disp, lr_stream_t stream);
 
+/* ---- validation metrics (RegistrationNet.py:198-218 _compute_metrics) --------------------------------------------
+ * PARITY UNPINNED: the reference's utils/utils.py and utils/metrics.py import mermaid and SimpleITK and are not part of
+ * the reference tree, so which determinant, boundary crop, background rule and empty-label score they use is unknown.
+ * These entries are defined from first principles, are not signature-compatible replacements, and no golden pins them.
+ *
+ * lr_jacobian_det replaces the host-side folding statistic of utils/utils.py:20-55 (numpy Jacobian determinant of phi
+ * with mermaid's finite differences, each item's 3*D*H*W map copied to the host).
+ *   phi (B,3,D,H,W) float32 in [-1,1], channel c addressing volume axis c (lr_warp_forward's convention); D,H,W >= 2.
+ *   J[c][a] = central difference of phi_c along axis a * 0.5/(2/(n_a-1)), with the face rule `boundary` of
+ *   lr_diffusion_reg_sum (LR_FD_LINEAR / LR_FD_NEUMANN_ZERO); the identity map has J = I.
+ *   det = J00*(J11*J22 - J12*J21) - J01*(J10*J22 - J12*J20) + J02*(J10*J21 - J11*J20), each product and difference
+ *   rounded to fp32 on its own, left to right.
+ *   det (B,D,H,W) nullable: the determinant map.
+ *   stats (B,7) float64, zeroed / initialised by the call, over the voxels at least `margin` (2*margin < every axis)
+ *   from every face: [#det<0, sum |det| over det<0, min det, max det, sum det, sum det^2, #non-finite det]; sums
+ *   accumulate in fp64, counts are exact, and min / max / the sums cover finite values only (min = +inf, max = -inf
+ *   when there is none).  B*3*D*H*W must stay below 2^31.
+ *
+ * lr_label_confusion replaces the Python-set overlap scoring of utils/metrics.py:6-121 (get_multi_metric / cal_metric):
+ * every per-label Dice, IoU, recall and precision follows from the L x L confusion matrix of (predicted, target) labels.
+ *   pred, target (B,N) float32 label maps (what the nearest-mode warp returns); 1 <= L <= 128.
+ *   counts (B,L,L) int64: counts[b][p][t] = #voxels with pred == p and target == t (exact).
+ *   invalid (B) int64: #voxels where either value is not an integer in [0, L) (negative, >= L, fractional, NaN).
+ *   Both outputs are zeroed by the call. */
+LR_API int lr_jacobian_det(const float *phi, int B, int D, int H, int W, int boundary, int margin,
+                           float *det, double *stats, lr_stream_t stream);
+LR_API int lr_label_confusion(const float *pred, const float *target, int B, int64_t N, int L,
+                              int64_t *counts, int64_t *invalid, lr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

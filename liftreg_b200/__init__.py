@@ -7,5 +7,6 @@ Host-side mirror of the reference's operator interface over a C-ABI CUDA library
     liftreg_b200.ops                     functional autograd ops over include/liftreg_b200.h
     liftreg_b200.dropin                  makes an installed reference use the above
     liftreg_b200.sharding                multi-GPU partitioning (view-sharded DRR, slab-sharded backprojection/warp)
+    liftreg_b200.metrics                 validation metrics on the GPU (Jacobian folding, per-label overlap; parity unpinned)
 """
 __version__ = "0.1.0"

@@ -63,6 +63,8 @@ SIGNATURES = {
     "lr_ncc_backward": (_i, [_vp, _vp, _i, _i64, _vp, _vp, _vp, _vp]),
     "lr_diffusion_reg_sum": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp]),
     "lr_diffusion_reg_backward": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "lr_jacobian_det": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "lr_label_confusion": (_i, [_vp, _vp, _i, _i64, _i, _vp, _vp, _vp]),
 }
 
 _lib = None

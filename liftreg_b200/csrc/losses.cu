@@ -504,6 +504,282 @@ static bool reg_use_pairs(const void *a, const void *b, int W) {
     return enabled && (W % 2 == 0) && ((uintptr_t)a % 8 == 0) && ((uintptr_t)b % 8 == 0);
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Validation metrics (the host-side scoring of RegistrationNet.py:198-218).  PARITY UNPINNED: the reference's
+// utils.py:20-55 (Jacobian folding) and metrics.py:6-121 (label overlap) import mermaid and SimpleITK and are not part of
+// this tree; the definitions here are stated from first principles (include/liftreg_b200.h).
+//
+// Jacobian determinant of a map phi (B,3,D,H,W) in [-1,1], channel c addressing volume axis c: J[c][a] is the
+// regulariser's central difference of channel c along axis a, same face rules and scales (0.5/(2/(n-1)), so the identity
+// has J = I whatever the per-axis normalisation), and the 3x3 determinant is expanded along the first row with every
+// product and difference rounded on its own, left to right, so an fp32 torch restatement reproduces it bit for bit.
+constexpr int JAC_STATS = 7;     // per item: #det<0, sum |det| over det<0, min, max, sum det, sum det^2, #non-finite
+
+__device__ __forceinline__ float det3(const float (&j)[3][3]) {
+    const float a = mul_rn(j[0][0], sub_rn(mul_rn(j[1][1], j[2][2]), mul_rn(j[1][2], j[2][1])));
+    const float b = mul_rn(j[0][1], sub_rn(mul_rn(j[1][0], j[2][2]), mul_rn(j[1][2], j[2][0])));
+    const float c = mul_rn(j[0][2], sub_rn(mul_rn(j[1][0], j[2][1]), mul_rn(j[1][1], j[2][0])));
+    return add_rn(sub_rn(a, b), c);
+}
+
+// per-thread statistics; sums in fp64 (the det is fp32, so det^2 is exact in fp64), counts in integers
+struct JacAcc {
+    unsigned neg = 0, nonfinite = 0;
+    double neg_abs = 0.0, sum = 0.0, sum2 = 0.0;
+    float mn = INFINITY, mx = -INFINITY;
+    __device__ __forceinline__ void add(float v, bool in) {
+        if (!in) return;
+        if (!isfinite(v)) { ++nonfinite; return; }
+        const double d = (double)v;
+        sum += d;
+        sum2 = fma(d, d, sum2);
+        if (v < 0.0f) { ++neg; neg_abs -= d; }
+        mn = fminf(mn, v); mx = fmaxf(mx, v);
+    }
+};
+
+__device__ __forceinline__ void atomic_min_f64(double *p, double v) {
+    unsigned long long *a = reinterpret_cast<unsigned long long *>(p), old = *a;
+    while (v < __longlong_as_double((long long)old)) {
+        const unsigned long long seen = atomicCAS(a, old, (unsigned long long)__double_as_longlong(v));
+        if (seen == old) break;
+        old = seen;
+    }
+}
+__device__ __forceinline__ void atomic_max_f64(double *p, double v) {
+    unsigned long long *a = reinterpret_cast<unsigned long long *>(p), old = *a;
+    while (v > __longlong_as_double((long long)old)) {
+        const unsigned long long seen = atomicCAS(a, old, (unsigned long long)__double_as_longlong(v));
+        if (seen == old) break;
+        old = seen;
+    }
+}
+
+// block reduction of the per-thread statistics, then one atomic per statistic and block (skipped when it cannot change
+// the result: most blocks have no folds and no non-finite values)
+__device__ __forceinline__ void jac_block_flush(const JacAcc &t, double *__restrict__ st) {
+    __shared__ double sd[NCC_THREADS / 32][3];
+    __shared__ float sf[NCC_THREADS / 32][2];
+    __shared__ unsigned su[NCC_THREADS / 32][2];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const double a = warp_sum(t.neg_abs), s = warp_sum(t.sum), s2 = warp_sum(t.sum2);
+    const unsigned n = __reduce_add_sync(0xffffffffu, t.neg), nf = __reduce_add_sync(0xffffffffu, t.nonfinite);
+    float mn = t.mn, mx = t.mx;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+        mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    }
+    if (lane == 0) {
+        sd[warp][0] = a; sd[warp][1] = s; sd[warp][2] = s2;
+        sf[warp][0] = mn; sf[warp][1] = mx;
+        su[warp][0] = n; su[warp][1] = nf;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double ta = 0.0, ts = 0.0, ts2 = 0.0;
+        unsigned tn = 0, tnf = 0;
+        float tmn = INFINITY, tmx = -INFINITY;
+#pragma unroll
+        for (int w = 0; w < NCC_THREADS / 32; ++w) {
+            ta += sd[w][0]; ts += sd[w][1]; ts2 += sd[w][2];
+            tn += su[w][0]; tnf += su[w][1];
+            tmn = fminf(tmn, sf[w][0]); tmx = fmaxf(tmx, sf[w][1]);
+        }
+        if (tn) { atomicAdd(st + 0, (double)tn); atomicAdd(st + 1, ta); }
+        if (tmn <= tmx) { atomic_min_f64(st + 2, (double)tmn); atomic_max_f64(st + 3, (double)tmx); }
+        if (ts != 0.0) atomicAdd(st + 4, ts);
+        if (ts2 != 0.0) atomicAdd(st + 5, ts2);
+        if (tnf) atomicAdd(st + 6, (double)tnf);
+    }
+}
+
+__global__ void jac_init_kernel(double *__restrict__ stats, int B) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < B * JAC_STATS) {
+        const int k = i % JAC_STATS;
+        stats[i] = k == 2 ? INFINITY : (k == 3 ? -INFINITY : 0.0);
+    }
+}
+
+// one voxel per thread: the march of diffusion_reg_kernel, the nine differences kept instead of squared and summed
+template <int MODE>
+__global__ void __launch_bounds__(NCC_THREADS) jacobian_det_kernel(const float *__restrict__ phi, RegDims g, int margin,
+                                                                   float *__restrict__ det, double *__restrict__ stats) {
+    const int x = blockIdx.x * REG_TX + (threadIdx.x & 31), y = blockIdx.y * REG_TY + (threadIdx.x >> 5);
+    const int zc = blockIdx.z % g.n_zchunks, b = blockIdx.z / g.n_zchunks;
+    const int z0 = zc * g.zchunk, z1 = min(g.d, z0 + g.zchunk);
+    JacAcc acc;
+    if (x < g.w && y < g.h) {
+        const bool xlo = x == 0, xhi = x == g.w - 1, ylo = y == 0, yhi = y == g.h - 1;
+        const int oxu = xhi ? 0 : 1, oxd = xlo ? 0 : -1;
+        const int oyu = yhi ? 0 : g.w, oyd = ylo ? 0 : -g.w;
+        const bool in_xy = x >= margin && x < g.w - margin && y >= margin && y < g.h - margin;
+        const unsigned pl = (unsigned)(g.h * g.w), cs = pl * (unsigned)g.d;       // 32-bit indices (B*3*D*H*W < 2^31)
+        unsigned i0 = ((unsigned)b * 3u * (unsigned)g.d + (unsigned)z0) * pl + (unsigned)y * (unsigned)g.w + (unsigned)x;
+        unsigned o0 = ((unsigned)b * (unsigned)g.d + (unsigned)z0) * pl + (unsigned)y * (unsigned)g.w + (unsigned)x;
+        float vm[3], vc[3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            vc[c] = __ldg(phi + (i0 + c * cs));
+            vm[c] = z0 > 0 ? __ldg(phi + (i0 + c * cs - pl)) : vc[c];
+        }
+        for (int z = z0; z < z1; ++z, i0 += pl, o0 += pl) {
+            const bool zlo = z == 0, zhi = z == g.d - 1;
+            float j[3][3];
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                const unsigned ic = i0 + c * cs;
+                const float cc = vc[c];
+                const float vp = zhi ? cc : __ldg(phi + (ic + pl));
+                if (LR_REG_PF > 0 && z + LR_REG_PF <= z1) prefetch_l2(phi + (ic + LR_REG_PF * pl));
+                const float yu = __ldg(phi + (ic + oyu)), yd = __ldg(phi + (ic + oyd));
+                const float xu = __ldg(phi + (ic + oxu)), xd = __ldg(phi + (ic + oxd));
+                j[c][0] = mul_rn(fd_delta<MODE>(vp, vm[c], cc, zlo, zhi), g.sd);
+                j[c][1] = mul_rn(fd_delta<MODE>(yu, yd, cc, ylo, yhi), g.sh);
+                j[c][2] = mul_rn(fd_delta<MODE>(xu, xd, cc, xlo, xhi), g.sw);
+                vm[c] = cc; vc[c] = vp;
+            }
+            const float v = det3(j);
+            if (det) st_stream(det + o0, v);
+            acc.add(v, in_xy && z >= margin && z < g.d - margin);
+        }
+    }
+    jac_block_flush(acc, stats + b * JAC_STATS);
+}
+
+// two voxels per thread (W even, 8-byte-aligned map and output): the loads and differences of diffusion_reg_pair_kernel,
+// the determinant per voxel in scalar fp32 (packed products would be contracted into the subtractions by ptxas)
+template <int MODE>
+__global__ void __launch_bounds__(NCC_THREADS, LR_REGP_MINB) jacobian_det_pair_kernel(const float *__restrict__ phi, RegDims g, int margin,
+                                                                                     float *__restrict__ det, double *__restrict__ stats) {
+    const int x = (blockIdx.x * REGP_TX + (threadIdx.x & (REGP_TX - 1))) * 2, y = blockIdx.y * REGP_TY + (threadIdx.x / REGP_TX);
+    const int zc = blockIdx.z % g.n_zchunks, b = blockIdx.z / g.n_zchunks;
+    const int z0 = zc * g.zchunk, z1 = min(g.d, z0 + g.zchunk);
+    JacAcc acc;
+    if (x < g.w && y < g.h) {
+        const bool xlo = x == 0, xhi = x + 2 == g.w, ylo = y == 0, yhi = y == g.h - 1;
+        const int oxl = xlo ? 0 : -1, oxr = xhi ? 1 : 2;
+        const int oyu = yhi ? 0 : g.w, oyd = ylo ? 0 : -g.w;
+        const bool in_y = y >= margin && y < g.h - margin;
+        const bool in0 = in_y && x >= margin && x < g.w - margin, in1 = in_y && x + 1 >= margin && x + 1 < g.w - margin;
+        const unsigned pl = (unsigned)(g.h * g.w), cs = pl * (unsigned)g.d;
+        unsigned i0 = ((unsigned)b * 3u * (unsigned)g.d + (unsigned)z0) * pl + (unsigned)y * (unsigned)g.w + (unsigned)x;
+        unsigned o0 = ((unsigned)b * (unsigned)g.d + (unsigned)z0) * pl + (unsigned)y * (unsigned)g.w + (unsigned)x;
+        const f32x2 sd2 = splat2(g.sd), sh2 = splat2(g.sh), sw2 = splat2(g.sw);
+        f32x2 vm[3], vc[3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            vc[c] = ldg2(phi + (i0 + c * cs));
+            vm[c] = z0 > 0 ? ldg2(phi + (i0 + c * cs - pl)) : vc[c];
+        }
+        for (int z = z0; z < z1; ++z, i0 += pl, o0 += pl) {
+            const bool zlo = z == 0, zhi = z == g.d - 1;
+            float j0[3][3], j1[3][3];
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                const unsigned ic = i0 + c * cs;
+                const f32x2 cc = vc[c];
+                const f32x2 vp = zhi ? cc : ldg2(phi + (ic + pl));
+                if (LR_REG_PF > 0 && z + LR_REG_PF <= z1) prefetch_l2(phi + (ic + LR_REG_PF * pl));
+                const f32x2 yu = ldg2(phi + (ic + oyu)), yd = ldg2(phi + (ic + oyd));
+                float xl = __ldg(phi + (ic + oxl)), xr = __ldg(phi + (ic + oxr));
+                float c0, c1;
+                unpack2(cc, c0, c1);
+                f32x2 dx;
+                if (MODE == 0) {
+                    if (xlo) xl = fmaf(2.0f, c0, -c1);
+                    if (xhi) xr = fmaf(2.0f, c1, -c0);
+                    dx = sub2(pack2(c1, xr), pack2(xl, c0));
+                } else {
+                    dx = pack2(xlo ? 0.0f : sub_rn(c1, xl), xhi ? 0.0f : sub_rn(xr, c0));
+                }
+                unpack2(mul2(fd_delta2<MODE>(vp, vm[c], cc, zlo, zhi), sd2), j0[c][0], j1[c][0]);
+                unpack2(mul2(fd_delta2<MODE>(yu, yd, cc, ylo, yhi), sh2), j0[c][1], j1[c][1]);
+                unpack2(mul2(dx, sw2), j0[c][2], j1[c][2]);
+                vm[c] = cc; vc[c] = vp;
+            }
+            const float v0 = det3(j0), v1 = det3(j1);
+            if (det) __stcs(reinterpret_cast<float2 *>(det + o0), make_float2(v0, v1));
+            const bool in_z = z >= margin && z < g.d - margin;
+            acc.add(v0, in0 && in_z);
+            acc.add(v1, in1 && in_z);
+        }
+    }
+    jac_block_flush(acc, stats + b * JAC_STATS);
+}
+
+// ---- label confusion matrix: counts[b][p][t] = #voxels with pred == p and target == t ------------------------------
+// Every (pred, target) pair that is not two integers in [0, L) goes to one extra bin, key L*L, reported as `invalid`.
+// The histogram is privatised in shared memory ((L*L+1) 32-bit bins, <= 64 KB at L = 128) and merged into the int64
+// output with one 64-bit atomic per non-empty bin and block.  Label maps are mostly background, so equal keys are
+// first aggregated within the warp (all lanes equal: one atomic; otherwise __match_any_sync groups) before the shared
+// atomic: without that, L = 2 would serialise every warp on one bin.
+constexpr int CONF_THREADS = 256;
+
+// key of a (pred, target) pair; (v + 1.5*2^23) - 1.5*2^23 == v holds exactly for the integers |v| < 2^22, and the
+// integer is in the mantissa (rint_i): no F2I / FRND on the XU pipe
+__device__ __forceinline__ int label_key(float p, float t, int L, float fL) {
+    const float M = 12582912.0f;
+    const float tp = __fadd_rn(p, M), tt = __fadd_rn(t, M);
+    const bool ok = p >= 0.0f && p < fL && t >= 0.0f && t < fL && __fsub_rn(tp, M) == p && __fsub_rn(tt, M) == t;
+    return ok ? (__float_as_int(tp) - 0x4B400000) * L + (__float_as_int(tt) - 0x4B400000) : L * L;
+}
+
+// one key per lane (key < 0: lane has nothing), called by the whole warp
+__device__ __forceinline__ void hist_add_warp(unsigned *__restrict__ h, int key, int lane) {
+    const int k0 = __shfl_sync(0xffffffffu, key, 0);
+    if (__all_sync(0xffffffffu, key == k0)) {
+        if (lane == 0 && k0 >= 0) atomicAdd(h + k0, 32u);
+        return;
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, key);
+    if (key >= 0 && lane == __ffs(peers) - 1) atomicAdd(h + key, (unsigned)__popc(peers));
+}
+
+__global__ void __launch_bounds__(CONF_THREADS) label_confusion_kernel(const float *__restrict__ pred, const float *__restrict__ target,
+                                                                       int64_t N, int L, unsigned long long *__restrict__ counts,
+                                                                       unsigned long long *__restrict__ invalid) {
+    extern __shared__ unsigned hist[];
+    const int nbins = L * L + 1, b = blockIdx.y, lane = threadIdx.x & 31;
+    for (int i = threadIdx.x; i < nbins; i += CONF_THREADS) hist[i] = 0u;
+    __syncthreads();
+    const float fL = (float)L;
+    const float *pb = pred + (int64_t)b * N, *tb = target + (int64_t)b * N;
+    // warp-uniform trip counts (every lane of a warp runs every iteration; lanes past the end carry key -1)
+    const int64_t wid = ((int64_t)blockIdx.x * CONF_THREADS + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * CONF_THREADS) >> 5;
+    const int64_t n4 = (((uintptr_t)pb | (uintptr_t)tb) % 16 == 0) ? N / 4 : 0;
+    for (int64_t base = wid * 32; base < n4; base += nwarps * 32) {
+        const int64_t i = base + lane;
+        int k[4] = {-1, -1, -1, -1};
+        if (i < n4) {
+            const float4 p = ld_stream4(reinterpret_cast<const float4 *>(pb) + i), t = ld_stream4(reinterpret_cast<const float4 *>(tb) + i);
+            k[0] = label_key(p.x, t.x, L, fL); k[1] = label_key(p.y, t.y, L, fL);
+            k[2] = label_key(p.z, t.z, L, fL); k[3] = label_key(p.w, t.w, L, fL);
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) hist_add_warp(hist, k[j], lane);
+    }
+    for (int64_t base = 4 * n4 + wid * 32; base < N; base += nwarps * 32) {
+        const int64_t i = base + lane;
+        hist_add_warp(hist, i < N ? label_key(ld_stream(pb + i), ld_stream(tb + i), L, fL) : -1, lane);
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < nbins; i += CONF_THREADS) {
+        const unsigned c = hist[i];
+        if (c) atomicAdd(i < nbins - 1 ? counts + (int64_t)b * (nbins - 1) + i : invalid + b, (unsigned long long)c);
+    }
+}
+
+static unsigned conf_blocks(int64_t N, int B, int L, int per_sm) {
+    int64_t want = (N + CONF_THREADS * 16 - 1) / (CONF_THREADS * 16);          // >= 16 voxels per thread
+    const int64_t by_bins = N / (4 * (int64_t)L * L);                          // the merge stays small next to the streaming
+    if (want > by_bins) want = by_bins;
+    const int64_t cap = ((int64_t)sm_count() * per_sm + B - 1) / B;              // one wave over the whole grid
+    if (want > cap) want = cap;
+    return (unsigned)(want < 1 ? 1 : want);
+}
+
 }  // namespace lr
 
 using namespace lr;
@@ -583,4 +859,63 @@ extern "C" int lr_diffusion_reg_backward(const float *disp, int B, int D, int H,
     if (boundary == LR_FD_LINEAR) diffusion_reg_backward_kernel<0><<<grid, NCC_THREADS, 0, st>>>(disp, g, B, grad_loss, grad_disp);
     else diffusion_reg_backward_kernel<1><<<grid, NCC_THREADS, 0, st>>>(disp, g, B, grad_loss, grad_disp);
     return check_launch("diffusion_reg_backward_kernel");
+}
+
+template <int MODE>
+static int jacobian_launch(const float *phi, int B, int D, int H, int W, int margin, float *det, double *stats, cudaStream_t st) {
+    RegDims g; dim3 grid;
+    const bool pairs = reg_use_pairs(phi, det, W);
+    const int rd = pairs ? reg_dims(jacobian_det_pair_kernel<MODE>, true, LR_REG_WAVES, B, D, H, W, g, grid)
+                         : reg_dims(jacobian_det_kernel<MODE>, false, LR_REG_WAVES, B, D, H, W, g, grid);
+    LR_REQUIRE(rd == 0, "jacobian_det: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)", B, D, H, W);
+    jac_init_kernel<<<(B * JAC_STATS + 127) / 128, 128, 0, st>>>(stats, B);
+    if (int e = check_launch("jac_init_kernel")) return e;
+    if (pairs) {
+        jacobian_det_pair_kernel<MODE><<<grid, NCC_THREADS, 0, st>>>(phi, g, margin, det, stats);
+        return check_launch("jacobian_det_pair_kernel");
+    }
+    jacobian_det_kernel<MODE><<<grid, NCC_THREADS, 0, st>>>(phi, g, margin, det, stats);
+    return check_launch("jacobian_det_kernel");
+}
+
+extern "C" int lr_jacobian_det(const float *phi, int B, int D, int H, int W, int boundary, int margin, float *det, double *stats,
+                               lr_stream_t stream) {
+    LR_REQUIRE(phi && stats, "jacobian_det: null pointer");
+    LR_REQUIRE(B > 0 && D >= 2 && H >= 2 && W >= 2, "jacobian_det: every axis needs >= 2 entries (B=%d, %dx%dx%d)", B, D, H, W);
+    LR_REQUIRE(boundary == LR_FD_LINEAR || boundary == LR_FD_NEUMANN_ZERO, "jacobian_det: unknown boundary mode %d", boundary);
+    LR_REQUIRE(margin >= 0 && 2 * (int64_t)margin < D && 2 * (int64_t)margin < H && 2 * (int64_t)margin < W,
+               "jacobian_det: margin %d leaves no interior voxel of %dx%dx%d (2*margin must be < every axis)", margin, D, H, W);
+    LR_REQUIRE((int64_t)B * 3 * D * H * W < ((int64_t)1 << 31),
+               "jacobian_det: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)", B, D, H, W);
+    cudaStream_t st = as_stream(stream);
+    return boundary == LR_FD_LINEAR ? jacobian_launch<0>(phi, B, D, H, W, margin, det, stats, st)
+                                    : jacobian_launch<1>(phi, B, D, H, W, margin, det, stats, st);
+}
+
+extern "C" int lr_label_confusion(const float *pred, const float *target, int B, int64_t N, int L, int64_t *counts, int64_t *invalid,
+                                  lr_stream_t stream) {
+    LR_REQUIRE(pred && target && counts && invalid, "label_confusion: null pointer");
+    LR_REQUIRE(L >= 1 && L <= 128, "label_confusion: number of labels L=%d must be in [1, 128]", L);
+    LR_REQUIRE(B > 0 && B <= 65535 && N > 0, "label_confusion: bad size (B=%d N=%lld)", B, (long long)N);
+    cudaStream_t st = as_stream(stream);
+    const size_t smem = sizeof(unsigned) * ((size_t)L * L + 1);
+    static thread_local int attr_dev = -1, per_sm = 0;       // the > 48 KB opt-in is per device
+    int dev = 0;
+    cudaError_t ce = cudaGetDevice(&dev);
+    if (ce == cudaSuccess && dev != attr_dev) {
+        ce = cudaFuncSetAttribute(label_confusion_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(unsigned) * (128 * 128 + 1)));
+        if (ce == cudaSuccess) attr_dev = dev;
+    }
+    if (ce != cudaSuccess) { set_error("label_confusion: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, label_confusion_kernel, CONF_THREADS, smem) != cudaSuccess || per_sm < 1) {
+        cudaGetLastError();
+        per_sm = 1;
+    }
+    ce = cudaMemsetAsync(counts, 0, sizeof(int64_t) * (size_t)B * L * L, st);
+    if (ce == cudaSuccess) ce = cudaMemsetAsync(invalid, 0, sizeof(int64_t) * (size_t)B, st);
+    if (ce != cudaSuccess) { set_error("label_confusion: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    const dim3 grid(conf_blocks(N, B, L, per_sm), (unsigned)B);
+    label_confusion_kernel<<<grid, CONF_THREADS, smem, st>>>(pred, target, N, L, reinterpret_cast<unsigned long long *>(counts),
+                                                              reinterpret_cast<unsigned long long *>(invalid));
+    return check_launch("label_confusion_kernel");
 }

@@ -494,3 +494,61 @@ def diffusion_reg(disp, boundary="linear"):
     if boundary not in FD_BOUNDARY:
         raise ValueError("boundary must be one of %s, got %r" % (sorted(FD_BOUNDARY), boundary))
     return _DiffusionReg.apply(disp, FD_BOUNDARY[boundary])
+
+
+# --------------------------------------------------------------------------- validation metrics (not differentiable)
+JACOBIAN_STATS = ("folding_count", "folding_abs_sum", "det_min", "det_max", "det_sum", "det_sum_sq", "nonfinite_count")
+
+
+def jacobian_det(phi, boundary="linear", margin=0, want_map=False):
+    """Jacobian determinant of a map phi (B,3,D,H,W) in [-1,1] (channel c addresses volume axis c) with the
+    regulariser's central differences and face rule `boundary`, scaled so that the identity map has det 1.
+
+    Returns (stats, det): stats is a (B,7) float64 CUDA tensor ordered as JACOBIAN_STATS, over the voxels at least
+    `margin` from every face (sums and min / max over finite values only); det is the (B,D,H,W) float32 map when
+    want_map, else None.  Parity with the reference's utils.py:20-55 is unpinned (include/liftreg_b200.h)."""
+    if not isinstance(phi, torch.Tensor) or phi.dim() != 5 or phi.shape[1] != 3:
+        raise ValueError("phi must be a (B,3,D,H,W) tensor, got %s" % (tuple(phi.shape) if isinstance(phi, torch.Tensor) else type(phi).__name__,))
+    if boundary not in FD_BOUNDARY:
+        raise ValueError("boundary must be one of %s, got %r" % (sorted(FD_BOUNDARY), boundary))
+    phi = _need_cuda_f32(phi, "phi")
+    B, _, D, H, W = phi.shape
+    stats = torch.empty((B, 7), device=phi.device, dtype=torch.float64)
+    det = torch.empty((B, D, H, W), device=phi.device, dtype=torch.float32) if want_map else None
+    with torch.cuda.device(phi.device):
+        _native.check(_native.lib().lr_jacobian_det(_ptr(phi), B, D, H, W, FD_BOUNDARY[boundary], int(margin), _ptr(det),
+                                                    _ptr(stats), _stream()), "lr_jacobian_det")
+    return stats, det
+
+
+def _label_map(t, name):
+    if not isinstance(t, torch.Tensor):
+        raise TypeError("%s must be a torch.Tensor, got %s" % (name, type(t).__name__))
+    if not t.is_cuda:
+        raise RuntimeError("%s must be a CUDA tensor: liftreg_b200 has no CPU path (got device %s)" % (name, t.device))
+    if t.dtype in (torch.uint8, torch.int8, torch.int16, torch.int32, torch.int64, torch.bool):
+        t = t.float()
+    return _need_cuda_f32(t, name)
+
+
+def label_confusion(pred, target, num_labels):
+    """Confusion matrix of two label maps with a leading batch axis (any trailing shape, equal for both):
+    counts (B,L,L) int64 with counts[b,p,t] = #voxels where pred == p and target == t, and invalid (B,) int64 = #voxels
+    where either value is not an integer in [0, L).  Float32 maps (what the nearest-mode warp returns) are read as they
+    are, integer maps are converted with .float().  1 <= num_labels <= 128."""
+    if pred.shape != target.shape or pred.dim() < 1:
+        raise ValueError("pred %s and target %s must have the same shape (B, ...)" % (tuple(pred.shape), tuple(target.shape)))
+    L = int(num_labels)
+    if not 1 <= L <= 128:
+        raise ValueError("num_labels must be in [1, 128], got %d" % L)
+    pred, target = _label_map(pred, "pred"), _label_map(target, "target")
+    if pred.device != target.device:
+        raise ValueError("pred and target must be on the same device")
+    B = pred.shape[0]
+    N = pred.numel() // B if B else 0
+    counts = torch.empty((B, L, L), device=pred.device, dtype=torch.int64)
+    invalid = torch.empty((B,), device=pred.device, dtype=torch.int64)
+    with torch.cuda.device(pred.device):
+        _native.check(_native.lib().lr_label_confusion(_ptr(pred), _ptr(target), B, N, L, _ptr(counts), _ptr(invalid),
+                                                       _stream()), "lr_label_confusion")
+    return counts, invalid

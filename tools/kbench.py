@@ -120,13 +120,41 @@ def main():
     def k_reg_bwd(s, st):
         _native.check(lib.lr_diffusion_reg_backward(vp(s["phi"]), 1, *VOL, 0, vp(ncc_g), vp(s["gphi"]), st), "reg_bwd")
 
+    jac_stats = torch.zeros((1, 7), device=dev, dtype=torch.float64)
+
+    def k_jac(s, st):          # Jacobian-determinant statistics of the map (validation folding metric): one pass over phi
+        _native.check(lib.lr_jacobian_det(vp(s["phi"]), 1, *VOL, 0, 0, None, vp(jac_stats), st), "jac")
+
+    def k_jac_map(s, st):      # ... and the determinant map written out
+        _native.check(lib.lr_jacobian_det(vp(s["phi"]), 1, *VOL, 0, 0, vp(s["warped"]), vp(jac_stats), st), "jac_map")
+
+    if "labels2" in which or "labels6" in which:
+        # label maps as a validation item has them: mostly background, a few organ-sized blobs, target = shifted pred
+        zz, yy, xx = np.meshgrid(*[np.arange(n) for n in VOL], indexing="ij")
+        for i, s_ in enumerate(sets):
+            for L in (2, 6):
+                lab = np.zeros(VOL, np.float32)
+                for k in range(1, L):
+                    c = rs.randint(40, 120, 3)
+                    lab[(zz - c[0]) ** 2 + (yy - c[1]) ** 2 + (xx - c[2]) ** 2 < 30 ** 2] = k
+                s_["pred%d" % L] = torch.from_numpy(lab).to(dev)
+                s_["target%d" % L] = torch.from_numpy(np.roll(lab, 3, axis=0)).to(dev)
+    conf_counts, conf_invalid = torch.zeros((1, 36), device=dev, dtype=torch.int64), torch.zeros(1, device=dev, dtype=torch.int64)
+
+    def k_labels(L):           # confusion matrix of two label maps (validation overlap metrics)
+        def k(s, st):
+            _native.check(lib.lr_label_confusion(vp(s["pred%d" % L]), vp(s["target%d" % L]), 1, nv, L, vp(conf_counts),
+                                                 vp(conf_invalid), st), "labels%d" % L)
+        return k
+
     def k_atten(s, st):        # HU -> attenuation (sdct:6-13), elementwise
         _native.check(lib.lr_atten_coef(vp(s["moving"]), nv, vp(s["warped"]), st), "atten")
 
     def k_idmap(s, st):        # identity map (net_utils.py:59-87), write-only
         _native.check(lib.lr_identity_map(*VOL, vp(s["gphi"]), st), "idmap")
 
-    units = {"atten": (k_atten, nv, 8 * nv), "idmap": (k_idmap, nv, 12 * nv), "reg": (k_reg, nv, 12 * nv), "reg_bwd": (k_reg_bwd, nv, 24 * nv), "ncc": (k_ncc, nv, 8 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
+    units = {"atten": (k_atten, nv, 8 * nv), "idmap": (k_idmap, nv, 12 * nv), "reg": (k_reg, nv, 12 * nv), "jac": (k_jac, nv, 12 * nv), "jac_map": (k_jac_map, nv, 16 * nv),
+             "labels2": (k_labels(2), nv, 8 * nv), "labels6": (k_labels(6), nv, 8 * nv), "reg_bwd": (k_reg_bwd, nv, 24 * nv), "ncc": (k_ncc, nv, 8 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
              "pca_bwd": (k_pca_bwd, 3 * nv, 4 * 3 * nv * 56 + 4 * 3 * nv), "warp_bwd": (k_warp_bwd, nv, 32 * nv),
              "drr_bwd": (k_drr_bwd, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240), "backproject": (k_backproject, batch * P * nv, batch * (4 * P * nv + 4 * P * DET[0] * DET[1])),
              "backproject_planned": (k_backproject_planned, batch * P * nv, batch * (4 * P * nv + 4 * P * DET[0] * DET[1])),
