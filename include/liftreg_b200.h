@@ -202,7 +202,8 @@ LR_API int lr_stream_synchronize(lr_stream_t stream);
  *   using_scale: sample (img+1)/2 and return 2*out-1 (:48-52), fused.
  *   disp_plus_identity != 0: phi holds the DISPLACEMENT and the normalised identity map
  *   (net_utils.py:59-87) is added in-kernel, i.e. the `disp_field + self.id_transform` of model :68 is fused;
- *   the sum is rounded to fp32 exactly as the torch add would. */
+ *   the sum is rounded to fp32 exactly as the torch add would.  The identity map needs D, H, W >= 2 (as
+ *   lr_identity_map); a size-1 axis with disp_plus_identity != 0 is rejected (LR_ERR_BAD_ARGUMENT). */
 LR_API int lr_warp_forward(const float *img, const float *phi, int B, int C, int D, int H, int W,
                            int padding, int mode, int using_scale, int disp_plus_identity,
                            float *out, lr_stream_t stream);

@@ -721,8 +721,11 @@ static WarpDims make_dims(int C, int D, int H, int W, int z_begin = 0, int z_cou
     return g;
 }
 
-static int check_warp_args(int B, int C, int D, int H, int W, int padding, int mode) {
+static int check_warp_args(int B, int C, int D, int H, int W, int padding, int mode, int disp_plus_identity = 0) {
     LR_REQUIRE(B > 0 && C > 0 && D > 0 && H > 0 && W > 0, "warp: non-positive dimension (B=%d C=%d D=%d H=%d W=%d)", B, C, D, H, W);
+    // the identity map divides by S-1 (as lr_identity_map, which rejects these sizes): undefined on a size-1 axis
+    LR_REQUIRE(!disp_plus_identity || (D > 1 && H > 1 && W > 1),
+               "warp: disp_plus_identity needs every size >= 2 (D=%d H=%d W=%d)", D, H, W);
     LR_REQUIRE((int64_t)D * H * W < (1ll << 31) - 2 * (int64_t)H * W - 4, "warp: D*H*W must fit 32-bit voxel offsets");
     LR_REQUIRE(D < 65536 && (H + WARP_TY - 1) / WARP_TY <= 65535, "warp: D and H/8 must be < 65536 (grid limits)");
     LR_REQUIRE(W < (1 << 21) && H < (1 << 21), "warp: H and W must be < 2^21 (mantissa floor)");
@@ -828,7 +831,7 @@ extern "C" int lr_warp_forward_slab(const float *img, const float *phi, int B, i
                                     int z_count, int padding, int mode, int using_scale, int disp_plus_identity,
                                     float *out, lr_stream_t stream) {
     LR_REQUIRE(img && phi && out, "warp_forward: null pointer");
-    if (int e = check_warp_args(B, C, D, H, W, padding, mode)) return e;
+    if (int e = check_warp_args(B, C, D, H, W, padding, mode, disp_plus_identity)) return e;
     if (int e = check_slab(D, z_begin, z_count)) return e;
     WarpDims g = make_dims(C, D, H, W, z_begin, z_count);
     cudaStream_t st = as_stream(stream);
@@ -875,7 +878,7 @@ extern "C" int lr_warp_backward_slab(const float *grad_out, const float *img, co
                                      int W, int z_begin, int z_count, int padding, int mode, int using_scale,
                                      int disp_plus_identity, float *grad_img, float *grad_phi, lr_stream_t stream) {
     LR_REQUIRE(grad_out && img && phi, "warp_backward: null pointer");
-    if (int e = check_warp_args(B, C, D, H, W, padding, mode)) return e;
+    if (int e = check_warp_args(B, C, D, H, W, padding, mode, disp_plus_identity)) return e;
     if (int e = check_slab(D, z_begin, z_count)) return e;
     if (!grad_img && !grad_phi) return LR_OK;
     cudaStream_t st = as_stream(stream);
