@@ -158,20 +158,6 @@ LR_API int lr_backproject_forward_slab(const float *proj, const float *poses, in
                                        int d_total, int w, int h, int i_begin, int i_count, float *out,
                                        int64_t out_batch_stride, int64_t out_chan_stride, lr_stream_t stream);
 
-/* Geometry plan.  Everything lr_backproject_forward derives from (poses, shapes) -- floor detector rows / columns and
- * interpolation weights of every plane and voxel column, per view and coronal row -- can be evaluated ONCE into a
- * caller-owned device buffer, exactly as the reference caches its (1,P,2,d,w,h) sample grid on the first batch
- * (LiftRegDeformSubspaceBackproj.py:85-87; 131 MB there, 3 MB here).  lr_backproject_forward_planned then only gathers,
- * blends and stores (fast numerics: the separable blend of LR_NUMERICS_FAST, whatever lr_set_numerics says; indices and
- * weights are the same bit-exact chain).  The plan depends on (poses, P, pw, ph, d_total, w, h) only: any batch size,
- * any z-slab [i_begin, i_begin+i_count) and any output strides may use it.  plan must be 16-byte aligned. */
-LR_API size_t lr_backproject_plan_bytes(int P, int pw, int ph, int d_total, int w, int h);
-LR_API int lr_backproject_plan_build(const float *poses, int P, int pw, int ph, int d_total, int w, int h,
-                                     void *plan, size_t plan_bytes, lr_stream_t stream);
-LR_API int lr_backproject_forward_planned(const float *proj, const void *plan, int B, int P, int pw, int ph,
-                                          int d_total, int w, int h, int i_begin, int i_count, float *out,
-                                          int64_t out_batch_stride, int64_t out_chan_stride, lr_stream_t stream);
-
 /* adjoint wrt proj; grad_proj (B,P,pw,ph) is ACCUMULATED into (caller zero-initialises). */
 LR_API int lr_backproject_backward(const float *grad_out, int64_t go_batch_stride, int64_t go_chan_stride,
                                    const float *poses, int B, int P, int pw, int ph, int d, int w, int h,

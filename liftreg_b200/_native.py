@@ -34,9 +34,6 @@ SIGNATURES = {
     "lr_drr_forward_host": (_i, [_vp, _i, _i, _i, _i, c_double_p, _i, _i, _i, _i, c_float_p, _i, _f, _vp, _vp, _sz, _vp]),
     "lr_backproject_forward": (_i, [_vp, c_float_p, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _i64, _vp]),
     "lr_backproject_forward_slab": (_i, [_vp, c_float_p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _i64, _vp]),
-    "lr_backproject_plan_bytes": (_sz, [_i, _i, _i, _i, _i, _i]),
-    "lr_backproject_plan_build": (_i, [c_float_p, _i, _i, _i, _i, _i, _i, _vp, _sz, _vp]),
-    "lr_backproject_forward_planned": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _i64, _vp]),
     "lr_backproject_backward": (_i, [_vp, _i64, _i64, c_float_p, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "lr_backproj_grid": (_i, [c_float_p, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "lr_backproject_forward_host_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i]),

@@ -15,9 +15,6 @@
 // (lanes along h: coalesced 128 B stores, near-contiguous gathers), keeps its v-part in registers and walks a
 // chunk of i; the per-i u-part comes from a small shared-memory table built once per block and row j.  Batch items
 // are a grid dimension.
-#include <cstdio>
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace lr {
@@ -66,12 +63,11 @@ struct AxisTap {      // one axis of the bilinear footprint
 };
 
 // normalised coordinate -> (floor index, upper weight), ATen vector-kernel order
-__device__ __forceinline__ AxisTap axis_tap(float centred, float s_c, float scale, ConstDiv size, float half_sm1, float wide = 0.0f) {
+__device__ __forceinline__ AxisTap axis_tap(float centred, float s_c, float scale, ConstDiv size, float half_sm1) {
     float a = add_rn(mul_rn(sub_rn(centred, s_c), scale), s_c);   // (x - s)*scale + s
     float g = mul_rn(div_const(a, size), 2.0f);                   // / size * 2
     float ix = mul_rn(add_rn(g, 1.0f), half_sm1);                 // (g+1)*((S-1)/2)
-    // beyond [-2, S+1] no tap is in bounds; `wide` (the plan builder) only keeps floor_fi's |x| < 2^22 precondition
-    ix = wide > 0.0f ? fminf(fmaxf(ix, -wide), wide) : clamp_index(ix, half_sm1 * 2.0f + 3.0f);
+    ix = clamp_index(ix, half_sm1 * 2.0f + 3.0f);                 // beyond [-2, S+1] no tap is in bounds
     float fl;
     AxisTap t;
     floor_fi(ix, fl, t.i0);
@@ -293,7 +289,7 @@ __global__ void __launch_bounds__(256)
 //   rows      the per-plane table of the generic path: taken by a (block, j) whose planes do not move strictly down the
 //             detector (magnification < 1, clamped far-outside coordinates) or span more than BP_EV_MAX rows.
 // (Measured and dropped, profiles/README.md round 2: staging the block's output rows in shared memory and writing them
-// with cp.async.bulk -- 39 us vs 23 us; a precomputed geometry plan read from global memory -- see further down.)
+// with cp.async.bulk -- 39 us vs 23 us; a precomputed geometry plan read from global memory -- 25.6 us vs 21.4 us, DESIGN.md.)
 constexpr int BP_EV_MAX = 112;
 constexpr int BP_MAX_SUB = 8;
 constexpr int BP_JS_MAX = 4;       // rows j per block (the longest run)
@@ -319,9 +315,6 @@ __device__ __forceinline__ f32x2 bp_fetch_row(const float *lo0, const float *lo1
         const float a1 = (rv && c10) ? __ldg(q1) : 0.0f, b1 = (rv && c11) ? __ldg(q1 + 1) : 0.0f;
         va = pack2(a0, a1); vb = pack2(b0, b1);
     } else {
-#ifdef LR_BP_ABLATE_L1HIT       // experiment: every row fetch reads one of two detector rows (all L1 hits, same instruction stream)
-        roff = (roff & 1) * 256;
-#endif
         // ROWCHK: a row outside the detector is fetched from row 0 instead and its T replaced by +0 afterwards -- two
         // selects, no branch: a branch here would keep the compiler from batching the loads of the unrolled rows
         const unsigned o = ROWCHK ? (unsigned)max(roff, 0) : (unsigned)roff;
@@ -339,11 +332,6 @@ __device__ __forceinline__ f32x2 bp_fetch_row(const float *lo0, const float *lo1
 #define LR_STR2(x) #x
 #define LR_STR(x) LR_STR2(x)
 #define LR_BP_UNROLL_PRAGMA _Pragma(LR_STR(unroll LR_BP_UNROLL))
-#ifdef LR_BP_ROWS_MINB          // kernel experiments: explicit register cap
-#define LR_BP_ROWS_BOUNDS __launch_bounds__(LR_BP_ROWS_MAXT, LR_BP_ROWS_MINB)
-#else
-#define LR_BP_ROWS_BOUNDS __launch_bounds__(256)      // ptxas settles on 64 registers (6 blocks of 160 threads per SM)
-#endif
 
 // One thread's two columns over one sub-chunk of planes.
 template <bool ROWCHK, bool COLCHK>
@@ -367,7 +355,7 @@ __device__ __forceinline__ void bp_march_rows(const BpEvent *__restrict__ ev, in
     }
 }
 
-__global__ void LR_BP_ROWS_BOUNDS
+__global__ void __launch_bounds__(256)      // ptxas settles on 64 registers (6 blocks of 160 threads per SM)
     backproject_forward_rows_kernel(const float *__restrict__ proj, float *__restrict__ out, BpDims g, BpPoses poses) {
     __shared__ BpEvent ev_all[BP_JS_MAX][BP_EV_MAX];
     __shared__ BpRow rows_all[BP_JS_MAX][BP_ICHUNK];
@@ -481,9 +469,7 @@ __global__ void LR_BP_ROWS_BOUNDS
                 float *o0 = opaque(ob + k0), *o1 = opaque(ob + k1);
                 const unsigned ofs = (unsigned)ii0 * plane;
                 if (cols_in && rows_in) bp_march_rows<false, false>(ev_all[jr], s_lo, s_hi, lo0, lo1, o0, o1, ofs, plane, e2, w2, c00, c01, c10, c11, has1);
-#ifndef LR_BP_NO_ROWCHK_VARIANT
                 else if (cols_in) bp_march_rows<true, false>(ev_all[jr], s_lo, s_hi, lo0, lo1, o0, o1, ofs, plane, e2, w2, c00, c01, c10, c11, has1);
-#endif
                 else bp_march_rows<true, true>(ev_all[jr], s_lo, s_hi, lo0, lo1, o0, o1, ofs, plane, e2, w2, c00, c01, c10, c11, has1);
             } else {
                 // generic geometry: per-plane table, per-tap predicates, same separable blend
@@ -491,175 +477,6 @@ __global__ void LR_BP_ROWS_BOUNDS
                 unpack2(w2, wq0, wq1); unpack2(e2, e0, e1);
                 backproject_column_checked<true>(pv0 + c0, (char *)(ob + k0) + ii0 * plane_bytes, plane_bytes, rows, ii0, ii1, g.ph, c00, c01, e0, wq0);
                 if (has1) backproject_column_checked<true>(pv0 + c1, (char *)(ob + k1) + ii0 * plane_bytes, plane_bytes, rows, ii0, ii1, g.ph, c10, c11, e1, wq1);
-            }
-        }
-    }
-}
-
-// ---- forward with a precomputed geometry plan ---------------------------------------------------------------------
-// The tables the rows kernel rebuilds for every (block, row j) depend on the GEOMETRY only (poses and shapes), which a
-// registration run fixes once -- the reference caches its 131 MB sample grid for the same reason
-// (LiftRegDeformSubspaceBackproj.py:85-87: `self.backward_proj_grids`).  lr_backproject_plan_build evaluates them once
-// into a caller-owned device buffer (3 MB at cfg 2, L2-resident) and backproject_forward_plan_kernel only marches:
-// no shared memory, no barrier, no division, no axis_tap chain in the hot kernel.  MEASURED (profiles/README.md, round 2):
-// 30.4 us against 23.4 us for the rows kernel at cfg 2 -- the per-row table entry becomes a dependent global load (L2
-// latency) at the head of every gather, which costs more than rebuilding the tables in shared memory.  (After the
-// builder stopped clamping far-outside rows -- which had sent 31 % of the rows down the generic path -- it is 25.3 us;
-// a variant that first stages the block's slice of the plan in shared memory and then runs the rows kernel's march:
-// 27.6 us, 22 us per item at batch 8 against 17: every block starts with two L2 round trips during which its warps
-// idle, whereas the rows kernel's table building is arithmetic on kernel parameters.)  The entry points are kept (any
-// z-slab / stride, bit-identical results, tested) but ops.backproject does not use them.
-// One record per (view p, coronal row j), 16-byte aligned, all 4-byte words:
-//   [0] r_base   floor detector row of plane 0      [1] flags  bit 0: planes move strictly down the detector and the
-//   [2] n_slots  rows r_base .. r_base+n_slots-1         row range fits the event table (fast path allowed)
-//   rowtab[d]    (int r0, float n)      per plane: floor row and upper-row weight (generic path; slot = r0 - r_base)
-//   evtab[EVP]   (float n, int roff)    per detector row: see BpEvent
-//   coltab[h]    (int c, float wq)      per voxel column: floor detector column and upper-column weight
-struct BpPlanLayout {
-    int d, h, evp;          // planes, columns, event slots per record
-    int rec_words;          // record pitch in 4-byte words (multiple of 4)
-    __host__ __device__ int rowtab() const { return 4; }
-    __host__ __device__ int evtab() const { return 4 + 2 * d; }
-    __host__ __device__ int coltab() const { return 4 + 2 * d + 2 * evp; }
-};
-static BpPlanLayout plan_layout(int d, int h) {
-    BpPlanLayout L;
-    L.d = d; L.h = h;
-    L.evp = 3 * d + 8;
-    L.rec_words = (4 + 2 * d + 2 * L.evp + 2 * h + 3) & ~3;
-    return L;
-}
-
-// grid (w, P); block 256.  Uses the same axis_tap chain as the kernels, so every index and weight is the reference's.
-__global__ void __launch_bounds__(256) backproject_plan_kernel(int *__restrict__ plan, BpPlanLayout L, BpDims g, BpPoses poses) {
-    const int j = blockIdx.x, pl = blockIdx.y, p = g.p0 + pl;
-    int *rec = plan + ((int64_t)p * g.w + j) * L.rec_words;
-    const float sx = poses.s[pl][0], sy = poses.s[pl][1], sz = poses.s[pl][2];
-    const float scale = view_scale(sy, g.w, j);
-    int2 *rowtab = reinterpret_cast<int2 *>(rec + L.rowtab());
-    int2 *evtab = reinterpret_cast<int2 *>(rec + L.evtab());
-    int2 *coltab = reinterpret_cast<int2 *>(rec + L.coltab());
-    for (int i = threadIdx.x; i < L.d; i += blockDim.x) {
-        // wide clamp: planes whose detector rows lie far outside keep DISTINCT floor rows (axis_tap's clamp to [-2, S+2]
-        // would make them equal and fail the strictly-increasing test for the whole row j; their taps are skipped either
-        // way, so the result is the same)
-        const AxisTap t = axis_tap((float)i - g.half_d, sx, scale, g.div_pw, g.hpw, 2097152.0f);
-        rowtab[i] = make_int2(t.i0, __float_as_int(t.w1));
-    }
-    for (int k = threadIdx.x; k < L.h; k += blockDim.x) {
-        const AxisTap t = axis_tap((float)k - g.half_h, sz, scale, g.div_ph, g.hph);
-        coltab[k] = make_int2(t.i0, __float_as_int(t.w1));
-    }
-    __syncthreads();                                 // this block's global writes are visible to the block
-    const int r_base = rowtab[0].x, r_last = rowtab[L.d - 1].x;
-    int mono = 1;
-    for (int i = threadIdx.x + 1; i < L.d; i += blockDim.x) mono &= rowtab[i].x > rowtab[i - 1].x;
-    const int n_slots = r_last + 2 - r_base;
-    const bool fast = __syncthreads_and(mono) && n_slots <= L.evp && n_slots >= 2;
-    if (fast) {
-        for (int i = threadIdx.x; i < L.d; i += blockDim.x) {
-            const int2 t = rowtab[i];
-            const int slot = t.x + 1 - r_base;
-            for (int s2 = i == 0 ? 0 : rowtab[i - 1].x + 2 - r_base; s2 < slot; ++s2) {      // rows no plane ends at
-                const int r = r_base + s2;
-                evtab[s2] = make_int2(__float_as_int(-1.0f), (unsigned)r < (unsigned)g.pw ? r * g.ph : -1);
-            }
-            evtab[slot] = make_int2(t.y, (unsigned)(t.x + 1) < (unsigned)g.pw ? (t.x + 1) * g.ph : -1);
-        }
-    }
-    if (threadIdx.x == 0) { rec[0] = r_base; rec[1] = fast ? 1 : 0; rec[2] = n_slots; rec[3] = 0; }
-}
-
-// Generic geometry from the plan: per-plane (r0, n), per-tap predicates, separable blend (as the rows kernel's generic path)
-__device__ __forceinline__ void backproject_column_plan_checked(const float *pvf, float *o, unsigned plane, const int2 *__restrict__ rowtab,
-                                                                int ia, int ib, int pw, int ph, bool c0, bool c1, float e, float wq) {
-    for (int i = ia; i < ib; ++i) {
-        const int2 t = __ldg(rowtab + i);
-        const float n = __int_as_float(t.y), s = sub_rn(1.0f, n);
-        const bool rv0 = (unsigned)t.x < (unsigned)pw, rv1 = (unsigned)(t.x + 1) < (unsigned)pw;
-        const float *q0 = pvf + t.x * ph, *q1 = q0 + ph;
-        const float va = (rv0 && c0) ? __ldg(q0) : 0.0f, vb = (rv0 && c1) ? __ldg(q0 + 1) : 0.0f;
-        const float vc = (rv1 && c0) ? __ldg(q1) : 0.0f, vd = (rv1 && c1) ? __ldg(q1 + 1) : 0.0f;
-        st_stream(o, bilerp_sep(va, vb, vc, vd, s, n, e, wq));
-        o += plane;
-    }
-}
-
-template <bool CHK>
-__device__ __forceinline__ void bp_march_plan(const int2 *__restrict__ ev, int s_lo, int s_hi, const float *lo0, const float *lo1,
-                                              float *o0, float *o1, unsigned plane, f32x2 e2, f32x2 w2, bool c00, bool c01,
-                                              bool c10, bool c11, bool has1) {
-    f32x2 t_prev = bp_fetch_row<CHK, CHK>(lo0, lo1, __ldg(ev + s_lo).y, e2, w2, c00, c01, c10, c11);
-    unsigned ofs = 0;
-#pragma unroll 4
-    for (int s = s_lo + 1; s <= s_hi; ++s) {
-        const int2 e = __ldg(ev + s);
-        const f32x2 t = bp_fetch_row<CHK, CHK>(lo0, lo1, e.y, e2, w2, c00, c01, c10, c11);
-        const float n = __int_as_float(e.x);
-        if (n >= 0.0f) {
-            const f32x2 n2 = splat2(n), s2 = splat2(sub_rn(1.0f, n));
-            float r0v, r1v;
-            unpack2(fma2(t, n2, mul2(t_prev, s2)), r0v, r1v);
-            st_stream(o0 + ofs, r0v);
-            if (!CHK || has1) st_stream(o1 + ofs, r1v);
-            ofs += plane;
-        }
-        t_prev = t;
-    }
-}
-
-// Same launch shape as the rows kernel: block = (batch item, view, chunk of planes, run of rows j); threads = column
-// pairs x sub-chunks of planes.  Blocks share nothing: the grouping only sets the dispatch order (long runs first).
-__global__ void __launch_bounds__(256)
-    backproject_forward_plan_kernel(const float *__restrict__ proj, float *__restrict__ out, const int *__restrict__ plan,
-                                    BpPlanLayout L, BpDims g) {
-    int Lb = blockIdx.x, nj = g.nj0, js = g.js0, j_base = 0;
-    if (Lb >= g.nj0 * g.n_vc) {
-        Lb -= g.nj0 * g.n_vc; nj = g.nj1; js = g.js1; j_base = g.nj0 * g.js0;
-        if (Lb >= g.nj1 * g.n_vc) { Lb -= g.nj1 * g.n_vc; nj = g.nj2; js = g.js2; j_base += g.nj1 * g.js1; }
-    }
-    const int vc = Lb / nj;
-    const int bv = vc / g.n_chunks;
-    const int bi = bv / g.n_views;
-    const int p = g.p0 + (bv - bi * g.n_views);
-    const int i_begin = (vc - bv * g.n_chunks) * g.ichunk;
-    const int i_count = min(g.ichunk, g.d - i_begin);
-    const int j_begin = j_base + (Lb - vc * nj) * js, j_end = min(g.w, j_begin + js);
-    const int ii0 = threadIdx.y * g.isub, ii1 = min(i_count, ii0 + g.isub);
-    if (ii0 >= ii1) return;
-    const int ia = g.i_off + i_begin + ii0, ib = g.i_off + i_begin + ii1;     // absolute planes [ia, ib) of this thread
-    const unsigned plane = (unsigned)(g.w * g.h);
-    const float *pv0 = proj + bi * ((int64_t)g.P * g.proj_view_stride) + (int64_t)p * g.proj_view_stride;
-    float *ob0 = out + bi * g.out_batch_stride + (int64_t)p * g.out_chan_stride + (int64_t)(i_begin + ii0) * g.w * g.h;
-    const int *rec = plan + ((int64_t)p * g.w + j_begin) * L.rec_words;
-
-    for (int j = j_begin; j < j_end; ++j, rec += L.rec_words) {
-        const int4 hdr = __ldg(reinterpret_cast<const int4 *>(rec));
-        const int2 *rowtab = reinterpret_cast<const int2 *>(rec + L.rowtab());
-        const int2 *evtab = reinterpret_cast<const int2 *>(rec + L.evtab());
-        const int2 *coltab = reinterpret_cast<const int2 *>(rec + L.coltab());
-        for (int q = threadIdx.x; q < g.hp; q += blockDim.x) {
-            const int k0 = q, k1 = q + g.hp;
-            const bool has1 = k1 < g.h;
-            const int2 t0 = __ldg(coltab + k0), t1 = __ldg(coltab + (has1 ? k1 : k0));
-            const int c0 = t0.x, c1 = t1.x;
-            const f32x2 w2 = pack2(__int_as_float(t0.y), __int_as_float(t1.y)), e2 = sub2(splat2(1.0f), w2);
-            const bool c00 = (unsigned)c0 < (unsigned)g.ph, c01 = (unsigned)(c0 + 1) < (unsigned)g.ph;
-            const bool c10 = has1 && (unsigned)c1 < (unsigned)g.ph, c11 = has1 && (unsigned)(c1 + 1) < (unsigned)g.ph;
-            float *ob = ob0 + (unsigned)(j * g.h);
-            if (hdr.y & 1) {
-                const int s_lo = __ldg(rowtab + ia).x - hdr.x, s_hi = __ldg(rowtab + ib - 1).x + 1 - hdr.x;
-                const bool rows_in = hdr.x + s_lo >= 0 && hdr.x + s_hi < g.pw;
-                const float *lo0 = opaque(pv0 + c0), *lo1 = opaque(pv0 + c1);
-                float *o0 = opaque(ob + k0), *o1 = opaque(ob + k1);
-                const bool hot = __all_sync(__activemask(), rows_in && has1 && c00 && c01 && c10 && c11);
-                if (hot) bp_march_plan<false>(evtab, s_lo, s_hi, lo0, lo1, o0, o1, plane, e2, w2, c00, c01, c10, c11, has1);
-                else bp_march_plan<true>(evtab, s_lo, s_hi, lo0, lo1, o0, o1, plane, e2, w2, c00, c01, c10, c11, has1);
-            } else {
-                float wq0, wq1, e0, e1;
-                unpack2(w2, wq0, wq1); unpack2(e2, e0, e1);
-                backproject_column_plan_checked(pv0 + c0, ob + k0, plane, rowtab, ia, ib, g.pw, g.ph, c00, c01, e0, wq0);
-                if (has1) backproject_column_plan_checked(pv0 + c1, ob + k1, plane, rowtab, ia, ib, g.pw, g.ph, c10, c11, e1, wq1);
             }
         }
     }
@@ -767,13 +584,6 @@ static int block_threads(int h) {
 // equal blocks the launch ends with every SM draining from 6 resident blocks to 0 over a whole block duration.  The
 // runs therefore taper: 4 rows, then 2, then 1.
 static dim3 forward_shape(BpDims &g, int n_views, unsigned &grid, int min_threads = 1) {
-    static int f0_env = -1, f1_env = -1;   // LIFTREG_B200_BP_TAPER="f0,f1": percent of the rows in 4-row / 2-row runs
-    if (f0_env == -1) {
-        int a = -2, b = -2;     // kernel experiments; anything that does not parse as two sane percentages is ignored
-        if (const char *e = getenv("LIFTREG_B200_BP_TAPER"))
-            if (sscanf(e, "%d,%d", &a, &b) != 2 || a < 0 || b < 0 || a + b > 100) a = b = -2;
-        f1_env = b; f0_env = a;
-    }
     g.hp = (g.h + 1) / 2;
     g.bx = g.hp > 256 ? 256 : g.hp;
     int by = LR_BP_FWD_THREADS / g.bx;
@@ -797,14 +607,11 @@ static dim3 forward_shape(BpDims &g, int n_views, unsigned &grid, int min_thread
     g.js0 = LR_BP_JS0; g.js1 = LR_BP_JS0 / 2; g.js2 = LR_BP_JS0 / 4 > 0 ? LR_BP_JS0 / 4 : 1;
     // share of the short runs: about 1.2 waves of work, at most half (measured: 50/30/20 % is best at batch 1 = 0.9
     // waves of 4-row blocks on 6 resident blocks per SM, 90/8/2 % at batch 8)
-    int f0 = f0_env, f1 = f1_env;
-    if (f0 < 0) {
-        const double waves = (double)((g.w + g.js0 - 1) / g.js0) * g.n_vc / (6.0 * sm_count());
-        double small = 1.2 / (waves > 0.1 ? waves : 0.1);
-        if (small > 0.5) small = 0.5;
-        f0 = (int)(100.0 * (1.0 - small) + 0.5);
-        f1 = (int)(100.0 * 0.6 * small + 0.5);
-    }
+    const double waves = (double)((g.w + g.js0 - 1) / g.js0) * g.n_vc / (6.0 * sm_count());
+    double small = 1.2 / (waves > 0.1 ? waves : 0.1);
+    if (small > 0.5) small = 0.5;
+    const int f0 = (int)(100.0 * (1.0 - small) + 0.5);      // percent of the rows in 4-row / 2-row runs
+    const int f1 = (int)(100.0 * 0.6 * small + 0.5);
     g.nj0 = (g.w * f0 / 100) / g.js0;
     int rest = g.w - g.nj0 * g.js0;
     g.nj1 = f0 + f1 >= 100 ? (rest + g.js1 - 1) / g.js1 : (g.w * f1 / 100) / g.js1;
@@ -813,9 +620,6 @@ static dim3 forward_shape(BpDims &g, int n_views, unsigned &grid, int min_thread
     g.nj2 = rest > 0 ? rest : 0;
     grid = (unsigned)((g.nj0 + g.nj1 + g.nj2) * g.n_vc);
     auto magic = [&](int dvs) -> unsigned {      // exact for every block index of this grid, else 0 (plain division)
-#ifdef LR_BP_NO_MAGIC
-        return 0u;
-#endif
         if (dvs <= 1 || (uint64_t)grid * (uint64_t)dvs >= (1ull << 32)) return 0u;
         return (unsigned)(((1ull << 32) + (unsigned)dvs - 1) / (unsigned)dvs);
     };
@@ -853,59 +657,6 @@ extern "C" int lr_backproject_forward_slab(const float *proj, const float *poses
         const dim3 block = forward_shape(g, np, grid, 32);
         backproject_forward_rows_kernel<<<grid, block, 0, as_stream(stream)>>>(proj, out, g, ps);
         if (int e = check_launch("backproject_forward_rows_kernel")) return e;
-    }
-    return LR_OK;
-}
-
-extern "C" size_t lr_backproject_plan_bytes(int P, int pw, int ph, int d_total, int w, int h) {
-    if (P <= 0 || pw <= 0 || ph <= 0 || d_total <= 0 || w <= 0 || h <= 0) return 0;
-    const BpPlanLayout L = plan_layout(d_total, h);
-    return sizeof(int) * (size_t)P * w * L.rec_words;
-}
-
-extern "C" int lr_backproject_plan_build(const float *poses, int P, int pw, int ph, int d_total, int w, int h, void *plan,
-                                         size_t plan_bytes, lr_stream_t stream) {
-    LR_REQUIRE(poses && plan, "backproject_plan_build: null pointer");
-    BpDims g;
-    if (int e = fill_dims(g, 1, P, pw, ph, d_total, w, h, 0, 0)) return e;
-    LR_REQUIRE(((uintptr_t)plan & 15) == 0, "backproject_plan_build: plan must be 16-byte aligned");
-    const size_t need = lr_backproject_plan_bytes(P, pw, ph, d_total, w, h);
-    if (plan_bytes < need) {
-        set_error("backproject_plan_build: plan buffer too small (%zu < %zu bytes)", plan_bytes, need);
-        return LR_ERR_WORKSPACE;
-    }
-    LR_REQUIRE(w <= 65535, "backproject_plan_build: w must be <= 65535 (grid limit)");
-    const BpPlanLayout L = plan_layout(d_total, h);
-    for (int p0 = 0; p0 < P; p0 += BP_MAX_VIEWS) {
-        const int np = P - p0 < BP_MAX_VIEWS ? P - p0 : BP_MAX_VIEWS;
-        BpPoses ps;
-        for (int q = 0; q < np; ++q)
-            for (int c = 0; c < 3; ++c) ps.s[q][c] = poses[(p0 + q) * 3 + c];
-        g.p0 = p0;
-        backproject_plan_kernel<<<dim3((unsigned)w, (unsigned)np), 256, 0, as_stream(stream)>>>((int *)plan, L, g, ps);
-        if (int e = check_launch("backproject_plan_kernel")) return e;
-    }
-    return LR_OK;
-}
-
-extern "C" int lr_backproject_forward_planned(const float *proj, const void *plan, int B, int P, int pw, int ph, int d_total,
-                                              int w, int h, int i_begin, int i_count, float *out,
-                                              int64_t out_batch_stride, int64_t out_chan_stride, lr_stream_t stream) {
-    LR_REQUIRE(proj && plan && out, "backproject_forward_planned: null pointer");
-    BpDims g;
-    if (int e = fill_dims(g, B, P, pw, ph, d_total, w, h, out_batch_stride, out_chan_stride, i_begin, i_count)) return e;
-    const int d = g.d;
-    LR_REQUIRE(out_chan_stride >= (int64_t)d * w * h, "backproject_forward_planned: out_chan_stride smaller than a volume");
-    LR_REQUIRE(((uintptr_t)plan & 15) == 0, "backproject_forward_planned: plan must be 16-byte aligned");
-    const BpPlanLayout L = plan_layout(d_total, h);
-    for (int p0 = 0; p0 < P; p0 += BP_MAX_VIEWS) {
-        const int np = P - p0 < BP_MAX_VIEWS ? P - p0 : BP_MAX_VIEWS;
-        g.p0 = p0;
-        unsigned grid;
-        LR_REQUIRE((int64_t)w * ((d + 3) / 4) * np * B < (1ll << 31), "backproject_forward_planned: too many blocks for one launch");
-        const dim3 block = forward_shape(g, np, grid);
-        backproject_forward_plan_kernel<<<grid, block, 0, as_stream(stream)>>>(proj, out, (const int *)plan, L, g);
-        if (int e = check_launch("backproject_forward_plan_kernel")) return e;
     }
     return LR_OK;
 }

@@ -377,43 +377,15 @@ __global__ void __launch_bounds__(32 * DRR_PAIRS * DRR_SEGS, LR_DRR_MINB)
     }
 }
 
-// Adjoint wrt the volume: every sample scatters (go*out_scale*dx) * w_tap into its 8 taps (RED.ADD.F32).
-__global__ void __launch_bounds__(32 * DRR_ROWS)
-    drr_backward_kernel(const float *__restrict__ gproj, float *__restrict__ gvol, DrrDims g, DrrViews views) {
-    const int v = blockIdx.x * 32 + threadIdx.x;
-    const int u = blockIdx.y * DRR_ROWS + threadIdx.y;
-    if (v >= g.rh || u >= g.rd) return;
-    const DrrView vw = views.v[blockIdx.z];
-    const Ray r = ray_setup(vw, g, u, v);
-    float *V = gvol + (int64_t)vw.vol * g.nvox;
-    const int sy = g.h, sz = g.w * g.h;
-    float go = gproj[((int64_t)(g.view0 + blockIdx.z) * g.rd + u) * g.rh + v];
-    if (g.out_scale != 1.0f) go = mul_rn(go, g.out_scale);
-    const float gs = mul_rn(go, r.dx);
-    if (gs == 0.0f) return;
-    float jf = (float)r.j0;
-    for (int j = r.j0; j <= r.j1; ++j, jf += 1.0f) {
-        const Sample s = ray_point(r, g, jf);
-        const Taps t = make_taps(s, g);
-        const unsigned m = taps_mask(t, g);
-        if (m == 0u) continue;
-        float *b = V + t.base;
-#pragma unroll
-        for (int c = 0; c < 8; ++c) {
-            const int off = (c & 1) + ((c >> 1) & 1) * sy + (c >> 2) * sz;
-            if ((m >> c) & 1u) red_add(b + off, mul_rn(t.wt[c], gs));
-        }
-    }
-}
-
-// Warp-aggregated adjoint.  The scatter above is bound by the number of atomics reaching L2 (measured: half the atomics
-// = half the time, profiles/README.md), and the 32 rays of a warp -- neighbours along detector axis 1, marching the same
+// Adjoint wrt the volume: every sample scatters (go*out_scale*dx) * w_tap into its 8 taps, warp-aggregated.  A plain
+// per-sample scatter (RED.ADD.F32) is bound by the number of atomics reaching L2 (measured: half the atomics = half the
+// time, profiles/README.md), and the 32 rays of a warp -- neighbours along detector axis 1, marching the same
 // plane j -- hit heavily overlapping cells: consecutive lanes share their floor cell or sit one cell further along the
 // volume's contiguous axis, so lane l's upper-x tap is lane l+1's lower-x tap.  Per plane the warp therefore
 //   1. sums the 8 tap values of runs of consecutive lanes with the same floor cell into the run's first lane,
 //   2. hands a run's four upper-x sums to the next run when that run's cell is the next one along x,
 // and only then issues the atomics: ~22 cells x 4 rows instead of 32 x 8 per plane at cfg 1 (2.8x fewer).  Both steps are
-// exact regroupings of the same sum (fp32 addition order differs, as it already does between runs of the scatter).
+// exact regroupings of the same sum (fp32 addition order differs, as it already does between runs of the atomics).
 __global__ void __launch_bounds__(32 * DRR_ROWS)
     drr_backward_agg_kernel(const float *__restrict__ gproj, float *__restrict__ gvol, DrrDims g, DrrViews views) {
     const unsigned FULL = 0xffffffffu;
@@ -451,14 +423,11 @@ __global__ void __launch_bounds__(32 * DRR_ROWS)
         if (__ballot_sync(FULL, m != 0u) == 0u) continue;     // no lane touches the volume on this plane
         // ---- runs of consecutive lanes with the same floor cell
         const int key_prev = __shfl_up_sync(FULL, key, 1);
-#ifndef LR_DRR_AGG_MERGE
-#define LR_DRR_AGG_MERGE 1
-#endif
-        const bool follows = LR_DRR_AGG_MERGE && lane > 0 && m != 0u && key == key_prev;
+        const bool follows = lane > 0 && m != 0u && key == key_prev;
         const unsigned long long E = (unsigned long long)__ballot_sync(FULL, follows);
         const bool leader = m != 0u && !follows;
         const int len = leader ? __ffsll((long long)~(E >> (lane + 1))) : 0;      // 1 + set bits of E right above this lane
-        const int K = LR_DRR_AGG_MERGE ? (int)__reduce_max_sync(FULL, (unsigned)(len > 0 ? len - 1 : 0)) : 0;
+        const int K = (int)__reduce_max_sync(FULL, (unsigned)(len > 0 ? len - 1 : 0));
         for (int k = 1; k <= K; ++k) {
             const bool take = leader && k < len;
 #pragma unroll
@@ -615,14 +584,8 @@ extern "C" int lr_drr_backward(const float *grad_proj, int B, int d, int w, int 
     return for_each_view_chunk(poses, n_pose_sets, B, P, [&](int n, const DrrViews &vs, int v0) {
         g.view0 = v0;
         dim3 grid((unsigned)((rh + 31) / 32), (unsigned)((rd + DRR_ROWS - 1) / DRR_ROWS), (unsigned)n);
-        // LIFTREG_B200_DRR_BWD_AGG=0 selects the plain per-sample scatter
-        static const bool agg = [] { const char *e = getenv("LIFTREG_B200_DRR_BWD_AGG"); return !(e && e[0] == '0'); }();
-        if (agg) {
-            drr_backward_agg_kernel<<<grid, dim3(32, DRR_ROWS), 0, as_stream(stream)>>>(grad_proj, grad_vol, g, vs);
-            return check_launch("drr_backward_agg_kernel");
-        }
-        drr_backward_kernel<<<grid, dim3(32, DRR_ROWS), 0, as_stream(stream)>>>(grad_proj, grad_vol, g, vs);
-        return check_launch("drr_backward_kernel");
+        drr_backward_agg_kernel<<<grid, dim3(32, DRR_ROWS), 0, as_stream(stream)>>>(grad_proj, grad_vol, g, vs);
+        return check_launch("drr_backward_agg_kernel");
     });
 }
 

@@ -6,8 +6,7 @@
 //     ncc = mean(a*b) / sqrt(mean(a^2) * mean(b^2)),   loss = 1 - mean_over_batch(ncc)
 // The reference runs ~10 elementwise / reduction kernels over the two volumes (each re-reading 16 MB per item at 160^3);
 // here the forward is ONE pass over x and y (raw moments about the item's first voxel, rewritten into the centred ones by a
-// B-thread kernel; the two-pass op-for-op form -- sums, then fp32-centred second moments -- stays behind
-// LIFTREG_B200_NCC_TWO_PASS=1) and the backward is one pass.  Per-thread partial sums are fp32 over a handful of elements, everything above that
+// B-thread kernel) and the backward is one pass.  Per-thread partial sums are fp32 over a handful of elements, everything above that
 // is accumulated in fp64 (warp shuffles, shared memory, one fp64 atomic per block), so the result does not depend on the launch shape
 // beyond fp64 round-off.
 #include "common.cuh"
@@ -43,47 +42,18 @@ __device__ __forceinline__ void block_accumulate(const float (&v)[NV], double *_
     }
 }
 
-// pass 1: sums[b][0..1] += sum x, sum y
-__global__ void __launch_bounds__(NCC_THREADS) ncc_sum_kernel(const float *__restrict__ x, const float *__restrict__ y, int64_t N,
-                                                              double *__restrict__ sums) {
-    const int b = blockIdx.y;
-    const float *xb = x + (int64_t)b * N, *yb = y + (int64_t)b * N;
-    float sx = 0.0f, sy = 0.0f;
-    for (int64_t i = (int64_t)blockIdx.x * NCC_THREADS + threadIdx.x; i < N; i += (int64_t)gridDim.x * NCC_THREADS) {
-        sx += ld_stream(xb + i);
-        sy += ld_stream(yb + i);
-    }
-    const float v[2] = {sx, sy};
-    block_accumulate<2>(v, sums + b * NCC_SUMS);
-}
-
 // the centred values exactly as the reference forms them in fp32 (losses.py:21-22): (x - mean) + 1e-10
 __device__ __forceinline__ float centred(float v, float mean) { return add_rn(sub_rn(v, mean), 1e-10f); }
 
-// pass 2: sums[b][2..6] += sum a*b, a*a, b*b, a, b
-__global__ void __launch_bounds__(NCC_THREADS) ncc_moment_kernel(const float *__restrict__ x, const float *__restrict__ y, int64_t N,
-                                                                 double *__restrict__ sums) {
-    const int b = blockIdx.y;
-    const float *xb = x + (int64_t)b * N, *yb = y + (int64_t)b * N;
-    const float mx = (float)(sums[b * NCC_SUMS + 0] / (double)N), my = (float)(sums[b * NCC_SUMS + 1] / (double)N);
-    float sab = 0.0f, saa = 0.0f, sbb = 0.0f, sa = 0.0f, sb = 0.0f;
-    for (int64_t i = (int64_t)blockIdx.x * NCC_THREADS + threadIdx.x; i < N; i += (int64_t)gridDim.x * NCC_THREADS) {
-        const float a = centred(__ldg(xb + i), mx), c = centred(__ldg(yb + i), my);
-        sab = fmaf(a, c, sab); saa = fmaf(a, a, saa); sbb = fmaf(c, c, sbb);
-        sa += a; sb += c;
-    }
-    const float v[5] = {sab, saa, sbb, sa, sb};
-    block_accumulate<5>(v, sums + b * NCC_SUMS + 2);
-}
-
-// Single-pass forward.  The centring needs the means, which is why the restatement above reads x and y twice; but with
+// Single-pass forward.  The centring needs the means, which is why the reference reads x and y twice; but with
 // u = x - k, v = y - l for ANY constants k, l the centred moments follow from the raw moments of u and v:
 //     a = x - mean + eps = u - dx  (dx = mean - k - eps)   =>   sum a*a = sum u*u - 2 dx sum u + N dx^2, etc.
 // and the cancellation in these differences is mild when k, l lie within a few standard deviations of the means.  k and l are
 // the item's first voxels (every thread reads them); per-thread fp32 partials over a few elements, everything above in fp64
 // as before; a B-thread kernel then rewrites the five raw sums into the seven-entry layout the backward and the host use.
-// What is not reproduced is the reference's fp32 rounding of each (x - mean) + 1e-10 (the 1e-10 is below half an ulp of all
-// but the elements within 1e-3 of the mean): the loss differs from the two-pass kernels by ~1e-8.
+// What is not reproduced is the fp32 rounding of each (x - mean) + 1e-10 that the reference's op-for-op form performs
+// (oracle/torch_port.ncc_loss; the 1e-10 is below half an ulp of all but the elements within 1e-3 of the mean): that
+// rounding moves the loss by ~1e-8.
 __global__ void __launch_bounds__(NCC_THREADS) ncc_shifted_kernel(const float *__restrict__ x, const float *__restrict__ y, int64_t N,
                                                                   double *__restrict__ sums) {
     const int b = blockIdx.y;
@@ -498,10 +468,9 @@ static unsigned ncc_blocks(int64_t N, int B) {
     return (unsigned)(want < 1 ? 1 : want);
 }
 
-// the pair kernels need an even row length and 8-byte-aligned rows (LIFTREG_B200_REG_PAIRS=0 forces the scalar kernels)
+// the pair kernels need an even row length and 8-byte-aligned rows
 static bool reg_use_pairs(const void *a, const void *b, int W) {
-    static const bool enabled = [] { const char *e = getenv("LIFTREG_B200_REG_PAIRS"); return !(e && e[0] == '0'); }();
-    return enabled && (W % 2 == 0) && ((uintptr_t)a % 8 == 0) && ((uintptr_t)b % 8 == 0);
+    return (W % 2 == 0) && ((uintptr_t)a % 8 == 0) && ((uintptr_t)b % 8 == 0);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -791,18 +760,10 @@ extern "C" int lr_ncc_sums(const float *x, const float *y, int B, int64_t N, dou
     cudaError_t ce = cudaMemsetAsync(sums, 0, sizeof(double) * NCC_SUMS * (size_t)B, st);
     if (ce != cudaSuccess) { set_error("ncc_sums: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
     const dim3 grid(ncc_blocks(N, B), (unsigned)B);
-    // LIFTREG_B200_NCC_TWO_PASS=1: the op-for-op restatement (means first, then the fp32-centred moments)
-    static const bool two_pass = [] { const char *e = getenv("LIFTREG_B200_NCC_TWO_PASS"); return e && e[0] == '1'; }();
-    if (!two_pass) {
-        ncc_shifted_kernel<<<grid, NCC_THREADS, 0, st>>>(x, y, N, sums);
-        if (int e = check_launch("ncc_shifted_kernel")) return e;
-        ncc_finalize_kernel<<<(B + 127) / 128, 128, 0, st>>>(x, y, N, B, sums);
-        return check_launch("ncc_finalize_kernel");
-    }
-    ncc_sum_kernel<<<grid, NCC_THREADS, 0, st>>>(x, y, N, sums);
-    if (int e = check_launch("ncc_sum_kernel")) return e;
-    ncc_moment_kernel<<<grid, NCC_THREADS, 0, st>>>(x, y, N, sums);
-    return check_launch("ncc_moment_kernel");
+    ncc_shifted_kernel<<<grid, NCC_THREADS, 0, st>>>(x, y, N, sums);
+    if (int e = check_launch("ncc_shifted_kernel")) return e;
+    ncc_finalize_kernel<<<(B + 127) / 128, 128, 0, st>>>(x, y, N, B, sums);
+    return check_launch("ncc_finalize_kernel");
 }
 
 extern "C" int lr_ncc_backward(const float *x, const float *y, int B, int64_t N, const double *sums, const float *grad_loss,

@@ -12,8 +12,6 @@
 // batch's coefficients sit in shared memory as [k][b] and are read four batch items at a time (LDS.128 broadcast).
 // Accumulation is a sequential fp32 FMA chain over k (ascending), then + mean, then (optionally) + identity -- the
 // order the oracle restates.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace lr {
@@ -397,18 +395,13 @@ __global__ void __launch_bounds__(PD_ROWS)
     }
 }
 
-static bool pca_tma_enabled() {      // LIFTREG_B200_PCA_TMA=0: kernel experiments (the padded staging kernel)
-    static int v = -1;
-    if (v < 0) { const char *e = getenv("LIFTREG_B200_PCA_TMA"); v = (e && e[0] == '0') ? 0 : 1; }
-    return v != 0;
-}
 static int gcd_int(int a, int b) { return b == 0 ? a : gcd_int(b, a % b); }
 
 template <int BT>
 static int launch_pca(const float *coefs, const float *basis, const float *mean, float *out, const PcaDims &g,
                       cudaStream_t st) {
     const bool vec = g.K % 4 == 0 && ((uintptr_t)basis & 15) == 0;
-    if (vec && pca_tma_enabled() && gcd_int(g.K / 4, 8) <= 2) {
+    if (vec && gcd_int(g.K / 4, 8) <= 2) {
         // + 4 floats: the compiler reads the coefficient table four at a time in the k-loop's remainder iterations
         const size_t smem_t = sizeof(float) * ((size_t)PT_STAGES * PT_ROWS * g.K + (size_t)g.K * BT + 4);
         if (smem_t <= 110 * 1024) {
@@ -521,7 +514,7 @@ __global__ void __launch_bounds__(PT_ROWS)
 
 template <int BT>
 static int launch_pca_bwd(const float *gout, const float *basis, float *gcoefs, const PcaDims &g, cudaStream_t st) {
-    if (pca_tma_enabled() && g.K % 4 == 0 && ((uintptr_t)basis & 15) == 0 && g.N % 4 == 0 && ((uintptr_t)gout & 15) == 0 && g.K <= PT_ROWS) {
+    if (g.K % 4 == 0 && ((uintptr_t)basis & 15) == 0 && g.N % 4 == 0 && ((uintptr_t)gout & 15) == 0 && g.K <= PT_ROWS) {
         const size_t smem_t = sizeof(float) * (size_t)PT_STAGES * ((size_t)PT_ROWS * g.K + (size_t)BT * PT_ROWS);
         if (smem_t <= 110 * 1024) {
             static thread_local bool attr_done = false;

@@ -8,9 +8,6 @@
 // local gather served by L1/L2.  Arithmetic follows ATen's CPU grid_sampler_3d exactly: unnormalise
 // ((g+1)/2)*(S-1), weights (x1-x)*(y1-y)*(z1-z) left to right, taps accumulated in the order
 // tnw,tne,tsw,tse,bnw,bne,bsw,bse with separately rounded multiply and add.
-#include <cstdio>
-#include <cstdlib>
-
 #include "common.cuh"
 
 // resident blocks per SM the two packed kernels are compiled for (register cap = 65536 / (32 * WARP_TY * n))
@@ -748,13 +745,6 @@ static dim3 warp_grid(int nb, int D, int H, int W, int rows_per_thread = 1) {
 // into 4- and 2-plane blocks that are dispatched last (per batch item) and fill the tail.  The short blocks' share is about 1.2 waves of
 // work, at most 45 % (measured: 55/27/18 % is best at batch 1 = 1.7 waves, 100/0/0 at batch 8 = 13.5 waves).
 static void forward_z_blocking(WarpDims &g, int n_batch, double resident_blocks = 4.0, double max_small = 0.45) {
-    static int f0_env = -1, f1_env = -1;        // LIFTREG_B200_WARP_TAPER="f0,f1": percent of the planes in 8- / 4-plane blocks
-    if (f0_env == -1) {
-        int a = -2, b = -2;     // kernel experiments; anything that does not parse as two sane percentages is ignored
-        if (const char *e = getenv("LIFTREG_B200_WARP_TAPER"))
-            if (sscanf(e, "%d,%d", &a, &b) != 2 || a < 0 || b < 0 || a + b > 100) a = b = -2;
-        f1_env = b; f0_env = a;
-    }
     const int Do = g.Do;
     g.zs0 = WARP_NZ_MAX; g.zs1 = 4; g.zs2 = 2;
     if (Do < 32) {
@@ -762,15 +752,12 @@ static void forward_z_blocking(WarpDims &g, int n_batch, double resident_blocks 
         g.zn0 = (Do + WARP_NZ - 1) / WARP_NZ; g.zn1 = 0;
         g.zblocks = g.zn0;
     } else {
-        int f0 = f0_env, f1 = f1_env;
-        if (f0 < 0) {
-            const double tiles = (double)((g.W + WARP_TX - 1) / WARP_TX) * ((g.H + WARP_TY * WARP_VY - 1) / (WARP_TY * WARP_VY));
-            const double waves = tiles * n_batch * ((Do + g.zs0 - 1) / g.zs0) / (resident_blocks * sm_count());   // (tuned with these counts)
-            double small = 1.2 / (waves > 0.1 ? waves : 0.1);
-            if (small > max_small) small = max_small;
-            f0 = (int)(100.0 * (1.0 - small) + 0.5);
-            f1 = (int)(100.0 * 0.6 * small + 0.5);
-        }
+        const double tiles = (double)((g.W + WARP_TX - 1) / WARP_TX) * ((g.H + WARP_TY * WARP_VY - 1) / (WARP_TY * WARP_VY));
+        const double waves = tiles * n_batch * ((Do + g.zs0 - 1) / g.zs0) / (resident_blocks * sm_count());   // (tuned with these counts)
+        double small = 1.2 / (waves > 0.1 ? waves : 0.1);
+        if (small > max_small) small = max_small;
+        const int f0 = (int)(100.0 * (1.0 - small) + 0.5);      // percent of the planes in 8- / 4-plane blocks
+        const int f1 = (int)(100.0 * 0.6 * small + 0.5);
         g.zn0 = (Do * f0 / 100) / g.zs0;
         const int rest = Do - g.zn0 * g.zs0;
         g.zn1 = f0 + f1 >= 100 ? (rest + g.zs1 - 1) / g.zs1 : (Do * f1 / 100) / g.zs1;

@@ -162,38 +162,6 @@ def project_grid(poses, resolution, obj_shape, spacing, device, y_norm_mode=YNOR
 
 
 # --------------------------------------------------------------------------- backprojection
-_PLAN_CACHE = {}          # geometry -> device plan buffer (insertion-ordered; a handful of geometries per process)
-_PLAN_CACHE_MAX = 8
-
-
-def backproject_plan(poses, proj_shape, img_shape, device):
-    """Device buffer holding the geometry plan of lr_backproject_forward_planned for (poses, proj_shape, img_shape),
-    built once per geometry and cached -- the counterpart of the reference caching its sample grid on the first
-    batch (LiftRegDeformSubspaceBackproj.py:85-87).  poses: (P,3) float32.  (Measured slower than rebuilding the
-    tables in shared memory -- backproject() does not use it; kept as a tested entry point.)"""
-    poses = _poses32(poses)
-    P = poses.shape[0]
-    pw, ph = (int(s) for s in proj_shape)
-    d, w, h = (int(s) for s in img_shape)
-    dev = torch.device(device)
-    key = (poses.tobytes(), P, pw, ph, d, w, h, dev.index if dev.index is not None else torch.cuda.current_device())
-    plan = _PLAN_CACHE.get(key)
-    if plan is None:
-        lib = _native.lib()
-        nbytes = lib.lr_backproject_plan_bytes(P, pw, ph, d, w, h)
-        if nbytes == 0:
-            raise ValueError("bad backprojection geometry %r" % ((P, pw, ph, d, w, h),))
-        plan = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        with torch.cuda.device(dev):
-            _native.check(lib.lr_backproject_plan_build(_fp(poses), P, pw, ph, d, w, h, _ptr(plan), nbytes, _stream()),
-                          "lr_backproject_plan_build")
-            torch.cuda.current_stream().synchronize()      # once per geometry: later calls may come from any stream
-        while len(_PLAN_CACHE) >= _PLAN_CACHE_MAX:
-            _PLAN_CACHE.pop(next(iter(_PLAN_CACHE)))
-        _PLAN_CACHE[key] = plan
-    return plan
-
-
 class _Backproject(torch.autograd.Function):
     @staticmethod
     def forward(ctx, proj, poses, d_total, w, h, out, channel_offset, i_begin, i_count):

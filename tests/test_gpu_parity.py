@@ -756,7 +756,8 @@ def test_atten_coef_vector_and_tail_paths_bit_exact(dev, n, offset):
 
 # ------------------------------------------------------------------ PCA-subspace decode (row f2)
 @pytest.mark.parametrize("B,K,shape", [(1, 56, (6, 5, 7)), (3, 56, (20, 24, 28)), (8, 8, (4, 4, 4)), (33, 60, (5, 6, 7)), (2, 4, (3, 3, 3)),
-                                       (2, 3, (9, 8, 7)), (5, 57, (12, 10, 11)), (1, 1, (2, 2, 2))])
+                                       (2, 3, (9, 8, 7)), (5, 57, (12, 10, 11)), (1, 1, (2, 2, 2)),
+                                       (2, 16, (5, 6, 7)), (1, 160, (4, 5, 6))])       # K = 16, 160: the padded staging kernel
 def test_pca_decode_exact_vs_oracle(dev, B, K, shape):
     from liftreg_b200 import ops
     from oracle import c_oracle
@@ -1047,13 +1048,13 @@ def test_label_warp_mirror_of_mermaid_entry_point(dev):
     assert rel_l2(out01.cpu().numpy(), lin.cpu().numpy()) <= 1e-4       # coordinates round-trip through [0, 1] in fp32
 
 
-# ------------------------------------------------------------------ geometry plan
+# ------------------------------------------------------------------ backprojection rows kernel
 @pytest.mark.parametrize("shape,pshape,B,P", [((160, 160, 160), (256, 256), 1, 4), ((33, 6, 70), (40, 31), 3, 2),
                                               ((40, 9, 300), (64, 350), 1, 2), ((5, 7, 3), (9, 4), 2, 66), ((64, 48, 33), (20, 300), 1, 3)])
-def test_backproject_planned_equals_unplanned(dev, shape, pshape, B, P):
-    """lr_backproject_forward_planned (cached geometry tables) against
-    lr_backproject_forward (tables rebuilt in the kernel) in fast numerics: bit-identical, for the whole volume, for an
-    unaligned z-slab and through channel strides -- and both equal the oracle's fast blend order."""
+def test_backproject_rows_kernel_strided_slab_and_dense_agree(dev, shape, pshape, B, P):
+    """lr_backproject_forward (the rows kernel, fast numerics) into channels 1..P of a wider buffer, into a dense
+    buffer and, through lr_backproject_forward_slab, into an unaligned z-slab: bit-identical, the sentinel channels
+    untouched -- and equal to the oracle's fast blend order and to ops.backproject."""
     import ctypes
     from liftreg_b200 import _native, ops, synthetic
     from oracle import c_oracle
@@ -1070,18 +1071,17 @@ def test_backproject_planned_equals_unplanned(dev, shape, pshape, B, P):
         vp = lambda t: ctypes.c_void_p(t.data_ptr())
         nv = d * w * h
         ref = torch.empty((B, P, d, w, h), device=dev)
-        _native.check(lib.lr_backproject_forward(vp(tp), ops._fp(poses), B, P, pshape[0], pshape[1], d, w, h, vp(ref), P * nv, nv, st), "unplanned")
-        plan = ops.backproject_plan(poses, pshape, shape, dev)
+        _native.check(lib.lr_backproject_forward(vp(tp), ops._fp(poses), B, P, pshape[0], pshape[1], d, w, h, vp(ref), P * nv, nv, st), "dense")
         out = torch.full((B, P + 2, d, w, h), 3.0, device=dev)            # channels 1..P of a wider buffer
         view = out[:, 1:1 + P]
-        _native.check(lib.lr_backproject_forward_planned(vp(tp), vp(plan), B, P, pshape[0], pshape[1], d, w, h, 0, d,
-                                                         ctypes.c_void_p(view.data_ptr()), (P + 2) * nv, nv, st), "planned")
+        _native.check(lib.lr_backproject_forward(vp(tp), ops._fp(poses), B, P, pshape[0], pshape[1], d, w, h,
+                                                 ctypes.c_void_p(view.data_ptr()), (P + 2) * nv, nv, st), "strided")
         assert torch.equal(view, ref) and bool((out[:, 0] == 3.0).all()) and bool((out[:, -1] == 3.0).all())
         if d >= 5:
             z0, nz = d // 3, max(1, d // 2 - 1)
             slab = torch.empty((B, P, nz, w, h), device=dev)
-            _native.check(lib.lr_backproject_forward_planned(vp(tp), vp(plan), B, P, pshape[0], pshape[1], d, w, h, z0, nz,
-                                                             vp(slab), P * nz * w * h, nz * w * h, st), "planned slab")
+            _native.check(lib.lr_backproject_forward_slab(vp(tp), ops._fp(poses), B, P, pshape[0], pshape[1], d, w, h, z0, nz,
+                                                          vp(slab), P * nz * w * h, nz * w * h, st), "slab")
             assert torch.equal(slab, ref[:, :, z0:z0 + nz])
         if nv * B * P <= 4_000_000:
             prev_blend = c_oracle.set_blend("fast")
@@ -1090,6 +1090,5 @@ def test_backproject_planned_equals_unplanned(dev, shape, pshape, B, P):
             finally:
                 c_oracle.set_blend(prev_blend)
         assert torch.equal(ops.backproject(tp, poses, shape), ref)
-        assert ops.backproject_plan(poses, pshape, shape, dev).data_ptr() == plan.data_ptr()       # cached per geometry
     finally:
         _native.set_numerics(prev)

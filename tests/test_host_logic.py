@@ -216,12 +216,3 @@ def test_numerics_mode_is_settable_without_a_gpu_and_rejects_bad_values():
     finally:
         _native.set_numerics(prev)
 
-
-def test_backproject_plan_size_and_argument_checks_without_a_gpu():
-    from liftreg_b200 import _native
-    lib = _native.lib()
-    n = lib.lr_backproject_plan_bytes(4, 256, 256, 160, 160, 160)
-    # one record per (view, row): header + rowtab[d] + evtab[3d+8] + coltab[h], 8 bytes per entry, 16-byte aligned
-    rec_words = (4 + 2 * 160 + 2 * (3 * 160 + 8) + 2 * 160 + 3) // 4 * 4
-    assert n == 4 * 160 * rec_words * 4
-    assert lib.lr_backproject_plan_bytes(0, 256, 256, 160, 160, 160) == 0

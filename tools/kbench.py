@@ -56,12 +56,6 @@ def main():
         _native.check(lib.lr_backproject_forward(vp(s["proj"]), ops._fp(poses32), batch, P, DET[0], DET[1], *VOL, vp(s["lifted"]),
                                                  P * nv, nv, st), "backproject")
 
-    bp_plan = ops.backproject_plan(poses32, DET, VOL, dev)
-
-    def k_backproject_planned(s, st):
-        _native.check(lib.lr_backproject_forward_planned(vp(s["proj"]), vp(bp_plan), batch, P, DET[0], DET[1], *VOL, 0, VOL[0], vp(s["lifted"]),
-                                                         P * nv, nv, st), "backproject_planned")
-
     def k_drr(s, st):
         _native.check(lib.lr_drr_forward(vp(s["mu"]), 1, *VOL, ops._dp(p64), 1, P, 240, 240, ops._fp(sp3), 0,
                                          ctypes.c_float(0.1), vp(s["drr"]), st), "drr")
@@ -157,7 +151,6 @@ def main():
              "labels2": (k_labels(2), nv, 8 * nv), "labels6": (k_labels(6), nv, 8 * nv), "reg_bwd": (k_reg_bwd, nv, 24 * nv), "ncc": (k_ncc, nv, 8 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
              "pca_bwd": (k_pca_bwd, 3 * nv, 4 * 3 * nv * 56 + 4 * 3 * nv), "warp_bwd": (k_warp_bwd, nv, 32 * nv),
              "drr_bwd": (k_drr_bwd, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240), "backproject": (k_backproject, batch * P * nv, batch * (4 * P * nv + 4 * P * DET[0] * DET[1])),
-             "backproject_planned": (k_backproject_planned, batch * P * nv, batch * (4 * P * nv + 4 * P * DET[0] * DET[1])),
              "drr": (k_drr, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240),
              "drr256": (k_drr256, P * 256 * 256 * VOL[1], 4 * nv + 4 * P * 256 * 256)}
     for name in which:
