@@ -321,6 +321,21 @@ LR_API int lr_jacobian_det(const float *phi, int B, int D, int H, int W, int bou
 LR_API int lr_label_confusion(const float *pred, const float *target, int B, int64_t N, int L,
                               int64_t *counts, int64_t *invalid, lr_stream_t stream);
 
+/* ---- folding penalty (a training term; PARITY UNPINNED: the reference has no such term) ----------------------------
+ *   fold(phi) = 1/(B*D*H*W) * sum_b sum_v max(0, -det_b(v))
+ * det is, bit for bit, the determinant lr_jacobian_det computes for the same phi and boundary, over every voxel (no
+ * margin).  A voxel whose det is not finite contributes nothing, to the value or to the gradient (as in the
+ * statistics).  The subgradient is taken over the strict fold set det < 0 (the voxels stats[:,0] counts), so det == 0
+ * contributes 0.  The value needs no kernel of its own: fold = sum_b stats[b][1] / (B*D*H*W) with the stats of
+ * lr_jacobian_det(phi, ..., margin = 0, det = NULL, ...).
+ * lr_jacobian_fold_backward: grad_phi (B,3,D,H,W) is OVERWRITTEN with grad_loss[0] * d fold / d phi (grad_loss: one
+ * float in device memory).  With J[c][a] = s_a * (D_a phi_c), C[c][a] = d det / d J[c][a] and m = 1 where det is finite
+ * and < 0 (0 elsewhere):  grad_phi_c = -(grad_loss / (B*D*H*W)) * sum_a s_a * D_a^T (m * C[c][a]), D_a^T the transpose
+ * of the difference operator with its face rows.  Each element is written once, without atomics, so repeated calls
+ * give the same bits.  Same argument rules as lr_jacobian_det (D,H,W >= 2, B*3*D*H*W < 2^31). */
+LR_API int lr_jacobian_fold_backward(const float *phi, int B, int D, int H, int W, int boundary,
+                                     const float *grad_loss, float *grad_phi, lr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -61,6 +61,7 @@ SIGNATURES = {
     "lr_diffusion_reg_sum": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp]),
     "lr_diffusion_reg_backward": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "lr_jacobian_det": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "lr_jacobian_fold_backward": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "lr_label_confusion": (_i, [_vp, _vp, _i, _i64, _i, _vp, _vp, _vp]),
 }
 

@@ -437,9 +437,10 @@ __global__ void __launch_bounds__(NCC_THREADS, LR_REGP_BWD_MINB) diffusion_reg_b
     }
 }
 
+// Plane-march launch shape of a kernel whose block of `threads` threads owns a tile_w x tile_h tile of (last, second)
+// axis positions: the per-axis scales, the chunking of the first axis and the grid.
 template <typename K>
-static int reg_dims(K kernel, bool pairs, int waves, int B, int D, int H, int W, RegDims &g, dim3 &grid) {
-    const int tile_w = pairs ? 2 * REGP_TX : REG_TX, tile_h = pairs ? REGP_TY : REG_TY;
+static int march_dims(K kernel, int threads, int tile_w, int tile_h, int waves, int B, int D, int H, int W, RegDims &g, dim3 &grid) {
     g.d = D; g.h = H; g.w = W;
     const double sp[3] = {1.0 / (double)(D - 1) * 2.0, 1.0 / (double)(H - 1) * 2.0, 1.0 / (double)(W - 1) * 2.0};   // spacing*2 (:53-54)
     g.sd = (float)(0.5 / sp[0]); g.sh = (float)(0.5 / sp[1]); g.sw = (float)(0.5 / sp[2]);
@@ -447,7 +448,7 @@ static int reg_dims(K kernel, bool pairs, int waves, int B, int D, int H, int W,
     // ONE wave of blocks when the tiles allow it (a second, nearly empty wave would double the time of this short
     // kernel): as many chunks of planes as fit the resident-block capacity, chunks of at least 4 planes
     int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, NCC_THREADS, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
     const int64_t capacity = (int64_t)sm_count() * per_sm * waves;
     int64_t chunks = capacity / tiles;
     if (chunks < 1) chunks = 1;
@@ -459,6 +460,11 @@ static int reg_dims(K kernel, bool pairs, int waves, int B, int D, int H, int W,
     if ((int64_t)B * 3 * D * H * W >= ((int64_t)1 << 31)) return -1;          // the kernels index with 32 bits
     grid = dim3((unsigned)((W + tile_w - 1) / tile_w), (unsigned)((H + tile_h - 1) / tile_h), (unsigned)gz);
     return 0;
+}
+
+template <typename K>
+static int reg_dims(K kernel, bool pairs, int waves, int B, int D, int H, int W, RegDims &g, dim3 &grid) {
+    return march_dims(kernel, NCC_THREADS, pairs ? 2 * REGP_TX : REG_TX, pairs ? REGP_TY : REG_TY, waves, B, D, H, W, g, grid);
 }
 
 static unsigned ncc_blocks(int64_t N, int B) {
@@ -678,6 +684,145 @@ __global__ void __launch_bounds__(NCC_THREADS, LR_REGP_MINB) jacobian_det_pair_k
     jac_block_flush(acc, stats + b * JAC_STATS);
 }
 
+// ---- d fold / d phi, fold = 1/(B*D*H*W) * sum over voxels of max(0, -det) (include/liftreg_b200.h) -----------------
+// With G[c][a](u) = m(u) * C[c][a](u), C the cofactor d det / d J[c][a] and m(u) = 1 where det(u) is finite and < 0:
+//     d fold / d phi_c = -(1/(B*D*H*W)) * sum_a s_a * D_a^T G[c][a]
+// where D_a is the regulariser's difference operator along axis a (see fd_adjoint for its transpose).  Voxel v needs
+// G[.][a] at v - e_a and v + e_a (and at v itself on the faces), so G is computed once per voxel and shared:
+//   first axis  (a = 0): the block marches planes; G[.][0] of planes z-1, z, z+1 rolls through registers;
+//   second axis (a = 1): the warps of a block are 16 consecutive rows; G[.][1] of the plane goes through shared memory;
+//   last axis   (a = 2): a warp is 32 consecutive voxels of a row; G[.][2] comes from the neighbouring lanes.
+// The outermost lanes and warps compute the halo (G of the voxels next to the tile), so a block writes the 30 x 14
+// voxels of lanes 1..30 of warps 1..14: each output element is written once, by one thread, with no atomics.
+constexpr int FOLD_WARPS = 16, FOLD_THREADS = 32 * FOLD_WARPS;
+constexpr int FOLD_OX = 30, FOLD_OY = FOLD_WARPS - 2;
+
+// J of the thread's column at plane z (the march and differences of jacobian_det_kernel, so det is bit for bit the
+// forward's), then G = m * C; advances the plane window (vm, vc) by one plane
+template <int MODE>
+__device__ __forceinline__ void fold_cofactors(const float *__restrict__ phi, const RegDims &g, unsigned i0, unsigned cs, unsigned pl,
+                                               int z, int oxu, int oxd, int oyu, int oyd, bool xlo, bool xhi, bool ylo, bool yhi,
+                                               bool inside, float (&vm)[3], float (&vc)[3], float (&G)[3][3]) {
+    const bool zlo = z == 0, zhi = z == g.d - 1;
+    float j[3][3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const unsigned ic = i0 + c * cs;
+        const float cc = vc[c];
+        const float vp = zhi ? cc : __ldg(phi + (ic + pl));
+        if (LR_REG_PF > 0 && z + LR_REG_PF < g.d) prefetch_l2(phi + (ic + LR_REG_PF * pl));
+        const float yu = __ldg(phi + (ic + oyu)), yd = __ldg(phi + (ic + oyd));
+        const float xu = __ldg(phi + (ic + oxu)), xd = __ldg(phi + (ic + oxd));
+        j[c][0] = mul_rn(fd_delta<MODE>(vp, vm[c], cc, zlo, zhi), g.sd);
+        j[c][1] = mul_rn(fd_delta<MODE>(yu, yd, cc, ylo, yhi), g.sh);
+        j[c][2] = mul_rn(fd_delta<MODE>(xu, xd, cc, xlo, xhi), g.sw);
+        vm[c] = cc; vc[c] = vp;
+    }
+    const float det = det3(j);
+    const bool fold = inside && det < 0.0f && isfinite(det);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            const int c1 = (c + 1) % 3, c2 = (c + 2) % 3, a1 = (a + 1) % 3, a2 = (a + 2) % 3;
+            const float C = sub_rn(mul_rn(j[c1][a1], j[c2][a2]), mul_rn(j[c1][a2], j[c2][a1]));
+            G[c][a] = fold ? C : 0.0f;
+        }
+    }
+}
+
+// (D^T G)(v) along one axis from G at v - e, v, v + e, for v at index i of n: interior G(v-e) - G(v+e); in linear mode
+// rows 0 and n-1 of D enter with +-2 (fd_adjoint), in neumann_zero mode they are zero.  Terms outside the axis are
+// selected away, never multiplied by zero, so a non-finite value there cannot leak in.
+template <int MODE>
+__device__ __forceinline__ float fold_adjoint(float gm, float g0, float gp, int i, int n) {
+    float t = 0.0f;
+    if (i >= 2) t = gm;
+    else if (MODE == 0 && i == 1) t = 2.0f * gm;
+    if (i <= n - 3) t = sub_rn(t, gp);
+    else if (MODE == 0 && i == n - 2) t = sub_rn(t, 2.0f * gp);
+    if (MODE == 0 && i == 0) t = sub_rn(t, 2.0f * g0);
+    if (MODE == 0 && i == n - 1) t = add_rn(t, 2.0f * g0);
+    return t;
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(FOLD_THREADS) jacobian_fold_backward_kernel(const float *__restrict__ phi, RegDims g, int B,
+                                                                              const float *__restrict__ grad_loss,
+                                                                              float *__restrict__ grad_phi) {
+    __shared__ float g1s[2][3][FOLD_WARPS][32];       // G[.][1] of one plane, double-buffered over planes
+    const int lane = threadIdx.x & 31, wy = threadIdx.x >> 5;
+    const int x = blockIdx.x * FOLD_OX - 1 + lane, y = blockIdx.y * FOLD_OY - 1 + wy;
+    const int zc = blockIdx.z % g.n_zchunks, b = blockIdx.z / g.n_zchunks;
+    const int z0 = zc * g.zchunk, z1 = min(g.d, z0 + g.zchunk);
+    const bool inside = x >= 0 && x < g.w && y >= 0 && y < g.h;
+    const bool writer = inside && lane >= 1 && lane <= FOLD_OX && wy >= 1 && wy <= FOLD_OY;
+    // halo threads outside the volume run the march on the nearest voxel (in-bounds loads) and contribute G = 0
+    const int xc = min(max(x, 0), g.w - 1), yc = min(max(y, 0), g.h - 1);
+    const bool xlo = xc == 0, xhi = xc == g.w - 1, ylo = yc == 0, yhi = yc == g.h - 1;
+    const int oxu = xhi ? 0 : 1, oxd = xlo ? 0 : -1;
+    const int oyu = yhi ? 0 : g.w, oyd = ylo ? 0 : -g.w;
+    const unsigned pl = (unsigned)(g.h * g.w), cs = pl * (unsigned)g.d;       // 32-bit indices (B*3*D*H*W < 2^31)
+    const unsigned col = (unsigned)yc * (unsigned)g.w + (unsigned)xc, item = (unsigned)b * 3u * (unsigned)g.d * pl;
+    const float k = (float)((double)grad_loss[0] / ((double)B * (double)g.d * (double)pl));
+    const float kd = -k * g.sd, kh = -k * g.sh, kw = -k * g.sw;
+
+    // prologue: G[.][0] of plane z0-1 and all of G at plane z0
+    const int zs = z0 > 0 ? z0 - 1 : 0;
+    float vm[3], vc[3], Gc[3][3], g0m[3] = {0.0f, 0.0f, 0.0f};
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        vc[c] = __ldg(phi + (item + c * cs + (unsigned)zs * pl + col));
+        vm[c] = zs > 0 ? __ldg(phi + (item + c * cs + (unsigned)(zs - 1) * pl + col)) : vc[c];
+    }
+    if (z0 > 0) {
+        fold_cofactors<MODE>(phi, g, item + (unsigned)zs * pl + col, cs, pl, zs, oxu, oxd, oyu, oyd, xlo, xhi, ylo, yhi, inside, vm, vc, Gc);
+#pragma unroll
+        for (int c = 0; c < 3; ++c) g0m[c] = Gc[c][0];
+    }
+    fold_cofactors<MODE>(phi, g, item + (unsigned)z0 * pl + col, cs, pl, z0, oxu, oxd, oyu, oyd, xlo, xhi, ylo, yhi, inside, vm, vc, Gc);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) g1s[z0 & 1][c][wy][lane] = Gc[c][1];
+    __syncthreads();
+
+    for (int z = z0; z < z1; ++z) {
+        float gy[3][2], gx[3][2];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            gy[c][0] = g1s[z & 1][c][max(wy - 1, 0)][lane];
+            gy[c][1] = g1s[z & 1][c][min(wy + 1, FOLD_WARPS - 1)][lane];
+            gx[c][0] = __shfl_up_sync(0xffffffffu, Gc[c][2], 1);
+            gx[c][1] = __shfl_down_sync(0xffffffffu, Gc[c][2], 1);
+        }
+        float Gn[3][3];
+        if (z + 1 < g.d) {
+            fold_cofactors<MODE>(phi, g, item + (unsigned)(z + 1) * pl + col, cs, pl, z + 1, oxu, oxd, oyu, oyd, xlo, xhi, ylo, yhi, inside,
+                                 vm, vc, Gn);
+        } else {
+#pragma unroll
+            for (int c = 0; c < 3; ++c) Gn[c][0] = Gn[c][1] = Gn[c][2] = 0.0f;
+        }
+#pragma unroll
+        for (int c = 0; c < 3; ++c) g1s[(z + 1) & 1][c][wy][lane] = Gn[c][1];
+        if (writer) {
+            const unsigned o = item + (unsigned)z * pl + col;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                float gr = mul_rn(kd, fold_adjoint<MODE>(g0m[c], Gc[c][0], Gn[c][0], z, g.d));
+                gr = fmaf(kh, fold_adjoint<MODE>(gy[c][0], Gc[c][1], gy[c][1], y, g.h), gr);
+                gr = fmaf(kw, fold_adjoint<MODE>(gx[c][0], Gc[c][2], gx[c][1], x, g.w), gr);
+                st_stream(grad_phi + (o + c * cs), gr);
+            }
+        }
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            g0m[c] = Gc[c][0];
+            Gc[c][0] = Gn[c][0]; Gc[c][1] = Gn[c][1]; Gc[c][2] = Gn[c][2];
+        }
+        __syncthreads();
+    }
+}
+
 // ---- label confusion matrix: counts[b][p][t] = #voxels with pred == p and target == t ------------------------------
 // Every (pred, target) pair that is not two integers in [0, L) goes to one extra bin, key L*L, reported as `invalid`.
 // The histogram is privatised in shared memory ((L*L+1) 32-bit bins, <= 64 KB at L = 128) and merged into the int64
@@ -851,6 +996,27 @@ extern "C" int lr_jacobian_det(const float *phi, int B, int D, int H, int W, int
     cudaStream_t st = as_stream(stream);
     return boundary == LR_FD_LINEAR ? jacobian_launch<0>(phi, B, D, H, W, margin, det, stats, st)
                                     : jacobian_launch<1>(phi, B, D, H, W, margin, det, stats, st);
+}
+
+template <int MODE>
+static int fold_backward_launch(const float *phi, int B, int D, int H, int W, const float *grad_loss, float *grad_phi, cudaStream_t st) {
+    RegDims g; dim3 grid;
+    const int rd = march_dims(jacobian_fold_backward_kernel<MODE>, FOLD_THREADS, FOLD_OX, FOLD_OY, LR_REG_WAVES, B, D, H, W, g, grid);
+    LR_REQUIRE(rd == 0, "jacobian_fold_backward: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)", B, D, H, W);
+    jacobian_fold_backward_kernel<MODE><<<grid, FOLD_THREADS, 0, st>>>(phi, g, B, grad_loss, grad_phi);
+    return check_launch("jacobian_fold_backward_kernel");
+}
+
+extern "C" int lr_jacobian_fold_backward(const float *phi, int B, int D, int H, int W, int boundary, const float *grad_loss,
+                                         float *grad_phi, lr_stream_t stream) {
+    LR_REQUIRE(phi && grad_loss && grad_phi, "jacobian_fold_backward: null pointer");
+    LR_REQUIRE(B > 0 && D >= 2 && H >= 2 && W >= 2, "jacobian_fold_backward: every axis needs >= 2 entries (B=%d, %dx%dx%d)", B, D, H, W);
+    LR_REQUIRE(boundary == LR_FD_LINEAR || boundary == LR_FD_NEUMANN_ZERO, "jacobian_fold_backward: unknown boundary mode %d", boundary);
+    LR_REQUIRE((int64_t)B * 3 * D * H * W < ((int64_t)1 << 31),
+               "jacobian_fold_backward: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)", B, D, H, W);
+    cudaStream_t st = as_stream(stream);
+    return boundary == LR_FD_LINEAR ? fold_backward_launch<0>(phi, B, D, H, W, grad_loss, grad_phi, st)
+                                    : fold_backward_launch<1>(phi, B, D, H, W, grad_loss, grad_phi, st);
 }
 
 extern "C" int lr_label_confusion(const float *pred, const float *target, int B, int64_t N, int L, int64_t *counts, int64_t *invalid,

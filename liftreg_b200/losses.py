@@ -46,7 +46,10 @@ class SubspaceLoss(nn.Module):
 
     The similarity is `NCCLoss` (the reference's default sim_class, :12) and the regulariser the fused
     finite-difference kernel (`ops.diffusion_reg`), both differentiable.  `fd_boundary` selects the face rule of
-    mermaid's finite differences ("linear" = FD_torch's default)."""
+    mermaid's finite differences ("linear" = FD_torch's default).
+
+    Opt key `fold_factor` (default 0, not in the reference): when > 0, `fold_factor * ops.fold_penalty(phi)` is added to
+    the total, with phi = params + identity (the model's `disp_field + id_transform`), and reported as "fold_loss"."""
 
     def __init__(self, opt=None, sim=None, fd_boundary="linear"):
         super().__init__()
@@ -55,13 +58,27 @@ class SubspaceLoss(nn.Module):
         self.initial_reg_factor = _opt(opt, 'initial_reg_factor', 10)
         self.min_reg_factor = _opt(opt, 'min_reg_factor', 1e-3)
         self.reg_factor_decay_from = _opt(opt, 'reg_factor_decay_from', 10)
+        self.fold_factor = _opt(opt, 'fold_factor', 0)
         self.fd_boundary = fd_boundary
+        self._identity = {}
 
     def forward(self, input):
         sim_loss = self.sim(input["warped"], input["target"])
         reg_loss = self.compute_reg_loss(input["params"])
         total_loss = self.sim_factor * sim_loss + self.get_reg_factor(input["epoch"]) * reg_loss
-        return {"total_loss": total_loss, "sim_loss": sim_loss.item(), "reg_loss": reg_loss.item()}
+        out = {"total_loss": total_loss, "sim_loss": sim_loss.item(), "reg_loss": reg_loss.item()}
+        if self.fold_factor > 0:
+            fold_loss = self.compute_fold_loss(input["params"])
+            out["total_loss"] = total_loss + self.fold_factor * fold_loss
+            out["fold_loss"] = fold_loss.item()
+        return out
+
+    def compute_fold_loss(self, disp):
+        """mean over (B, D, H, W) of max(0, -det J) of the map disp + identity (ops.fold_penalty)"""
+        key = (tuple(disp.shape[2:]), disp.device)
+        if key not in self._identity:
+            self._identity[key] = ops.identity_map(disp.shape[2:], disp.device)
+        return ops.fold_penalty(disp + self._identity[key], self.fd_boundary)
 
     def get_reg_factor(self, epoch):
         """:40-49"""

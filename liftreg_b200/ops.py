@@ -468,6 +468,14 @@ def diffusion_reg(disp, boundary="linear"):
 JACOBIAN_STATS = ("folding_count", "folding_abs_sum", "det_min", "det_max", "det_sum", "det_sum_sq", "nonfinite_count")
 
 
+def _need_map(phi, boundary):
+    if not isinstance(phi, torch.Tensor) or phi.dim() != 5 or phi.shape[1] != 3:
+        raise ValueError("phi must be a (B,3,D,H,W) tensor, got %s" % (tuple(phi.shape) if isinstance(phi, torch.Tensor) else type(phi).__name__,))
+    if boundary not in FD_BOUNDARY:
+        raise ValueError("boundary must be one of %s, got %r" % (sorted(FD_BOUNDARY), boundary))
+    return _need_cuda_f32(phi, "phi")
+
+
 def jacobian_det(phi, boundary="linear", margin=0, want_map=False):
     """Jacobian determinant of a map phi (B,3,D,H,W) in [-1,1] (channel c addresses volume axis c) with the
     regulariser's central differences and face rule `boundary`, scaled so that the identity map has det 1.
@@ -475,11 +483,7 @@ def jacobian_det(phi, boundary="linear", margin=0, want_map=False):
     Returns (stats, det): stats is a (B,7) float64 CUDA tensor ordered as JACOBIAN_STATS, over the voxels at least
     `margin` from every face (sums and min / max over finite values only); det is the (B,D,H,W) float32 map when
     want_map, else None.  Parity with the reference's utils.py:20-55 is unpinned (include/liftreg_b200.h)."""
-    if not isinstance(phi, torch.Tensor) or phi.dim() != 5 or phi.shape[1] != 3:
-        raise ValueError("phi must be a (B,3,D,H,W) tensor, got %s" % (tuple(phi.shape) if isinstance(phi, torch.Tensor) else type(phi).__name__,))
-    if boundary not in FD_BOUNDARY:
-        raise ValueError("boundary must be one of %s, got %r" % (sorted(FD_BOUNDARY), boundary))
-    phi = _need_cuda_f32(phi, "phi")
+    phi = _need_map(phi, boundary)
     B, _, D, H, W = phi.shape
     stats = torch.empty((B, 7), device=phi.device, dtype=torch.float64)
     det = torch.empty((B, D, H, W), device=phi.device, dtype=torch.float32) if want_map else None
@@ -487,6 +491,41 @@ def jacobian_det(phi, boundary="linear", margin=0, want_map=False):
         _native.check(_native.lib().lr_jacobian_det(_ptr(phi), B, D, H, W, FD_BOUNDARY[boundary], int(margin), _ptr(det),
                                                     _ptr(stats), _stream()), "lr_jacobian_det")
     return stats, det
+
+
+# --------------------------------------------------------------------------- folding penalty (training term)
+class _FoldPenalty(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, phi, boundary):
+        phi = _need_map(phi, boundary)
+        B, _, D, H, W = phi.shape
+        stats = torch.empty((B, 7), device=phi.device, dtype=torch.float64)
+        with torch.cuda.device(phi.device):
+            _native.check(_native.lib().lr_jacobian_det(_ptr(phi), B, D, H, W, FD_BOUNDARY[boundary], 0, None, _ptr(stats),
+                                                        _stream()), "lr_jacobian_det")
+        ctx.save_for_backward(phi)
+        ctx.boundary = boundary
+        return (stats[:, 1].sum() / float(B * D * H * W)).to(torch.float32)
+
+    @staticmethod
+    def backward(ctx, grad_loss):
+        phi, = ctx.saved_tensors
+        B, _, D, H, W = phi.shape
+        g = grad_loss.to(device=phi.device, dtype=torch.float32).reshape(1).contiguous()
+        gphi = torch.empty_like(phi)
+        with torch.cuda.device(phi.device):
+            _native.check(_native.lib().lr_jacobian_fold_backward(_ptr(phi), B, D, H, W, FD_BOUNDARY[ctx.boundary], _ptr(g),
+                                                                  _ptr(gphi), _stream()), "lr_jacobian_fold_backward")
+        return gphi, None
+
+
+def fold_penalty(phi, boundary="linear"):
+    """Folding penalty of a map phi (B,3,D,H,W) in [-1,1]: the mean over (B, D, H, W) of max(0, -det J), with det the
+    value jacobian_det computes (same boundary, every voxel, non-finite values skipped).  A float32 scalar on phi's
+    device, computed without a host synchronisation; differentiable wrt phi (subgradient over the strict fold set
+    det < 0).  The reference has no such term, so parity is unpinned (include/liftreg_b200.h,
+    lr_jacobian_fold_backward)."""
+    return _FoldPenalty.apply(phi, boundary)
 
 
 def _label_map(t, name):

@@ -122,6 +122,19 @@ def main():
     def k_jac_map(s, st):      # ... and the determinant map written out
         _native.check(lib.lr_jacobian_det(vp(s["phi"]), 1, *VOL, 0, 0, vp(s["warped"]), vp(jac_stats), st), "jac_map")
 
+    def k_fold_bwd(s, st):     # d fold / d phi (folding penalty adjoint): reads phi, writes grad_phi
+        _native.check(lib.lr_jacobian_fold_backward(vp(s["phi"]), 1, *VOL, 0, vp(ncc_g), vp(s["gphi"]), st), "fold_bwd")
+
+    if "fold_bwd8" in which:
+        phi8 = [torch.from_numpy((synthetic.smooth_displacement(VOL, seed=b) + synthetic.identity_map_np(VOL))[None]).to(dev)
+                for b in range(8)]
+        for i, s_ in enumerate(sets):
+            s_["phi8"] = torch.cat(phi8, 0) + 1e-3 * i
+            s_["gphi8"] = torch.empty((8, 3) + VOL, device=dev)
+
+    def k_fold_bwd8(s, st):
+        _native.check(lib.lr_jacobian_fold_backward(vp(s["phi8"]), 8, *VOL, 0, vp(ncc_g), vp(s["gphi8"]), st), "fold_bwd8")
+
     if "labels2" in which or "labels6" in which:
         # label maps as a validation item has them: mostly background, a few organ-sized blobs, target = shifted pred
         zz, yy, xx = np.meshgrid(*[np.arange(n) for n in VOL], indexing="ij")
@@ -148,7 +161,7 @@ def main():
         _native.check(lib.lr_identity_map(*VOL, vp(s["gphi"]), st), "idmap")
 
     units = {"atten": (k_atten, nv, 8 * nv), "idmap": (k_idmap, nv, 12 * nv), "reg": (k_reg, nv, 12 * nv), "jac": (k_jac, nv, 12 * nv), "jac_map": (k_jac_map, nv, 16 * nv),
-             "labels2": (k_labels(2), nv, 8 * nv), "labels6": (k_labels(6), nv, 8 * nv), "reg_bwd": (k_reg_bwd, nv, 24 * nv), "ncc": (k_ncc, nv, 8 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
+             "labels2": (k_labels(2), nv, 8 * nv), "labels6": (k_labels(6), nv, 8 * nv), "reg_bwd": (k_reg_bwd, nv, 24 * nv), "fold_bwd": (k_fold_bwd, nv, 24 * nv), "fold_bwd8": (k_fold_bwd8, 8 * nv, 8 * 24 * nv), "ncc": (k_ncc, nv, 8 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
              "pca_bwd": (k_pca_bwd, 3 * nv, 4 * 3 * nv * 56 + 4 * 3 * nv), "warp_bwd": (k_warp_bwd, nv, 32 * nv),
              "drr_bwd": (k_drr_bwd, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240), "backproject": (k_backproject, batch * P * nv, batch * (4 * P * nv + 4 * P * DET[0] * DET[1])),
              "drr": (k_drr, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240),
