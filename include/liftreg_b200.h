@@ -336,6 +336,36 @@ LR_API int lr_label_confusion(const float *pred, const float *target, int B, int
 LR_API int lr_jacobian_fold_backward(const float *phi, int B, int D, int H, int W, int boundary,
                                      const float *grad_loss, float *grad_phi, lr_stream_t stream);
 
+/* ---- local (windowed) NCC similarity (a training term; PARITY UNPINNED: the reference has none) --------------------
+ * VoxelMorph's NCC(win) form, per batch item b, with x = warped, y = target, both (B,1,D,H,W) float32 and an odd
+ * window side w in [3, 15]:
+ *   N(v) is the w x w x w cube centred on voxel v; voxels outside the volume count as 0 (zero padding) and
+ *   n = w^3 is fixed (it is not the number of voxels inside).  Sx, Sy, Sxx, Syy, Sxy are the sums over N(v);
+ *   cross = Sxy - Sx*Sy/n,  var_x = Sxx - Sx^2/n,  var_y = Syy - Sy^2/n,  d = var_x*var_y + eps,
+ *   cc(v) = cross^2 / d  (cc = 0 where d <= 0: a window with zero variance and eps = 0),
+ *   loss = 1 - mean over (B, D, H, W) of cc.
+ * The gradient is taken wrt x only (the target is data).  With mu = S/n and, per window centre u with d > 0,
+ *   alpha_u = 2*cross/d,  beta_u = 2*cross^2*var_y/d^2,  gamma_u = beta_u*mu_x - alpha_u*mu_y   (all 0 where d <= 0),
+ *   d loss / d x_v = -(grad_loss / (B*D*H*W)) * (y_v * sum alpha - x_v * sum beta + sum gamma),
+ * each sum over the centres u in N(v) inside the volume (with zero padding and a fixed n, v in N(u) <=> u in N(v), so
+ * the adjoint is again a box sum).
+ * Every window sum is accumulated in fp64 (the products of the fp32 inputs are exact there) as a plain sum of its terms
+ * in a fixed order, so no result depends on the launch shape or the batch size.
+ * lr_local_ncc_sum: sum (B) float64, zeroed by the call, = the fp64 sum of cc over each item;
+ *   loss = 1 - (sum_b sum[b]) / (B*D*H*W).
+ * lr_local_ncc_backward: grad_x (B,1,D,H,W) is OVERWRITTEN with grad_loss[0] * d loss / d x (grad_loss: one float in
+ *   device memory); each element is written once, without atomics, so repeated calls give the same bits.  It needs a
+ *   caller-owned device workspace of lr_local_ncc_workspace_bytes(B, D, H, W, win) bytes (alpha, beta, gamma as
+ *   float32: 12 bytes per voxel; the call never allocates).
+ * Arguments: win odd in [3, 15]; eps finite and >= 0; every axis >= 1 (an axis may be smaller than the window)
+ * and <= 2^30; B*D*H*W < 2^31; no null pointer.  lr_local_ncc_workspace_bytes returns 0 for arguments the calls reject. */
+LR_API int lr_local_ncc_sum(const float *x, const float *y, int B, int D, int H, int W, int win, double eps,
+                            double *sum, lr_stream_t stream);
+LR_API size_t lr_local_ncc_workspace_bytes(int B, int D, int H, int W, int win);
+LR_API int lr_local_ncc_backward(const float *x, const float *y, int B, int D, int H, int W, int win, double eps,
+                                 const float *grad_loss, float *grad_x, void *workspace, size_t workspace_bytes,
+                                 lr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

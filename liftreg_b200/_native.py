@@ -63,6 +63,9 @@ SIGNATURES = {
     "lr_jacobian_det": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "lr_jacobian_fold_backward": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "lr_label_confusion": (_i, [_vp, _vp, _i, _i64, _i, _vp, _vp, _vp]),
+    "lr_local_ncc_sum": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.c_double, _vp, _vp]),
+    "lr_local_ncc_workspace_bytes": (_sz, [_i, _i, _i, _i, _i]),
+    "lr_local_ncc_backward": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.c_double, _vp, _vp, _vp, _sz, _vp]),
 }
 
 _lib = None

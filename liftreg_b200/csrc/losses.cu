@@ -9,6 +9,8 @@
 // B-thread kernel) and the backward is one pass.  Per-thread partial sums are fp32 over a handful of elements, everything above that
 // is accumulated in fp64 (warp shuffles, shared memory, one fp64 atomic per block), so the result does not depend on the launch shape
 // beyond fp64 round-off.
+#include <cfloat>
+
 #include "common.cuh"
 
 namespace lr {
@@ -894,6 +896,153 @@ static unsigned conf_blocks(int64_t N, int B, int L, int per_sm) {
     return (unsigned)(want < 1 ? 1 : want);
 }
 
+// ---- local (windowed) NCC, a training similarity (include/liftreg_b200.h; PARITY UNPINNED: the reference has none) ----
+// Every quantity is a zero-padded box sum over the w x w x w cube centred on a voxel: the forward sums the five moments
+// x, y, x^2, y^2, xy; the adjoint sums the three per-centre coefficients alpha, beta, gamma.  One plane-march kernel
+// serves all three passes (LNCC_FWD: cc summed per item; LNCC_COEF: alpha, beta, gamma written to the workspace;
+// LNCC_GRAD: their box sums combined with x and y into grad_x).  A block owns a 32 x 8 tile of (last, second) axis
+// positions and marches a chunk of planes of the first axis.  Per input plane it
+//   stages the plane's moments over the tile plus a halo of w-1 in shared memory (fp64: the products x*x, x*y of fp32
+//     values are exact there),
+//   sums w consecutive entries along the last axis (row pass, shared memory) and then w rows (column pass),
+//   and keeps the 2-D sum in a ring of w planes per thread (shared memory), from which an output's window sum is the
+//     sum of its w planes in plane order.
+// Every window sum is thus a plain fp64 sum of its own terms in a fixed order -- no running add / subtract along an
+// axis, no dependence on the tiling, the z chunking or the batch size -- so results repeat bit for bit and the
+// cancellation in var = Sxx - Sx^2/n (the CT body at ~1 with 0.01 noise: var / Sxx ~ 1e-4) costs fp64, not fp32, digits.
+// Each output element is written once, with no atomics.
+constexpr int LNCC_TX = 32, LNCC_TY = 8, LNCC_THREADS = LNCC_TX * LNCC_TY, LNCC_WMAX = 15;
+static_assert(LNCC_THREADS == NCC_THREADS, "local_ncc_kernel<fwd> reduces with block_accumulate_f64, sized for NCC_THREADS");
+enum { LNCC_FWD = 0, LNCC_COEF = 1, LNCC_GRAD = 2 };
+
+struct LnccDims {
+    int D, H, W, w, tiles_x, tiles_y, zchunk, n_zchunks;
+    unsigned N, total;     // voxels per item and in all B items (B*D*H*W < 2^31)
+    double n, eps, count;  // n = w^3, count = B*D*H*W
+};
+
+template <int KIND> struct LnccMoments { static constexpr int NM = KIND == LNCC_GRAD ? 3 : 5; };
+
+// dynamic shared memory of one block: ring[w][NM][threads] + rows[NM][TY+w-1][TX] + tile[NM][TY+w-1][TX+w-1], fp64
+template <int KIND>
+static size_t lncc_smem_bytes(int w) {
+    const int nm = LnccMoments<KIND>::NM;
+    return sizeof(double) * (size_t)nm * ((size_t)w * LNCC_THREADS + (size_t)(LNCC_TY + w - 1) * LNCC_TX +
+                                          (size_t)(LNCC_TY + w - 1) * (LNCC_TX + w - 1));
+}
+
+template <int KIND>
+__global__ void __launch_bounds__(LNCC_THREADS) local_ncc_kernel(const float *__restrict__ x, const float *__restrict__ y,
+                                                                 const float *__restrict__ coef, LnccDims g,
+                                                                 const float *__restrict__ grad_loss, double *__restrict__ sum,
+                                                                 float *__restrict__ out) {
+    constexpr int NM = LnccMoments<KIND>::NM;
+    extern __shared__ double lncc_smem[];
+    const int w = g.w, r = w >> 1, th = LNCC_TY + w - 1, tw = LNCC_TX + w - 1;
+    double *ring = lncc_smem;                                   // [w][NM][LNCC_THREADS], private to each thread
+    double *rows = ring + (size_t)w * NM * LNCC_THREADS;        // [NM][th][LNCC_TX]
+    double *tile = rows + (size_t)NM * th * LNCC_TX;            // [NM][th][tw]
+    const int tid = threadIdx.x, lane = tid & 31, wy = tid >> 5;
+
+    unsigned blk = blockIdx.x;                                  // (tile x, tile y, z chunk, item), x fastest
+    const int tx = blk % g.tiles_x; blk /= g.tiles_x;
+    const int ty = blk % g.tiles_y; blk /= g.tiles_y;
+    const int zc = blk % g.n_zchunks;
+    const int b = blk / g.n_zchunks;
+    const int x0 = tx * LNCC_TX, y0 = ty * LNCC_TY, z0 = zc * g.zchunk, z1 = min(g.D, z0 + g.zchunk);
+    const int ox = x0 + lane, oy = y0 + wy;
+    const bool writer = ox < g.W && oy < g.H;
+    const unsigned plane = (unsigned)g.H * (unsigned)g.W, item = (unsigned)b * g.N;
+    const float *c0 = coef, *c1 = coef + g.total, *c2 = coef + 2 * (size_t)g.total;     // alpha, beta, gamma (LNCC_GRAD)
+    double acc = 0.0;
+
+    for (int p = z0 - r; p < z1 + r; ++p) {
+        const int slot = (p + w) % w;                           // p >= -r > -w
+        double P[NM];
+        if (p < 0 || p >= g.D) {                                // a plane of the zero padding
+#pragma unroll
+            for (int m = 0; m < NM; ++m) P[m] = 0.0;
+        } else {
+            // stage the plane's moments over tile + halo (zero outside the volume)
+            const unsigned pbase = item + (unsigned)p * plane;
+            for (int i = tid; i < th * tw; i += LNCC_THREADS) {
+                const int gy = y0 - r + i / tw, gx = x0 - r + i % tw;
+                double v[NM];
+#pragma unroll
+                for (int m = 0; m < NM; ++m) v[m] = 0.0;
+                if (gy >= 0 && gy < g.H && gx >= 0 && gx < g.W) {
+                    const unsigned e = pbase + (unsigned)gy * (unsigned)g.W + (unsigned)gx;
+                    if (KIND == LNCC_GRAD) {
+                        v[0] = (double)__ldg(c0 + e); v[1] = (double)__ldg(c1 + e); v[2] = (double)__ldg(c2 + e);
+                    } else {
+                        const double a = (double)__ldg(x + e), c = (double)__ldg(y + e);
+                        v[0] = a; v[1] = c; v[2] = a * a; v[3] = c * c; v[NM - 1] = a * c;      // exact products
+                    }
+                }
+#pragma unroll
+                for (int m = 0; m < NM; ++m) tile[(size_t)m * th * tw + i] = v[m];
+            }
+            __syncthreads();
+            // row pass: w consecutive entries along the last axis, in index order
+            for (int i = tid; i < th * LNCC_TX; i += LNCC_THREADS) {
+                const int ry = i / LNCC_TX, rx = i % LNCC_TX;
+#pragma unroll
+                for (int m = 0; m < NM; ++m) {
+                    const double *t = tile + (size_t)m * th * tw + ry * tw + rx;
+                    double s = t[0];
+                    for (int d = 1; d < w; ++d) s += t[d];
+                    rows[(size_t)m * th * LNCC_TX + i] = s;
+                }
+            }
+            __syncthreads();
+            // column pass: w rows, in index order
+#pragma unroll
+            for (int m = 0; m < NM; ++m) {
+                const double *t = rows + (size_t)m * th * LNCC_TX + wy * LNCC_TX + lane;
+                double s = t[0];
+                for (int d = 1; d < w; ++d) s += t[d * LNCC_TX];
+                P[m] = s;
+            }
+        }
+#pragma unroll
+        for (int m = 0; m < NM; ++m) ring[((size_t)slot * NM + m) * LNCC_THREADS + tid] = P[m];
+
+        const int z = p - r;                                    // the output plane whose window closes with plane p
+        if (z < z0 || !writer) continue;
+        double S[NM];
+#pragma unroll
+        for (int m = 0; m < NM; ++m) S[m] = 0.0;
+        for (int q = z - r; q <= z + r; ++q) {                  // plane order, whatever the ring's phase
+            const double *s = ring + (size_t)((q + w) % w) * NM * LNCC_THREADS + tid;
+#pragma unroll
+            for (int m = 0; m < NM; ++m) S[m] += s[(size_t)m * LNCC_THREADS];
+        }
+        const unsigned e = item + (unsigned)z * plane + (unsigned)oy * (unsigned)g.W + (unsigned)ox;
+        if (KIND == LNCC_GRAD) {
+            // grad_x = -(g / (B*D*H*W)) * (y * sum alpha - x * sum beta + sum gamma)
+            const double k = (double)grad_loss[0] / g.count;
+            const double t = (double)__ldg(y + e) * S[0] - (double)__ldg(x + e) * S[1] + S[2];
+            out[e] = (float)(-k * t);
+        } else {
+            const double cross = S[4] - S[0] * S[1] / g.n;
+            const double vx = S[2] - S[0] * S[0] / g.n, vy = S[3] - S[1] * S[1] / g.n;
+            const double d = vx * vy + g.eps;
+            if (KIND == LNCC_FWD) {
+                if (d > 0.0) acc += cross * cross / d;
+            } else {
+                double al = 0.0, be = 0.0, ga = 0.0;
+                if (d > 0.0) {
+                    al = 2.0 * cross / d;
+                    be = 2.0 * cross * cross * vy / (d * d);
+                    ga = be * (S[0] / g.n) - al * (S[1] / g.n);
+                }
+                out[e] = (float)al; out[e + (size_t)g.total] = (float)be; out[e + 2 * (size_t)g.total] = (float)ga;
+            }
+        }
+    }
+    if (KIND == LNCC_FWD) block_accumulate_f64(acc, sum + b);
+}
+
 }  // namespace lr
 
 using namespace lr;
@@ -1045,4 +1194,82 @@ extern "C" int lr_label_confusion(const float *pred, const float *target, int B,
     label_confusion_kernel<<<grid, CONF_THREADS, smem, st>>>(pred, target, N, L, reinterpret_cast<unsigned long long *>(counts),
                                                               reinterpret_cast<unsigned long long *>(invalid));
     return check_launch("label_confusion_kernel");
+}
+
+// argument rules shared by the local NCC entries; 0 when they hold
+static int lncc_check(const char *who, int B, int D, int H, int W, int win, double eps) {
+    LR_REQUIRE(win % 2 == 1 && win >= 3 && win <= LNCC_WMAX, "%s: window %d must be odd and in [3, %d]", who, win, LNCC_WMAX);
+    LR_REQUIRE(eps >= 0.0 && eps <= DBL_MAX, "%s: eps must be finite and >= 0 (got %g)", who, eps);
+    LR_REQUIRE(B >= 1 && D >= 1 && H >= 1 && W >= 1, "%s: every axis needs >= 1 entry (B=%d, %dx%dx%d)", who, B, D, H, W);
+    // tile origins plus the 32 + 14 tile-and-halo offsets stay in int
+    LR_REQUIRE(D <= (1 << 30) && H <= (1 << 30) && W <= (1 << 30), "%s: every axis must be <= 2^30 (%dx%dx%d)", who, D, H, W);
+    LR_REQUIRE((int64_t)B * D * H * W < ((int64_t)1 << 31), "%s: too large for one launch (B=%d, %dx%dx%d; B*D*H*W must stay below 2^31)",
+               who, B, D, H, W);
+    return 0;
+}
+
+template <int KIND>
+static int lncc_launch(const float *x, const float *y, const float *coef, int B, int D, int H, int W, int win, double eps,
+                       const float *grad_loss, double *sum, float *out, cudaStream_t st, const char *name) {
+    static thread_local int attr_dev = -1;          // the > 48 KB opt-in is per device
+    int dev = 0;
+    cudaError_t ce = cudaGetDevice(&dev);
+    if (ce == cudaSuccess && dev != attr_dev) {
+        ce = cudaFuncSetAttribute(local_ncc_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lncc_smem_bytes<KIND>(LNCC_WMAX));
+        if (ce == cudaSuccess) attr_dev = dev;
+    }
+    if (ce != cudaSuccess) { set_error("%s: %s", name, cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    const size_t smem = lncc_smem_bytes<KIND>(win);
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, local_ncc_kernel<KIND>, LNCC_THREADS, smem) != cudaSuccess || per_sm < 1) {
+        cudaGetLastError();
+        per_sm = 1;
+    }
+    LnccDims g;
+    g.D = D; g.H = H; g.W = W; g.w = win;
+    g.N = (unsigned)D * (unsigned)H * (unsigned)W;
+    g.total = g.N * (unsigned)B;
+    g.n = (double)win * win * win; g.eps = eps; g.count = (double)g.total;
+    g.tiles_x = (W + LNCC_TX - 1) / LNCC_TX;
+    g.tiles_y = (H + LNCC_TY - 1) / LNCC_TY;
+    // enough z chunks for two waves of resident blocks, but a chunk of at least w planes (a chunk re-reads w-1 planes)
+    const int64_t tiles = (int64_t)g.tiles_x * g.tiles_y * B;
+    int64_t chunks = (2 * (int64_t)sm_count() * per_sm + tiles - 1) / tiles;
+    if (chunks > D / win) chunks = D / win;
+    if (chunks < 1) chunks = 1;
+    g.zchunk = (int)((D + chunks - 1) / chunks);
+    g.n_zchunks = (D + g.zchunk - 1) / g.zchunk;
+    const int64_t blocks = tiles * g.n_zchunks;     // <= B*D*H*W < 2^31
+    local_ncc_kernel<KIND><<<(unsigned)blocks, LNCC_THREADS, smem, st>>>(x, y, coef, g, grad_loss, sum, out);
+    return check_launch(name);
+}
+
+extern "C" int lr_local_ncc_sum(const float *x, const float *y, int B, int D, int H, int W, int win, double eps, double *sum,
+                                lr_stream_t stream) {
+    LR_REQUIRE(x && y && sum, "local_ncc_sum: null pointer");
+    if (int e = lncc_check("local_ncc_sum", B, D, H, W, win, eps)) return e;
+    cudaStream_t st = as_stream(stream);
+    cudaError_t ce = cudaMemsetAsync(sum, 0, sizeof(double) * (size_t)B, st);
+    if (ce != cudaSuccess) { set_error("local_ncc_sum: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    return lncc_launch<LNCC_FWD>(x, y, nullptr, B, D, H, W, win, eps, nullptr, sum, nullptr, st, "local_ncc_kernel<fwd>");
+}
+
+extern "C" size_t lr_local_ncc_workspace_bytes(int B, int D, int H, int W, int win) {
+    if (win % 2 != 1 || win < 3 || win > LNCC_WMAX || B < 1 || D < 1 || H < 1 || W < 1) return 0;
+    if (D > (1 << 30) || H > (1 << 30) || W > (1 << 30)) return 0;
+    if ((int64_t)B * D * H * W >= ((int64_t)1 << 31)) return 0;
+    return 3 * sizeof(float) * (size_t)B * D * H * W;          // alpha, beta, gamma per voxel
+}
+
+extern "C" int lr_local_ncc_backward(const float *x, const float *y, int B, int D, int H, int W, int win, double eps,
+                                     const float *grad_loss, float *grad_x, void *workspace, size_t workspace_bytes,
+                                     lr_stream_t stream) {
+    LR_REQUIRE(x && y && grad_loss && grad_x && workspace, "local_ncc_backward: null pointer");
+    if (int e = lncc_check("local_ncc_backward", B, D, H, W, win, eps)) return e;
+    const size_t need = lr_local_ncc_workspace_bytes(B, D, H, W, win);
+    LR_REQUIRE(workspace_bytes >= need, "local_ncc_backward: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+    cudaStream_t st = as_stream(stream);
+    float *coef = static_cast<float *>(workspace);
+    if (int e = lncc_launch<LNCC_COEF>(x, y, nullptr, B, D, H, W, win, eps, nullptr, nullptr, coef, st, "local_ncc_kernel<coef>")) return e;
+    return lncc_launch<LNCC_GRAD>(x, y, coef, B, D, H, W, win, eps, grad_loss, nullptr, grad_x, st, "local_ncc_kernel<grad>");
 }

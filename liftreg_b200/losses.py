@@ -22,6 +22,20 @@ class NCCLoss(nn.Module):
         return loss
 
 
+class LocalNCCLoss(nn.Module):
+    """1 - mean local NCC of VoxelMorph's NCC(win=window) form (ops.local_ncc_loss): the squared correlation of each
+    window x window x window neighbourhood, zero padding.  Not in the reference; select it with
+    `SubspaceLoss(opt, sim=LocalNCCLoss())` or by its dotted name (`sim_class = "liftreg_b200.losses.LocalNCCLoss"`)."""
+
+    def __init__(self, window=9, eps=1e-5):
+        super().__init__()
+        self.window = int(window)
+        self.eps = float(eps)
+
+    def forward(self, input, target):
+        return ops.local_ncc_loss(input, target, self.window, self.eps)
+
+
 def sigmoid_decay(ep, static=5, k=5):
     """reference utils/utils.py:93-107: 1 for the first `static` epochs, then k / (k + exp((ep - static) / k))."""
     if ep < static:

@@ -422,6 +422,55 @@ def ncc_loss(input, target):
     return _Ncc.apply(input, target)
 
 
+# --------------------------------------------------------------------------- local NCC similarity (training term)
+def _volume(t, name):
+    """(B,1,D,H,W) or (B,D,H,W) CUDA float32 -> contiguous tensor and (B, D, H, W)"""
+    if not isinstance(t, torch.Tensor) or not (t.dim() == 4 or (t.dim() == 5 and t.shape[1] == 1)):
+        raise ValueError("%s must be (B,1,D,H,W) or (B,D,H,W), got %s"
+                         % (name, tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__))
+    t = _need_cuda_f32(t, name)
+    return t, (t.shape[0],) + tuple(t.shape[-3:])
+
+
+class _LocalNcc(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, y, window, eps):
+        x, (B, D, H, W) = _volume(x, "input")
+        y, _ = _volume(y, "target")
+        sums = torch.empty(B, device=x.device, dtype=torch.float64)
+        with torch.cuda.device(x.device):
+            _native.check(_native.lib().lr_local_ncc_sum(_ptr(x), _ptr(y), B, D, H, W, window, eps, _ptr(sums), _stream()),
+                          "lr_local_ncc_sum")
+        ctx.save_for_backward(x, y)
+        ctx.cfg = (window, eps)
+        return (1.0 - sums.sum() / float(B * D * H * W)).to(torch.float32)
+
+    @staticmethod
+    def backward(ctx, grad_loss):
+        x, y = ctx.saved_tensors
+        window, eps = ctx.cfg
+        B, D, H, W = x.shape[0], *x.shape[-3:]
+        g = grad_loss.to(device=x.device, dtype=torch.float32).reshape(1).contiguous()
+        gx = torch.empty_like(x)
+        lib = _native.lib()
+        ws = torch.empty(lib.lr_local_ncc_workspace_bytes(B, D, H, W, window), device=x.device, dtype=torch.uint8)
+        with torch.cuda.device(x.device):
+            _native.check(lib.lr_local_ncc_backward(_ptr(x), _ptr(y), B, D, H, W, window, eps, _ptr(g), _ptr(gx), _ptr(ws),
+                                                    ws.numel(), _stream()), "lr_local_ncc_backward")
+        return gx, None, None, None
+
+
+def local_ncc_loss(input, target, window=9, eps=1e-5):
+    """1 - mean over (B, D, H, W) of the local (windowed) squared correlation cc of VoxelMorph's NCC(win): window sums
+    over the window x window x window cube around each voxel, zero padding, cc = cross^2 / (var_x var_y + eps)
+    (definition: include/liftreg_b200.h, lr_local_ncc_sum).  input and target are (B,1,D,H,W) or (B,D,H,W) CUDA
+    float32; window is odd, in [3, 15].  Differentiable wrt `input` (the warped image); `target` is data.  The reference
+    has no such term, so parity is unpinned."""
+    if input.shape != target.shape:
+        raise ValueError("input %s and target %s must have the same shape" % (tuple(input.shape), tuple(target.shape)))
+    return _LocalNcc.apply(input, target, int(window), float(eps))
+
+
 # --------------------------------------------------------------------------- displacement regulariser (row f4)
 FD_BOUNDARY = {"linear": 0, "neumann_zero": 1}       # LR_FD_LINEAR / LR_FD_NEUMANN_ZERO (mermaid FD modes)
 

@@ -135,6 +135,26 @@ def main():
     def k_fold_bwd8(s, st):
         _native.check(lib.lr_jacobian_fold_backward(vp(s["phi8"]), 8, *VOL, 0, vp(ncc_g), vp(s["gphi8"]), st), "fold_bwd8")
 
+    lncc_sum = torch.zeros(8, device=dev, dtype=torch.float64)
+    lncc_ws = torch.empty(lib.lr_local_ncc_workspace_bytes(8 if "lncc_bwd8" in which else 1, *VOL, 9), device=dev, dtype=torch.uint8)
+
+    def k_lncc(s, st):         # local NCC forward, w = 9: one pass over two volumes
+        _native.check(lib.lr_local_ncc_sum(vp(s["moving"]), vp(s["mu"]), 1, *VOL, 9, 1e-5, vp(lncc_sum), st), "lncc")
+
+    def k_lncc_bwd(s, st):     # local NCC adjoint, w = 9: coefficient pass (x, y -> 12 B workspace) + box-sum pass
+        _native.check(lib.lr_local_ncc_backward(vp(s["moving"]), vp(s["mu"]), 1, *VOL, 9, 1e-5, vp(ncc_g), vp(s["gvol"]),
+                                                vp(lncc_ws), lncc_ws.numel(), st), "lncc_bwd")
+
+    if "lncc_bwd8" in which:
+        for i, s_ in enumerate(sets):
+            s_["x8"] = torch.from_numpy(rs.uniform(-1, 1, (8, 1) + VOL).astype(np.float32)).to(dev)
+            s_["y8"] = torch.from_numpy(rs.uniform(-1, 1, (8, 1) + VOL).astype(np.float32)).to(dev)
+            s_["g8"] = torch.empty((8, 1) + VOL, device=dev)
+
+    def k_lncc_bwd8(s, st):
+        _native.check(lib.lr_local_ncc_backward(vp(s["x8"]), vp(s["y8"]), 8, *VOL, 9, 1e-5, vp(ncc_g), vp(s["g8"]),
+                                                vp(lncc_ws), lncc_ws.numel(), st), "lncc_bwd8")
+
     if "labels2" in which or "labels6" in which:
         # label maps as a validation item has them: mostly background, a few organ-sized blobs, target = shifted pred
         zz, yy, xx = np.meshgrid(*[np.arange(n) for n in VOL], indexing="ij")
@@ -161,7 +181,8 @@ def main():
         _native.check(lib.lr_identity_map(*VOL, vp(s["gphi"]), st), "idmap")
 
     units = {"atten": (k_atten, nv, 8 * nv), "idmap": (k_idmap, nv, 12 * nv), "reg": (k_reg, nv, 12 * nv), "jac": (k_jac, nv, 12 * nv), "jac_map": (k_jac_map, nv, 16 * nv),
-             "labels2": (k_labels(2), nv, 8 * nv), "labels6": (k_labels(6), nv, 8 * nv), "reg_bwd": (k_reg_bwd, nv, 24 * nv), "fold_bwd": (k_fold_bwd, nv, 24 * nv), "fold_bwd8": (k_fold_bwd8, 8 * nv, 8 * 24 * nv), "ncc": (k_ncc, nv, 8 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
+             "labels2": (k_labels(2), nv, 8 * nv), "labels6": (k_labels(6), nv, 8 * nv), "reg_bwd": (k_reg_bwd, nv, 24 * nv), "fold_bwd": (k_fold_bwd, nv, 24 * nv), "fold_bwd8": (k_fold_bwd8, 8 * nv, 8 * 24 * nv), "ncc": (k_ncc, nv, 8 * nv), "lncc": (k_lncc, nv, 8 * nv), "lncc_bwd": (k_lncc_bwd, nv, 44 * nv),
+             "lncc_bwd8": (k_lncc_bwd8, 8 * nv, 8 * 44 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
              "pca_bwd": (k_pca_bwd, 3 * nv, 4 * 3 * nv * 56 + 4 * 3 * nv), "warp_bwd": (k_warp_bwd, nv, 32 * nv),
              "drr_bwd": (k_drr_bwd, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240), "backproject": (k_backproject, batch * P * nv, batch * (4 * P * nv + 4 * P * DET[0] * DET[1])),
              "drr": (k_drr, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240),
