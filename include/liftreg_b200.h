@@ -366,6 +366,35 @@ LR_API int lr_local_ncc_backward(const float *x, const float *y, int B, int D, i
                                  const float *grad_loss, float *grad_x, void *workspace, size_t workspace_bytes,
                                  lr_stream_t stream);
 
+/* ---- soft Dice of the warped label map (a training term; PARITY UNPINNED: the reference has none) -------------------
+ * VoxelMorph's semi-supervised Dice term (one-hot moving labels, trilinear warp, 1 - soft Dice) without the one-hot
+ * channels.  phi (B,3,D,H,W) float32 in [-1,1], channel c addressing volume axis c (lr_warp_forward's convention);
+ * src (moving) and tgt (target) (B,D,H,W) float32 label maps; 2 <= L <= 128.  A value that is not an integer in [0, L)
+ * (negative, >= L, fractional, NaN) is "no label", as in lr_label_confusion.
+ * Sampling is lr_warp_forward's with zeros padding and no using_scale, bit for bit: per axis i = (g+1)*((S-1)/2) in
+ * fp32, clamp_index, floor; fractions w1 = i - floor(i), w0 = (floor(i)+1) - i; the weight of tap (tx,ty,tz) is the fp32
+ * product (wx*wy)*wz.  A tap outside the volume carries no label.  Nothing depends on lr_set_numerics.
+ * Per item b and label l, over all voxels v and their 8 taps t with weight w_t(v):
+ *   P[b,l] = sum_v sum_t w_t(v) [src(t) = l]                 (soft size of the warped label)
+ *   I[b,l] = sum_v sum_t w_t(v) [src(t) = l] [tgt(v) = l]    (soft overlap)
+ *   T[b,l] = #{v : tgt(v) = l}
+ *   S_b = {l in [1, L) : P + T > 0}  (background excluded);  dice_b = mean over S_b of 2 I / (P + T)  (1 if S_b is empty);
+ *   loss = 1 - mean_b dice_b.
+ * lr_label_dice_sums: sums (B,L,3) float64 = [I, P, T], zeroed by the call; I and P accumulate in fp64 from the fp32
+ *   weights (the atomic order varies, so the last bits may differ between calls), T is exact.
+ * lr_label_dice_backward: grad_phi (B,3,D,H,W) is OVERWRITTEN with grad_loss[0] * d loss / d phi (grad_loss: one float in
+ *   device memory), from the sums of lr_label_dice_sums; the labels are data.  With a = d loss / d P, e = d loss / d I
+ *   (both 0 for l not in S_b) and s_c = (S_c - 1)/2:
+ *     grad_phi_c(v) = grad_loss * s_c * sum_t d w_t / d i_c * (a[b, src_t] + [src_t = tgt(v)] * e[b, src_t])
+ *   over the in-bounds taps with a label.  a and a + e are formed in fp64 (grad_loss and 1/B folded in) and rounded
+ *   once to fp32; the sum is evaluated as a tree over tap differences, so it is exactly 0 where the 8 taps carry one
+ *   coefficient.  Each element is written once, without atomics: the same sums give the same bits.
+ * Arguments: no null pointer; every axis >= 1 and < 2^21; B*3*D*H*W < 2^31; 2 <= L <= 128. */
+LR_API int lr_label_dice_sums(const float *phi, const float *src, const float *tgt, int B, int D, int H, int W, int L,
+                              double *sums, lr_stream_t stream);
+LR_API int lr_label_dice_backward(const float *phi, const float *src, const float *tgt, int B, int D, int H, int W, int L,
+                                  const double *sums, const float *grad_loss, float *grad_phi, lr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -160,6 +160,16 @@ int check_launch(const char *what);  // cudaGetLastError -> lr_status; bumps the
 int sm_count();                      // multiprocessors of the current device (cached per device)
 int numerics_mode();                 // LR_NUMERICS_FAST / LR_NUMERICS_EXACT (lr_set_numerics)
 inline cudaStream_t as_stream(lr_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }
+
+// ATen grid_sampler_unnormalize(align_corners) then optional clip_coordinates: the sample coordinate of the warp, and
+// of every kernel that samples as the warp does.
+template <int PAD>
+__device__ __forceinline__ float source_index(float g, float half_sm1, float sm1) {
+    // ((g+1)/2)*(S-1) == RN(RN(g+1) * ((S-1)/2)): /2 is exact and (S-1)/2 is representable.
+    float i = mul_rn(add_rn(g, 1.0f), half_sm1);
+    if (PAD == LR_PAD_BORDER) i = fminf(sm1, fmaxf(i, 0.0f));
+    return i;
+}
 }  // namespace lr
 
 #define LR_REQUIRE(cond, ...)                \

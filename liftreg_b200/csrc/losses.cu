@@ -842,6 +842,14 @@ __device__ __forceinline__ int label_key(float p, float t, int L, float fL) {
     return ok ? (__float_as_int(tp) - 0x4B400000) * L + (__float_as_int(tt) - 0x4B400000) : L * L;
 }
 
+// the same test for one value: its label l if it is an integer in [0, L), else -1.  (Written out again rather than
+// called from label_key, which then compiles differently.)
+__device__ __forceinline__ int label_of(float v, float fL) {
+    const float M = 12582912.0f;
+    const float t = __fadd_rn(v, M);
+    return v >= 0.0f && v < fL && __fsub_rn(t, M) == v ? __float_as_int(t) - 0x4B400000 : -1;
+}
+
 // one key per lane (key < 0: lane has nothing), called by the whole warp
 __device__ __forceinline__ void hist_add_warp(unsigned *__restrict__ h, int key, int lane) {
     const int k0 = __shfl_sync(0xffffffffu, key, 0);
@@ -1041,6 +1049,207 @@ __global__ void __launch_bounds__(LNCC_THREADS) local_ncc_kernel(const float *__
         }
     }
     if (KIND == LNCC_FWD) block_accumulate_f64(acc, sum + b);
+}
+
+// ---- soft Dice of the trilinearly warped label map, a training term (include/liftreg_b200.h; PARITY UNPINNED) ----------
+// VoxelMorph's semi-supervised term without its L one-hot channels: a voxel's soft probability of label l is the total
+// weight of its 8 taps whose moving label is l, so the sums need only the tap weights keyed by the tap's label, and the
+// adjoint one coefficient per tap (a[l], or a[l] + e[l] where the tap's label is the target's).  Both kernels march a
+// chunk of planes of a 32 x 8 tile of (last, second) axis positions, one voxel per thread; neither cost depends on L.
+constexpr int DICE_TX = 32, DICE_TY = 8, DICE_THREADS = DICE_TX * DICE_TY, DICE_LMAX = 128;
+static_assert(DICE_THREADS >= DICE_LMAX, "the adjoint derives one label's coefficients per thread");
+
+struct DiceDims {
+    RegDims m;                // d, h, w and the chunking of the first axis (march_dims)
+    float hx, hy, hz;         // (S-1)/2 per axis, the warp's unnormalisation
+    float cx, cy, cz;         // (S-1) + 2, the warp's clamp_index bound under zeros padding
+    int L;
+};
+
+// The sample position of voxel `vox` of an item under its map phi_b exactly as lr_warp_forward computes it (zeros
+// padding, no using_scale): the fractions w?[0] (lower tap) and w?[1] (upper tap) of each axis, and the label of each
+// of the 8 taps, t = tx + 2 ty + 4 tz (-1: outside the volume, or no label).
+__device__ __forceinline__ void dice_taps(const float *__restrict__ phi_b, const float *__restrict__ src_b, const DiceDims &g,
+                                          unsigned vox, unsigned N, float fL, float (&wx)[2], float (&wy)[2], float (&wz)[2],
+                                          int (&lab)[8]) {
+    // channel c of phi addresses volume axis c
+    const float iz = clamp_index(source_index<LR_PAD_ZEROS>(ld_stream(phi_b + vox), g.hz, 0.0f), g.cz);
+    const float iy = clamp_index(source_index<LR_PAD_ZEROS>(ld_stream(phi_b + N + vox), g.hy, 0.0f), g.cy);
+    const float ix = clamp_index(source_index<LR_PAD_ZEROS>(ld_stream(phi_b + 2u * N + vox), g.hx, 0.0f), g.cx);
+    float fx, fy, fz;
+    int x0, y0, z0;
+    floor_fi(ix, fx, x0);
+    floor_fi(iy, fy, y0);
+    floor_fi(iz, fz, z0);
+    wx[0] = sub_rn(add_rn(fx, 1.0f), ix); wx[1] = sub_rn(ix, fx);
+    wy[0] = sub_rn(add_rn(fy, 1.0f), iy); wy[1] = sub_rn(iy, fy);
+    wz[0] = sub_rn(add_rn(fz, 1.0f), iz); wz[1] = sub_rn(iz, fz);
+    const int W = g.m.w, HW = g.m.h * g.m.w;
+    const int base = z0 * HW + y0 * W + x0;                   // may be negative: only in-bounds taps are read
+#pragma unroll
+    for (int t = 0; t < 8; ++t) {
+        const int tx = t & 1, ty = (t >> 1) & 1, tz = t >> 2;
+        const bool ok = (unsigned)(x0 + tx) < (unsigned)W && (unsigned)(y0 + ty) < (unsigned)g.m.h && (unsigned)(z0 + tz) < (unsigned)g.m.d;
+        lab[t] = ok ? label_of(__ldg(src_b + (base + tx + ty * W + tz * HW)), fL) : -1;
+    }
+}
+
+// end-of-thread flush of the run accumulators into the block's bins: one shared atomic per warp when every lane holds
+// the same label (the common case), else one per lane
+__device__ __forceinline__ void dice_flush(int kp, double ap, double ai, int kt, unsigned at, double *sp, double *si,
+                                           unsigned *st, int lane) {
+    const int p0 = __shfl_sync(0xffffffffu, kp, 0);
+    if (__all_sync(0xffffffffu, kp == p0)) {
+        ap = warp_sum(ap); ai = warp_sum(ai);
+        if (lane == 0 && p0 >= 0) { atomicAdd(sp + p0, ap); atomicAdd(si + p0, ai); }
+    } else if (kp >= 0) {
+        atomicAdd(sp + kp, ap); atomicAdd(si + kp, ai);
+    }
+    const int t0 = __shfl_sync(0xffffffffu, kt, 0);
+    if (__all_sync(0xffffffffu, kt == t0)) {
+        const unsigned n = __reduce_add_sync(0xffffffffu, at);
+        if (lane == 0 && t0 >= 0) atomicAdd(st + t0, n);
+    } else if (kt >= 0) {
+        atomicAdd(st + kt, at);
+    }
+}
+
+// Forward: sums[b][l] = {I, P, T}.  Each thread keeps run accumulators for the last tap label (P and I, fp64 from the
+// fp32 tap weights) and the last target label (T, an integer count) and flushes a run to the block's shared bins when
+// the label changes; label maps are mostly large regions, so a thread marching planes rarely does.  The block then adds
+// each non-empty bin to sums with one fp64 atomic.
+__global__ void __launch_bounds__(DICE_THREADS) label_dice_sums_kernel(const float *__restrict__ phi, const float *__restrict__ src,
+                                                                      const float *__restrict__ tgt, DiceDims g, double *__restrict__ sums) {
+    __shared__ double sp[DICE_LMAX], si[DICE_LMAX];
+    __shared__ unsigned st[DICE_LMAX];
+    const int tid = threadIdx.x, lane = tid & 31;
+    for (int l = tid; l < g.L; l += DICE_THREADS) { sp[l] = 0.0; si[l] = 0.0; st[l] = 0u; }
+    __syncthreads();
+    const int x = blockIdx.x * DICE_TX + lane, y = blockIdx.y * DICE_TY + (tid >> 5);
+    const int zc = blockIdx.z % g.m.n_zchunks, b = blockIdx.z / g.m.n_zchunks;
+    const int z0 = zc * g.m.zchunk, z1 = min(g.m.d, z0 + g.m.zchunk);
+    const float fL = (float)g.L;
+    int kp = -1, kt = -1;
+    double ap = 0.0, ai = 0.0;
+    unsigned at = 0u;
+    if (x < g.m.w && y < g.m.h) {
+        const unsigned plane = (unsigned)g.m.h * (unsigned)g.m.w, N = plane * (unsigned)g.m.d;     // B*3*N < 2^31
+        const float *phi_b = phi + 3u * (unsigned)b * N, *src_b = src + (unsigned)b * N, *tgt_b = tgt + (unsigned)b * N;
+        unsigned vox = (unsigned)z0 * plane + (unsigned)y * (unsigned)g.m.w + (unsigned)x;
+        for (int z = z0; z < z1; ++z, vox += plane) {
+            float wx[2], wy[2], wz[2];
+            int lab[8];
+            dice_taps(phi_b, src_b, g, vox, N, fL, wx, wy, wz, lab);
+            const int lt = label_of(ld_stream(tgt_b + vox), fL);
+            if (lt != kt) {
+                if (kt >= 0) atomicAdd(st + kt, at);
+                kt = lt; at = 0u;
+            }
+            ++at;
+            // the weights of warp_one: (wx * wy) * wz
+            const float a00 = mul_rn(wx[0], wy[0]), a10 = mul_rn(wx[1], wy[0]), a01 = mul_rn(wx[0], wy[1]), a11 = mul_rn(wx[1], wy[1]);
+            const float wt[8] = {mul_rn(a00, wz[0]), mul_rn(a10, wz[0]), mul_rn(a01, wz[0]), mul_rn(a11, wz[0]),
+                                 mul_rn(a00, wz[1]), mul_rn(a10, wz[1]), mul_rn(a01, wz[1]), mul_rn(a11, wz[1])};
+#pragma unroll
+            for (int t = 0; t < 8; ++t) {
+                const int l = lab[t];
+                if (l < 0) continue;
+                if (l != kp) {
+                    if (kp >= 0) { atomicAdd(sp + kp, ap); atomicAdd(si + kp, ai); }
+                    kp = l; ap = 0.0; ai = 0.0;
+                }
+                const double w = (double)wt[t];
+                ap += w;
+                if (l == lt) ai += w;
+            }
+        }
+    }
+    dice_flush(kp, ap, ai, kt, at, sp, si, st, lane);
+    __syncthreads();
+    double *s = sums + (size_t)b * g.L * 3;
+    for (int l = tid; l < g.L; l += DICE_THREADS) {
+        if (si[l] != 0.0) atomicAdd(s + 3 * l, si[l]);
+        if (sp[l] != 0.0) atomicAdd(s + 3 * l + 1, sp[l]);
+        if (st[l] != 0u) atomicAdd(s + 3 * l + 2, (double)st[l]);
+    }
+}
+
+// Adjoint.  loss = 1 - (1/B) sum_b (1/|S_b|) sum_{l in S_b} 2 I / (P + T), so per label of S_b
+//     a = d loss / d P = 2 I / (B |S_b| (P + T)^2),   e = d loss / d I = -2 / (B |S_b| (P + T)),
+// both times grad_loss, formed in fp64 and rounded once to fp32 (a, and a + e for the taps whose label is the
+// target's).  The block derives them for its item into shared memory; then each thread gathers the 8 taps of its voxel
+// and evaluates d/di_c of the trilinear blend of the tap coefficients as the warp's d/dphi does: a tree of fused lerps
+// over tap differences, so a voxel whose 8 coefficients are equal gets exactly 0.  Each output is written once.
+__global__ void __launch_bounds__(DICE_THREADS) label_dice_backward_kernel(const float *__restrict__ phi, const float *__restrict__ src,
+                                                                          const float *__restrict__ tgt, DiceDims g, int B,
+                                                                          const double *__restrict__ sums,
+                                                                          const float *__restrict__ grad_loss,
+                                                                          float *__restrict__ grad_phi) {
+    __shared__ float sa[DICE_LMAX], sae[DICE_LMAX];
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int zc = blockIdx.z % g.m.n_zchunks, b = blockIdx.z / g.m.n_zchunks;
+    const double *s = sums + (size_t)b * g.L * 3;
+    double I = 0.0, den = 0.0;
+    bool in = false;                                          // l in S_b: l >= 1 and P + T > 0
+    if (tid >= 1 && tid < g.L) {
+        I = s[3 * tid]; den = s[3 * tid + 1] + s[3 * tid + 2];
+        in = den > 0.0;
+    }
+    const int n_in = __syncthreads_count(in);
+    if (tid < g.L) {
+        double a = 0.0, e = 0.0;
+        if (in) {
+            const double k = 2.0 * (double)grad_loss[0] / ((double)B * (double)n_in);
+            a = k * I / (den * den);
+            e = -k / den;
+        }
+        sa[tid] = (float)a;
+        sae[tid] = (float)(a + e);
+    }
+    __syncthreads();
+    const int x = blockIdx.x * DICE_TX + lane, y = blockIdx.y * DICE_TY + (tid >> 5);
+    if (x >= g.m.w || y >= g.m.h) return;
+    const int z0 = zc * g.m.zchunk, z1 = min(g.m.d, z0 + g.m.zchunk);
+    const float fL = (float)g.L;
+    const unsigned plane = (unsigned)g.m.h * (unsigned)g.m.w, N = plane * (unsigned)g.m.d;
+    const float *phi_b = phi + 3u * (unsigned)b * N, *src_b = src + (unsigned)b * N, *tgt_b = tgt + (unsigned)b * N;
+    float *gp = grad_phi + 3u * (unsigned)b * N;
+    unsigned vox = (unsigned)z0 * plane + (unsigned)y * (unsigned)g.m.w + (unsigned)x;
+    for (int z = z0; z < z1; ++z, vox += plane) {
+        float wx[2], wy[2], wz[2];
+        int lab[8];
+        dice_taps(phi_b, src_b, g, vox, N, fL, wx, wy, wz, lab);
+        const int lt = label_of(ld_stream(tgt_b + vox), fL);
+        float v[8];
+#pragma unroll
+        for (int t = 0; t < 8; ++t) {
+            const int l = max(lab[t], 0);
+            const float c = lab[t] == lt ? sae[l] : sa[l];
+            v[t] = lab[t] < 0 ? 0.0f : c;
+        }
+        // d/di_c = sum over the 4 tap pairs along axis c of (upper - lower coefficient) * (the pair's weight in the other
+        // two axes).  The differences come first, so equal coefficients give exactly 0; the pair weights are the fp32
+        // fractions' products (not the lerp form of the warp's d/dphi, whose implied 1 - w differs from w0), so each
+        // rounding is relative to a term of the abs-scale (DESIGN.md section 3)
+        float gxyz[3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {                         // c: 0 = x (last axis), 1 = y, 2 = z
+            const int step = 1 << c;                          // tap index step along axis c
+            float acc = 0.0f;
+#pragma unroll
+            for (int p = 0; p < 4; ++p) {
+                const int lo = c == 0 ? 2 * p : (c == 1 ? (p & 1) + 4 * (p >> 1) : p);       // lower tap of pair p
+                const int tx = lo & 1, ty = (lo >> 1) & 1, tz = lo >> 2;
+                const float w = c == 0 ? mul_rn(wy[ty], wz[tz]) : (c == 1 ? mul_rn(wx[tx], wz[tz]) : mul_rn(wx[tx], wy[ty]));
+                const float d = sub_rn(v[lo + step], v[lo]);
+                acc = p == 0 ? mul_rn(w, d) : fma_rn(w, d, acc);
+            }
+            gxyz[c] = acc;
+        }
+        st_stream(gp + vox, mul_rn(g.hz, gxyz[2]));
+        st_stream(gp + N + vox, mul_rn(g.hy, gxyz[1]));
+        st_stream(gp + 2u * N + vox, mul_rn(g.hx, gxyz[0]));
+    }
 }
 
 }  // namespace lr
@@ -1272,4 +1481,47 @@ extern "C" int lr_local_ncc_backward(const float *x, const float *y, int B, int 
     float *coef = static_cast<float *>(workspace);
     if (int e = lncc_launch<LNCC_COEF>(x, y, nullptr, B, D, H, W, win, eps, nullptr, nullptr, coef, st, "local_ncc_kernel<coef>")) return e;
     return lncc_launch<LNCC_GRAD>(x, y, coef, B, D, H, W, win, eps, grad_loss, nullptr, grad_x, st, "local_ncc_kernel<grad>");
+}
+
+// argument rules shared by the Dice entries (the warp's size limits); 0 when they hold
+static int dice_check(const char *who, int B, int D, int H, int W, int L) {
+    LR_REQUIRE(L >= 2 && L <= DICE_LMAX, "%s: number of labels L=%d must be in [2, %d]", who, L, DICE_LMAX);
+    LR_REQUIRE(B >= 1 && D >= 1 && H >= 1 && W >= 1, "%s: every axis needs >= 1 entry (B=%d, %dx%dx%d)", who, B, D, H, W);
+    LR_REQUIRE(D < (1 << 21) && H < (1 << 21) && W < (1 << 21), "%s: D, H and W must be < 2^21 (%dx%dx%d)", who, D, H, W);
+    LR_REQUIRE((int64_t)B * 3 * D * H * W < ((int64_t)1 << 31),
+               "%s: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)", who, B, D, H, W);
+    return 0;
+}
+
+template <typename K>
+static int dice_dims(K kernel, const char *who, int B, int D, int H, int W, int L, DiceDims &g, dim3 &grid) {
+    LR_REQUIRE(march_dims(kernel, DICE_THREADS, DICE_TX, DICE_TY, LR_REG_WAVES, B, D, H, W, g.m, grid) == 0,
+               "%s: too many blocks for one launch (B=%d, %dx%dx%d)", who, B, D, H, W);
+    g.hx = (float)(W - 1) / 2.0f; g.hy = (float)(H - 1) / 2.0f; g.hz = (float)(D - 1) / 2.0f;
+    g.cx = (float)(W - 1) + 2.0f; g.cy = (float)(H - 1) + 2.0f; g.cz = (float)(D - 1) + 2.0f;
+    g.L = L;
+    return 0;
+}
+
+extern "C" int lr_label_dice_sums(const float *phi, const float *src, const float *tgt, int B, int D, int H, int W, int L,
+                                  double *sums, lr_stream_t stream) {
+    LR_REQUIRE(phi && src && tgt && sums, "label_dice_sums: null pointer");
+    if (int e = dice_check("label_dice_sums", B, D, H, W, L)) return e;
+    DiceDims g; dim3 grid;
+    if (int e = dice_dims(label_dice_sums_kernel, "label_dice_sums", B, D, H, W, L, g, grid)) return e;
+    cudaStream_t st = as_stream(stream);
+    cudaError_t ce = cudaMemsetAsync(sums, 0, sizeof(double) * 3 * (size_t)B * L, st);
+    if (ce != cudaSuccess) { set_error("label_dice_sums: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    label_dice_sums_kernel<<<grid, DICE_THREADS, 0, st>>>(phi, src, tgt, g, sums);
+    return check_launch("label_dice_sums_kernel");
+}
+
+extern "C" int lr_label_dice_backward(const float *phi, const float *src, const float *tgt, int B, int D, int H, int W, int L,
+                                      const double *sums, const float *grad_loss, float *grad_phi, lr_stream_t stream) {
+    LR_REQUIRE(phi && src && tgt && sums && grad_loss && grad_phi, "label_dice_backward: null pointer");
+    if (int e = dice_check("label_dice_backward", B, D, H, W, L)) return e;
+    DiceDims g; dim3 grid;
+    if (int e = dice_dims(label_dice_backward_kernel, "label_dice_backward", B, D, H, W, L, g, grid)) return e;
+    label_dice_backward_kernel<<<grid, DICE_THREADS, 0, as_stream(stream)>>>(phi, src, tgt, g, B, sums, grad_loss, grad_phi);
+    return check_launch("label_dice_backward_kernel");
 }

@@ -51,15 +51,6 @@ struct WarpDims {
     float zero;          // +0.0f the compiler cannot constant-fold (see mul2_sep)
 };
 
-// ATen grid_sampler_unnormalize(align_corners) then optional clip_coordinates.
-template <int PAD>
-__device__ __forceinline__ float source_index(float g, float half_sm1, float sm1) {
-    // ((g+1)/2)*(S-1) == RN(RN(g+1) * ((S-1)/2)): /2 is exact and (S-1)/2 is representable.
-    float i = mul_rn(add_rn(g, 1.0f), half_sm1);
-    if (PAD == LR_PAD_BORDER) i = fminf(sm1, fmaxf(i, 0.0f));
-    return i;
-}
-
 // net_utils.py:81-85 with numpy>=2 casting: fp32(float64(idx)*spacing) * 2 - 1
 __device__ __forceinline__ float identity_coord(int idx, double spacing) {
     float v = __double2float_rn((double)idx * spacing);

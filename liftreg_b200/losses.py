@@ -63,7 +63,12 @@ class SubspaceLoss(nn.Module):
     mermaid's finite differences ("linear" = FD_torch's default).
 
     Opt key `fold_factor` (default 0, not in the reference): when > 0, `fold_factor * ops.fold_penalty(phi)` is added to
-    the total, with phi = params + identity (the model's `disp_field + id_transform`), and reported as "fold_loss"."""
+    the total, with phi = params + identity (the model's `disp_field + id_transform`), and reported as "fold_loss".
+
+    Opt keys `dice_factor` (default 0) and `dice_num_labels` (default 2: background and lung mask), not in the reference:
+    when dice_factor > 0, `dice_factor * ops.label_dice_loss(phi, input["source_label"], input["target_label"],
+    dice_num_labels)` is added to the total and reported as "dice_loss" (label-supervised training; both label maps
+    must be in the input).  phi is formed once when both terms are on."""
 
     def __init__(self, opt=None, sim=None, fd_boundary="linear"):
         super().__init__()
@@ -73,26 +78,36 @@ class SubspaceLoss(nn.Module):
         self.min_reg_factor = _opt(opt, 'min_reg_factor', 1e-3)
         self.reg_factor_decay_from = _opt(opt, 'reg_factor_decay_from', 10)
         self.fold_factor = _opt(opt, 'fold_factor', 0)
+        self.dice_factor = _opt(opt, 'dice_factor', 0)
+        self.dice_num_labels = _opt(opt, 'dice_num_labels', 2)
         self.fd_boundary = fd_boundary
         self._identity = {}
 
     def forward(self, input):
+        if self.dice_factor > 0:          # a missing label map fails before any work is done
+            labels = input["source_label"], input["target_label"]
         sim_loss = self.sim(input["warped"], input["target"])
         reg_loss = self.compute_reg_loss(input["params"])
         total_loss = self.sim_factor * sim_loss + self.get_reg_factor(input["epoch"]) * reg_loss
         out = {"total_loss": total_loss, "sim_loss": sim_loss.item(), "reg_loss": reg_loss.item()}
+        if self.fold_factor > 0 or self.dice_factor > 0:
+            phi = self.deformation_map(input["params"])
         if self.fold_factor > 0:
-            fold_loss = self.compute_fold_loss(input["params"])
-            out["total_loss"] = total_loss + self.fold_factor * fold_loss
+            fold_loss = ops.fold_penalty(phi, self.fd_boundary)
+            out["total_loss"] = out["total_loss"] + self.fold_factor * fold_loss
             out["fold_loss"] = fold_loss.item()
+        if self.dice_factor > 0:
+            dice_loss = ops.label_dice_loss(phi, *labels, self.dice_num_labels)
+            out["total_loss"] = out["total_loss"] + self.dice_factor * dice_loss
+            out["dice_loss"] = dice_loss.item()
         return out
 
-    def compute_fold_loss(self, disp):
-        """mean over (B, D, H, W) of max(0, -det J) of the map disp + identity (ops.fold_penalty)"""
+    def deformation_map(self, disp):
+        """the map disp + identity (the model's `disp_field + id_transform`), with the identity cached per shape and device"""
         key = (tuple(disp.shape[2:]), disp.device)
         if key not in self._identity:
             self._identity[key] = ops.identity_map(disp.shape[2:], disp.device)
-        return ops.fold_penalty(disp + self._identity[key], self.fd_boundary)
+        return disp + self._identity[key]
 
     def get_reg_factor(self, epoch):
         """:40-49"""

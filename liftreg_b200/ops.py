@@ -608,3 +608,73 @@ def label_confusion(pred, target, num_labels):
         _native.check(_native.lib().lr_label_confusion(_ptr(pred), _ptr(target), B, N, L, _ptr(counts), _ptr(invalid),
                                                        _stream()), "lr_label_confusion")
     return counts, invalid
+
+
+# --------------------------------------------------------------------------- soft Dice of the warped labels (training term)
+def _dice_loss_from_sums(sums):
+    """1 - mean_b of the mean over S_b = {l >= 1 : P + T > 0} of 2 I / (P + T) (1 where S_b is empty), from sums
+    (B,L,3) float64 = [I, P, T]; float64 on the sums' device, no host synchronisation"""
+    I, P, T = sums.unbind(-1)
+    den = P + T
+    in_s = den > 0
+    in_s[:, 0] = False
+    n = in_s.sum(1)
+    dice_l = torch.where(in_s, 2.0 * I / torch.where(in_s, den, 1.0), 0.0)
+    dice = torch.where(n > 0, dice_l.sum(1) / n.clamp(min=1), 1.0)
+    return 1.0 - dice.mean()
+
+
+class _LabelDice(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, phi, src, tgt, num_labels):
+        phi = _need_cuda_f32(phi, "phi")
+        B, _, D, H, W = phi.shape
+        sums = torch.empty((B, num_labels, 3), device=phi.device, dtype=torch.float64)
+        with torch.cuda.device(phi.device):
+            _native.check(_native.lib().lr_label_dice_sums(_ptr(phi), _ptr(src), _ptr(tgt), B, D, H, W, num_labels, _ptr(sums),
+                                                           _stream()), "lr_label_dice_sums")
+        ctx.save_for_backward(phi, src, tgt, sums)
+        return _dice_loss_from_sums(sums).to(torch.float32)
+
+    @staticmethod
+    def backward(ctx, grad_loss):
+        phi, src, tgt, sums = ctx.saved_tensors
+        B, _, D, H, W = phi.shape
+        g = grad_loss.to(device=phi.device, dtype=torch.float32).reshape(1).contiguous()
+        gphi = torch.empty_like(phi)
+        with torch.cuda.device(phi.device):
+            _native.check(_native.lib().lr_label_dice_backward(_ptr(phi), _ptr(src), _ptr(tgt), B, D, H, W, sums.shape[1],
+                                                               _ptr(sums), _ptr(g), _ptr(gphi), _stream()),
+                          "lr_label_dice_backward")
+        return gphi, None, None, None
+
+
+def label_dice_loss(phi, source_labels, target_labels, num_labels):
+    """Soft Dice loss of the moving label map warped trilinearly by phi, against the target labels: VoxelMorph's
+    semi-supervised term (one-hot labels, trilinear warp with zeros padding, 1 - soft Dice) without materialising the
+    one-hot channels.  1 - mean_b of the mean Dice over the labels 1..L-1 present in either map (definition:
+    include/liftreg_b200.h, lr_label_dice_sums).
+
+    phi (B,3,D,H,W) CUDA float32 in [-1,1] (channel c addresses volume axis c, as ops.warp); label maps (B,1,D,H,W) or
+    (B,D,H,W), float32 or an integer dtype (converted with .float()); a value that is not an integer in
+    [0, num_labels) counts as no label.  2 <= num_labels <= 128.  A float32 scalar on phi's device, computed without a
+    host synchronisation; differentiable wrt phi (the labels are data).  The reference has no such term, so parity is
+    unpinned."""
+    if not isinstance(phi, torch.Tensor) or phi.dim() != 5 or phi.shape[1] != 3:
+        raise ValueError("phi must be a (B,3,D,H,W) tensor, got %s"
+                         % (tuple(phi.shape) if isinstance(phi, torch.Tensor) else type(phi).__name__,))
+    L = int(num_labels)
+    if not 2 <= L <= 128:
+        raise ValueError("num_labels must be in [2, 128], got %d" % L)
+    want = (phi.shape[0],) + tuple(phi.shape[2:])
+    maps = []
+    for t, name in ((source_labels, "source_labels"), (target_labels, "target_labels")):
+        t = _label_map(t, name)
+        if t.dim() == 5 and t.shape[1] == 1:
+            t = t[:, 0]
+        if tuple(t.shape) != want:
+            raise ValueError("%s must be (B,1,D,H,W) or (B,D,H,W) with (B,D,H,W) = %s, got %s" % (name, want, tuple(t.shape)))
+        if t.device != phi.device:
+            raise ValueError("%s must be on phi's device %s (got %s)" % (name, phi.device, t.device))
+        maps.append(t.contiguous())
+    return _LabelDice.apply(phi, maps[0], maps[1], L)

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Quick per-kernel timing loop for kernel development (not the contract benchmark -- that is bench.py).
 
-    python tools/kbench.py [warp] [backproject] [drr] [--iters N]
+    python tools/kbench.py [warp] [backproject] [drr] [--iters N] [--labels L]
 
 Times each kernel at the cfg2 / cfg1 sizes with rotating buffers (cold L2) under a CUDA graph and prints us per launch."""
 import ctypes
@@ -29,6 +29,11 @@ def main():
     if "--batch" in args:        # batch items per launch for warp / backproject (BASELINE configs[2] uses 8)
         k = args.index("--batch")
         batch = int(args[k + 1])
+        del args[k:k + 2]
+    n_labels = 2
+    if "--labels" in args:       # labels of the dice entries: 2 or 6
+        k = args.index("--labels")
+        n_labels = int(args[k + 1])
         del args[k:k + 2]
     which = args or ["warp", "backproject", "drr"]
     dev = torch.device("cuda:0")
@@ -125,7 +130,7 @@ def main():
     def k_fold_bwd(s, st):     # d fold / d phi (folding penalty adjoint): reads phi, writes grad_phi
         _native.check(lib.lr_jacobian_fold_backward(vp(s["phi"]), 1, *VOL, 0, vp(ncc_g), vp(s["gphi"]), st), "fold_bwd")
 
-    if "fold_bwd8" in which:
+    if "fold_bwd8" in which or "dice_bwd8" in which:
         phi8 = [torch.from_numpy((synthetic.smooth_displacement(VOL, seed=b) + synthetic.identity_map_np(VOL))[None]).to(dev)
                 for b in range(8)]
         for i, s_ in enumerate(sets):
@@ -155,7 +160,8 @@ def main():
         _native.check(lib.lr_local_ncc_backward(vp(s["x8"]), vp(s["y8"]), 8, *VOL, 9, 1e-5, vp(ncc_g), vp(s["g8"]),
                                                 vp(lncc_ws), lncc_ws.numel(), st), "lncc_bwd8")
 
-    if "labels2" in which or "labels6" in which:
+    dice_names = ("dice", "dice_bwd", "dice_bwd8")
+    if "labels2" in which or "labels6" in which or any(n in which for n in dice_names):
         # label maps as a validation item has them: mostly background, a few organ-sized blobs, target = shifted pred
         zz, yy, xx = np.meshgrid(*[np.arange(n) for n in VOL], indexing="ij")
         for i, s_ in enumerate(sets):
@@ -166,6 +172,25 @@ def main():
                     lab[(zz - c[0]) ** 2 + (yy - c[1]) ** 2 + (xx - c[2]) ** 2 < 30 ** 2] = k
                 s_["pred%d" % L] = torch.from_numpy(lab).to(dev)
                 s_["target%d" % L] = torch.from_numpy(np.roll(lab, 3, axis=0)).to(dev)
+    if "dice_bwd8" in which:
+        for s_ in sets:
+            s_["src8"] = torch.stack([torch.roll(s_["pred%d" % n_labels], b, 0) for b in range(8)])
+            s_["tgt8"] = torch.stack([torch.roll(s_["target%d" % n_labels], b, 0) for b in range(8)])
+    dice_sums = torch.zeros((8, n_labels, 3), device=dev, dtype=torch.float64)
+    L_ = n_labels
+
+    def k_dice(s, st):         # soft Dice sums of the warped labels: phi, target labels and 8 moving-label taps per voxel
+        _native.check(lib.lr_label_dice_sums(vp(s["phi"]), vp(s["pred%d" % L_]), vp(s["target%d" % L_]), 1, *VOL, L_,
+                                             vp(dice_sums), st), "dice")
+
+    def k_dice_bwd(s, st):     # its adjoint: the same reads, grad_phi written
+        _native.check(lib.lr_label_dice_backward(vp(s["phi"]), vp(s["pred%d" % L_]), vp(s["target%d" % L_]), 1, *VOL, L_,
+                                                 vp(dice_sums), vp(ncc_g), vp(s["gphi"]), st), "dice_bwd")
+
+    def k_dice_bwd8(s, st):
+        _native.check(lib.lr_label_dice_backward(vp(s["phi8"]), vp(s["src8"]), vp(s["tgt8"]), 8, *VOL, L_, vp(dice_sums), vp(ncc_g),
+                                                 vp(s["gphi8"]), st), "dice_bwd8")
+
     conf_counts, conf_invalid = torch.zeros((1, 36), device=dev, dtype=torch.int64), torch.zeros(1, device=dev, dtype=torch.int64)
 
     def k_labels(L):           # confusion matrix of two label maps (validation overlap metrics)
@@ -182,7 +207,8 @@ def main():
 
     units = {"atten": (k_atten, nv, 8 * nv), "idmap": (k_idmap, nv, 12 * nv), "reg": (k_reg, nv, 12 * nv), "jac": (k_jac, nv, 12 * nv), "jac_map": (k_jac_map, nv, 16 * nv),
              "labels2": (k_labels(2), nv, 8 * nv), "labels6": (k_labels(6), nv, 8 * nv), "reg_bwd": (k_reg_bwd, nv, 24 * nv), "fold_bwd": (k_fold_bwd, nv, 24 * nv), "fold_bwd8": (k_fold_bwd8, 8 * nv, 8 * 24 * nv), "ncc": (k_ncc, nv, 8 * nv), "lncc": (k_lncc, nv, 8 * nv), "lncc_bwd": (k_lncc_bwd, nv, 44 * nv),
-             "lncc_bwd8": (k_lncc_bwd8, 8 * nv, 8 * 44 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
+             "lncc_bwd8": (k_lncc_bwd8, 8 * nv, 8 * 44 * nv), "dice": (k_dice, nv, 20 * nv), "dice_bwd": (k_dice_bwd, nv, 32 * nv),
+             "dice_bwd8": (k_dice_bwd8, 8 * nv, 8 * 32 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
              "pca_bwd": (k_pca_bwd, 3 * nv, 4 * 3 * nv * 56 + 4 * 3 * nv), "warp_bwd": (k_warp_bwd, nv, 32 * nv),
              "drr_bwd": (k_drr_bwd, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240), "backproject": (k_backproject, batch * P * nv, batch * (4 * P * nv + 4 * P * DET[0] * DET[1])),
              "drr": (k_drr, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240),
