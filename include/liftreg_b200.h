@@ -395,6 +395,31 @@ LR_API int lr_label_dice_sums(const float *phi, const float *src, const float *t
 LR_API int lr_label_dice_backward(const float *phi, const float *src, const float *tgt, int B, int D, int H, int W, int L,
                                   const double *sums, const float *grad_loss, float *grad_phi, lr_stream_t stream);
 
+/* ---- normalized gradient field (NGF) similarity (PARITY UNPINNED) ---------------------------------------------------
+ * The reference's layers/losses.py names an NGFLoss, but that file is not in its tree (and needs mermaid), so its eps,
+ * spacing and face rule are unknown; this definition is from first principles (Haber & Modersitzki 2006).
+ * x = warped, y = target, both (B,1,D,H,W) or (B,D,H,W) float32; `boundary` is LR_FD_LINEAR or LR_FD_NEUMANN_ZERO.
+ *   g_a = s_a * D_a x,  h_a = s_a * D_a y  (a = 0, 1, 2 over the axes, s_a = 0.5/(2/(n_a-1))): exactly the fp32
+ *   differences lr_jacobian_det forms for one channel (the face rule, then the product with the fp32 s_a).
+ *   Per voxel, in fp64 from the fp32 g and h (sums left to right):
+ *     a = g.h,  p = |g|^2 + eps^2,  q = |h|^2 + eps^2,  f = a^2 / (p*q)  in [0, 1];
+ *   loss = 1 - (1/(B*D*H*W)) * sum_b sum_v f.
+ * The gradient is taken wrt x only (the target is data):
+ *   c_a = (2a/(p*q)) * (h_a - (a/p)*g_a)  formed in fp64 and rounded once to fp32,
+ *   d loss / d x = -(1/(B*D*H*W)) * sum_a s_a * D_a^T c_a,  D_a^T the transposed difference with its face rows, as in
+ *   lr_jacobian_fold_backward.
+ * lr_ngf_sum: sum (B) float64, zeroed by the call, = the fp64 sum of f over each item (the atomic order varies, so the
+ *   last bits may differ between calls);  loss = 1 - (sum_b sum[b]) / (B*D*H*W).
+ * lr_ngf_backward: grad_x is OVERWRITTEN with grad_loss[0] * d loss / d x (grad_loss: one float in device memory); each
+ *   element is written once, without atomics, so repeated calls give the same bits.
+ * Nothing depends on lr_set_numerics.  Arguments: eps finite and > 0 (at least 1e-77, so that p*q >= eps^4 > 0;
+ * eps = 0 would make 0/0 wherever both gradients vanish); D, H, W >= 2; B*D*H*W < 2^31; boundary 0 or 1; no null
+ * pointer.  The checks run before any CUDA call.  ops.ngf_loss uses eps = 1 by default (DESIGN.md §1). */
+LR_API int lr_ngf_sum(const float *x, const float *y, int B, int D, int H, int W, int boundary, double eps,
+                      double *sum, lr_stream_t stream);
+LR_API int lr_ngf_backward(const float *x, const float *y, int B, int D, int H, int W, int boundary, double eps,
+                           const float *grad_loss, float *grad_x, lr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

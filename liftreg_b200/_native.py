@@ -68,6 +68,8 @@ SIGNATURES = {
     "lr_local_ncc_backward": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.c_double, _vp, _vp, _vp, _sz, _vp]),
     "lr_label_dice_sums": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp]),
     "lr_label_dice_backward": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "lr_ngf_sum": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.c_double, _vp, _vp]),
+    "lr_ngf_backward": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.c_double, _vp, _vp, _vp]),
 }
 
 _lib = None

@@ -440,9 +440,11 @@ __global__ void __launch_bounds__(NCC_THREADS, LR_REGP_BWD_MINB) diffusion_reg_b
 }
 
 // Plane-march launch shape of a kernel whose block of `threads` threads owns a tile_w x tile_h tile of (last, second)
-// axis positions: the per-axis scales, the chunking of the first axis and the grid.
+// axis positions: the per-axis scales, the chunking of the first axis and the grid.  `channels` is the number of
+// (D,H,W) volumes per item the kernel indexes with 32 bits.
 template <typename K>
-static int march_dims(K kernel, int threads, int tile_w, int tile_h, int waves, int B, int D, int H, int W, RegDims &g, dim3 &grid) {
+static int march_dims(K kernel, int threads, int tile_w, int tile_h, int waves, int B, int D, int H, int W, RegDims &g, dim3 &grid,
+                      int channels = 3) {
     g.d = D; g.h = H; g.w = W;
     const double sp[3] = {1.0 / (double)(D - 1) * 2.0, 1.0 / (double)(H - 1) * 2.0, 1.0 / (double)(W - 1) * 2.0};   // spacing*2 (:53-54)
     g.sd = (float)(0.5 / sp[0]); g.sh = (float)(0.5 / sp[1]); g.sw = (float)(0.5 / sp[2]);
@@ -459,7 +461,7 @@ static int march_dims(K kernel, int threads, int tile_w, int tile_h, int waves, 
     g.n_zchunks = (D + g.zchunk - 1) / g.zchunk;
     const int64_t gz = (int64_t)g.n_zchunks * B;
     if (gz > 65535 || (H + tile_h - 1) / tile_h > 65535) return -1;
-    if ((int64_t)B * 3 * D * H * W >= ((int64_t)1 << 31)) return -1;          // the kernels index with 32 bits
+    if ((int64_t)B * channels * D * H * W >= ((int64_t)1 << 31)) return -1;   // the kernels index with 32 bits
     grid = dim3((unsigned)((W + tile_w - 1) / tile_w), (unsigned)((H + tile_h - 1) / tile_h), (unsigned)gz);
     return 0;
 }
@@ -1252,6 +1254,141 @@ __global__ void __launch_bounds__(DICE_THREADS) label_dice_backward_kernel(const
     }
 }
 
+// ---- normalized gradient field (NGF) similarity (include/liftreg_b200.h, lr_ngf_sum; PARITY UNPINNED) -------------
+// g = s * D x and h = s * D y are the fp32 differences lr_jacobian_det forms for one channel.  Per voxel, in fp64,
+//     a = g.h,  p = |g|^2 + eps^2,  q = |h|^2 + eps^2,  f = a^2 / (p q);   loss = 1 - mean f
+//     d loss / d x = -(1/(B*D*H*W)) * sum_a s_a * D_a^T c_a,   c_a = (2a/(pq)) * (h_a - (a/p) * g_a)
+// The adjoint has the fold adjoint's shape with a 3-vector c per voxel in place of the nine cofactors, so it uses
+// jacobian_fold_backward_kernel's layout.  Every voxel is evaluated by one fixed sequence of operations (fp64 products
+// of fp32 values, left to right, no contraction), so f and c do not depend on the launch shape or the batch.
+
+// one volume's scaled differences at plane z of the thread's column (element index i); advances its plane window
+template <int MODE>
+__device__ __forceinline__ void ngf_diffs(const float *__restrict__ v, const RegDims &g, unsigned i, unsigned pl, int z, int oxu,
+                                          int oxd, int oyu, int oyd, bool xlo, bool xhi, bool ylo, bool yhi, float &vm, float &vc,
+                                          float (&d)[3]) {
+    const bool zlo = z == 0, zhi = z == g.d - 1;
+    const float cc = vc;
+    const float vp = zhi ? cc : __ldg(v + (i + pl));
+    if (LR_REG_PF > 0 && z + LR_REG_PF < g.d) prefetch_l2(v + (i + LR_REG_PF * pl));
+    const float yu = __ldg(v + (i + oyu)), yd = __ldg(v + (i + oyd));
+    const float xu = __ldg(v + (i + oxu)), xd = __ldg(v + (i + oxd));
+    d[0] = mul_rn(fd_delta<MODE>(vp, vm, cc, zlo, zhi), g.sd);
+    d[1] = mul_rn(fd_delta<MODE>(yu, yd, cc, ylo, yhi), g.sh);
+    d[2] = mul_rn(fd_delta<MODE>(xu, xd, cc, xlo, xhi), g.sw);
+    vm = cc; vc = vp;
+}
+
+// a, p, q of one voxel in fp64 (the products of fp32 values are exact; the sums are rounded left to right)
+__device__ __forceinline__ void ngf_terms(const float (&gx)[3], const float (&hy)[3], double eps2, double &a, double &p, double &q) {
+    const double g0 = gx[0], g1 = gx[1], g2 = gx[2], h0 = hy[0], h1 = hy[1], h2 = hy[2];
+    a = g0 * h0 + g1 * h1 + g2 * h2;
+    p = g0 * g0 + g1 * g1 + g2 * g2 + eps2;
+    q = h0 * h0 + h1 * h1 + h2 * h2 + eps2;
+}
+
+// forward: the march of jacobian_det_kernel over two single-channel volumes, f summed per thread in fp64
+template <int MODE>
+__global__ void __launch_bounds__(NCC_THREADS) ngf_sum_kernel(const float *__restrict__ x, const float *__restrict__ y, RegDims g,
+                                                              double eps2, double *__restrict__ sum) {
+    const int xi = blockIdx.x * REG_TX + (threadIdx.x & 31), yi = blockIdx.y * REG_TY + (threadIdx.x >> 5);
+    const int zc = blockIdx.z % g.n_zchunks, b = blockIdx.z / g.n_zchunks;
+    const int z0 = zc * g.zchunk, z1 = min(g.d, z0 + g.zchunk);
+    double acc = 0.0;
+    if (xi < g.w && yi < g.h) {
+        const bool xlo = xi == 0, xhi = xi == g.w - 1, ylo = yi == 0, yhi = yi == g.h - 1;
+        const int oxu = xhi ? 0 : 1, oxd = xlo ? 0 : -1;
+        const int oyu = yhi ? 0 : g.w, oyd = ylo ? 0 : -g.w;
+        const unsigned pl = (unsigned)(g.h * g.w);                                // 32-bit indices (B*D*H*W < 2^31)
+        unsigned i0 = ((unsigned)b * (unsigned)g.d + (unsigned)z0) * pl + (unsigned)yi * (unsigned)g.w + (unsigned)xi;
+        float xm, xc = __ldg(x + i0), ym, yc = __ldg(y + i0);
+        xm = z0 > 0 ? __ldg(x + (i0 - pl)) : xc;
+        ym = z0 > 0 ? __ldg(y + (i0 - pl)) : yc;
+        for (int z = z0; z < z1; ++z, i0 += pl) {
+            float gx[3], hy[3];
+            ngf_diffs<MODE>(x, g, i0, pl, z, oxu, oxd, oyu, oyd, xlo, xhi, ylo, yhi, xm, xc, gx);
+            ngf_diffs<MODE>(y, g, i0, pl, z, oxu, oxd, oyu, oyd, xlo, xhi, ylo, yhi, ym, yc, hy);
+            double a, p, q;
+            ngf_terms(gx, hy, eps2, a, p, q);
+            acc += a * a / (p * q);
+        }
+    }
+    block_accumulate_f64(acc, sum + b);
+}
+
+// c of the thread's column at plane z (0 for a halo thread outside the volume); advances both plane windows
+template <int MODE>
+__device__ __forceinline__ void ngf_coefs(const float *__restrict__ x, const float *__restrict__ y, const RegDims &g, unsigned i,
+                                          unsigned pl, int z, int oxu, int oxd, int oyu, int oyd, bool xlo, bool xhi, bool ylo,
+                                          bool yhi, bool inside, double eps2, float (&vm)[2], float (&vc)[2], float (&c)[3]) {
+    float gx[3], hy[3];
+    ngf_diffs<MODE>(x, g, i, pl, z, oxu, oxd, oyu, oyd, xlo, xhi, ylo, yhi, vm[0], vc[0], gx);
+    ngf_diffs<MODE>(y, g, i, pl, z, oxu, oxd, oyu, oyd, xlo, xhi, ylo, yhi, vm[1], vc[1], hy);
+    double a, p, q;
+    ngf_terms(gx, hy, eps2, a, p, q);
+    const double t = 2.0 * a / (p * q), r = a / p;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) c[k] = inside ? (float)(t * ((double)hy[k] - r * (double)gx[k])) : 0.0f;
+}
+
+// adjoint: jacobian_fold_backward_kernel's layout (16 warps, 30 x 14 outputs per block, halo threads clamped to the
+// nearest voxel): D_z^T from a 3-plane register window of c0, D_y^T through a double-buffered shared plane of c1,
+// D_x^T from lane shuffles of c2; each output element written once, no atomics
+template <int MODE>
+__global__ void __launch_bounds__(FOLD_THREADS) ngf_backward_kernel(const float *__restrict__ x, const float *__restrict__ y, RegDims g,
+                                                                    int B, double eps2, const float *__restrict__ grad_loss,
+                                                                    float *__restrict__ grad_x) {
+    __shared__ float c1s[2][FOLD_WARPS][32];          // c1 of one plane, double-buffered over planes
+    const int lane = threadIdx.x & 31, wy = threadIdx.x >> 5;
+    const int xi = blockIdx.x * FOLD_OX - 1 + lane, yi = blockIdx.y * FOLD_OY - 1 + wy;
+    const int zc = blockIdx.z % g.n_zchunks, b = blockIdx.z / g.n_zchunks;
+    const int z0 = zc * g.zchunk, z1 = min(g.d, z0 + g.zchunk);
+    const bool inside = xi >= 0 && xi < g.w && yi >= 0 && yi < g.h;
+    const bool writer = inside && lane >= 1 && lane <= FOLD_OX && wy >= 1 && wy <= FOLD_OY;
+    const int xc = min(max(xi, 0), g.w - 1), yc = min(max(yi, 0), g.h - 1);
+    const bool xlo = xc == 0, xhi = xc == g.w - 1, ylo = yc == 0, yhi = yc == g.h - 1;
+    const int oxu = xhi ? 0 : 1, oxd = xlo ? 0 : -1;
+    const int oyu = yhi ? 0 : g.w, oyd = ylo ? 0 : -g.w;
+    const unsigned pl = (unsigned)(g.h * g.w);                                    // 32-bit indices (B*D*H*W < 2^31)
+    const unsigned col = (unsigned)yc * (unsigned)g.w + (unsigned)xc, item = (unsigned)b * (unsigned)g.d * pl;
+    const float k = (float)((double)grad_loss[0] / ((double)B * (double)g.d * (double)pl));
+    const float kd = -k * g.sd, kh = -k * g.sh, kw = -k * g.sw;
+
+    // prologue: c0 of plane z0-1 and all of c at plane z0
+    const int zs = z0 > 0 ? z0 - 1 : 0;
+    float vm[2], vc[2], Cc[3], c0m = 0.0f;
+    vc[0] = __ldg(x + (item + (unsigned)zs * pl + col));
+    vc[1] = __ldg(y + (item + (unsigned)zs * pl + col));
+    vm[0] = zs > 0 ? __ldg(x + (item + (unsigned)(zs - 1) * pl + col)) : vc[0];
+    vm[1] = zs > 0 ? __ldg(y + (item + (unsigned)(zs - 1) * pl + col)) : vc[1];
+    if (z0 > 0) {
+        ngf_coefs<MODE>(x, y, g, item + (unsigned)zs * pl + col, pl, zs, oxu, oxd, oyu, oyd, xlo, xhi, ylo, yhi, inside, eps2, vm, vc, Cc);
+        c0m = Cc[0];
+    }
+    ngf_coefs<MODE>(x, y, g, item + (unsigned)z0 * pl + col, pl, z0, oxu, oxd, oyu, oyd, xlo, xhi, ylo, yhi, inside, eps2, vm, vc, Cc);
+    c1s[z0 & 1][wy][lane] = Cc[1];
+    __syncthreads();
+
+    for (int z = z0; z < z1; ++z) {
+        const float cym = c1s[z & 1][max(wy - 1, 0)][lane], cyp = c1s[z & 1][min(wy + 1, FOLD_WARPS - 1)][lane];
+        const float cxm = __shfl_up_sync(0xffffffffu, Cc[2], 1), cxp = __shfl_down_sync(0xffffffffu, Cc[2], 1);
+        float Cn[3] = {0.0f, 0.0f, 0.0f};
+        if (z + 1 < g.d)
+            ngf_coefs<MODE>(x, y, g, item + (unsigned)(z + 1) * pl + col, pl, z + 1, oxu, oxd, oyu, oyd, xlo, xhi, ylo, yhi, inside, eps2,
+                            vm, vc, Cn);
+        c1s[(z + 1) & 1][wy][lane] = Cn[1];
+        if (writer) {
+            float gr = mul_rn(kd, fold_adjoint<MODE>(c0m, Cc[0], Cn[0], z, g.d));
+            gr = fmaf(kh, fold_adjoint<MODE>(cym, Cc[1], cyp, yi, g.h), gr);
+            gr = fmaf(kw, fold_adjoint<MODE>(cxm, Cc[2], cxp, xi, g.w), gr);
+            st_stream(grad_x + (item + (unsigned)z * pl + col), gr);
+        }
+        c0m = Cc[0];
+        Cc[0] = Cn[0]; Cc[1] = Cn[1]; Cc[2] = Cn[2];
+        __syncthreads();
+    }
+}
+
 }  // namespace lr
 
 using namespace lr;
@@ -1524,4 +1661,53 @@ extern "C" int lr_label_dice_backward(const float *phi, const float *src, const 
     if (int e = dice_dims(label_dice_backward_kernel, "label_dice_backward", B, D, H, W, L, g, grid)) return e;
     label_dice_backward_kernel<<<grid, DICE_THREADS, 0, as_stream(stream)>>>(phi, src, tgt, g, B, sums, grad_loss, grad_phi);
     return check_launch("label_dice_backward_kernel");
+}
+
+// argument rules shared by the NGF entries; 0 when they hold.  eps >= 1e-77 keeps p*q >= eps^4 > 0 in fp64.
+static int ngf_check(const char *who, int B, int D, int H, int W, int boundary, double eps) {
+    LR_REQUIRE(eps >= 1e-77 && eps <= DBL_MAX, "%s: eps must be finite and > 0 (>= 1e-77; got %g)", who, eps);
+    LR_REQUIRE(B >= 1 && D >= 2 && H >= 2 && W >= 2, "%s: every axis needs >= 2 entries (B=%d, %dx%dx%d)", who, B, D, H, W);
+    LR_REQUIRE(boundary == LR_FD_LINEAR || boundary == LR_FD_NEUMANN_ZERO, "%s: unknown boundary mode %d", who, boundary);
+    LR_REQUIRE((int64_t)B * D * H * W < ((int64_t)1 << 31), "%s: too large for one launch (B=%d, %dx%dx%d; B*D*H*W must stay below 2^31)",
+               who, B, D, H, W);
+    return 0;
+}
+
+template <int MODE>
+static int ngf_sum_launch(const float *x, const float *y, int B, int D, int H, int W, double eps, double *sum, cudaStream_t st) {
+    RegDims g; dim3 grid;
+    LR_REQUIRE(march_dims(ngf_sum_kernel<MODE>, NCC_THREADS, REG_TX, REG_TY, LR_REG_WAVES, B, D, H, W, g, grid, 1) == 0,
+               "ngf_sum: too many blocks for one launch (B=%d, %dx%dx%d)", B, D, H, W);
+    cudaError_t ce = cudaMemsetAsync(sum, 0, sizeof(double) * (size_t)B, st);
+    if (ce != cudaSuccess) { set_error("ngf_sum: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    ngf_sum_kernel<MODE><<<grid, NCC_THREADS, 0, st>>>(x, y, g, eps * eps, sum);
+    return check_launch("ngf_sum_kernel");
+}
+
+template <int MODE>
+static int ngf_backward_launch(const float *x, const float *y, int B, int D, int H, int W, double eps, const float *grad_loss,
+                               float *grad_x, cudaStream_t st) {
+    RegDims g; dim3 grid;
+    LR_REQUIRE(march_dims(ngf_backward_kernel<MODE>, FOLD_THREADS, FOLD_OX, FOLD_OY, LR_REG_WAVES, B, D, H, W, g, grid, 1) == 0,
+               "ngf_backward: too many blocks for one launch (B=%d, %dx%dx%d)", B, D, H, W);
+    ngf_backward_kernel<MODE><<<grid, FOLD_THREADS, 0, st>>>(x, y, g, B, eps * eps, grad_loss, grad_x);
+    return check_launch("ngf_backward_kernel");
+}
+
+extern "C" int lr_ngf_sum(const float *x, const float *y, int B, int D, int H, int W, int boundary, double eps, double *sum,
+                          lr_stream_t stream) {
+    LR_REQUIRE(x && y && sum, "ngf_sum: null pointer");
+    if (int e = ngf_check("ngf_sum", B, D, H, W, boundary, eps)) return e;
+    cudaStream_t st = as_stream(stream);
+    return boundary == LR_FD_LINEAR ? ngf_sum_launch<0>(x, y, B, D, H, W, eps, sum, st)
+                                    : ngf_sum_launch<1>(x, y, B, D, H, W, eps, sum, st);
+}
+
+extern "C" int lr_ngf_backward(const float *x, const float *y, int B, int D, int H, int W, int boundary, double eps,
+                               const float *grad_loss, float *grad_x, lr_stream_t stream) {
+    LR_REQUIRE(x && y && grad_loss && grad_x, "ngf_backward: null pointer");
+    if (int e = ngf_check("ngf_backward", B, D, H, W, boundary, eps)) return e;
+    cudaStream_t st = as_stream(stream);
+    return boundary == LR_FD_LINEAR ? ngf_backward_launch<0>(x, y, B, D, H, W, eps, grad_loss, grad_x, st)
+                                    : ngf_backward_launch<1>(x, y, B, D, H, W, eps, grad_loss, grad_x, st);
 }

@@ -1,5 +1,6 @@
-"""Drop-in mirrors of the reference's loss-side classes on the warp output (SURVEY.md 8f row f4): the similarity class of
-src/liftreg/layers/losses.py and the subspace loss of src/liftreg/losses/SubspaceLoss.py.
+"""Drop-in mirrors of the reference's loss-side classes on the warp output (SURVEY.md 8f row f4): the similarity classes of
+src/liftreg/layers/losses.py (NCCLoss; NGFLoss, defined here from first principles) and the subspace loss of
+src/liftreg/losses/SubspaceLoss.py.
 
 `NCCLoss` is what `losses/SubspaceLoss.py:12` instantiates by its dotted name ('layers.losses.NCCLoss') and what
 `networks/RegistrationNet.py:210-212` uses as the validation score; both call it on the warp output.  The reference
@@ -34,6 +35,22 @@ class LocalNCCLoss(nn.Module):
 
     def forward(self, input, target):
         return ops.local_ncc_loss(input, target, self.window, self.eps)
+
+
+class NGFLoss(nn.Module):
+    """1 - mean normalized gradient field similarity (ops.ngf_loss): the squared cosine of the angle between the image
+    gradients, regularised by eps, so only edge alignment counts and intensity changes between the images do not.  The
+    reference's layers/losses.py names an NGFLoss that is not in its tree, so parity is unpinned.  Select it with
+    `SubspaceLoss(opt, sim=NGFLoss())` or by its dotted name (`sim_class = "liftreg_b200.losses.NGFLoss"`); it needs no
+    arguments, as `losses/SubspaceLoss.py:12` instantiates it."""
+
+    def __init__(self, eps=1.0, boundary="linear"):
+        super().__init__()
+        self.eps = float(eps)
+        self.boundary = boundary
+
+    def forward(self, input, target):
+        return ops.ngf_loss(input, target, self.eps, self.boundary)
 
 
 def sigmoid_decay(ep, static=5, k=5):

@@ -4,6 +4,7 @@ PyTorch is plumbing here (device memory, streams, autograd graph); all arithmeti
 libliftreg_b200.so.  CUDA float32 tensors only -- there is no CPU fallback.
 """
 import ctypes
+import math
 
 import numpy as np
 import torch
@@ -511,6 +512,58 @@ def diffusion_reg(disp, boundary="linear"):
     if boundary not in FD_BOUNDARY:
         raise ValueError("boundary must be one of %s, got %r" % (sorted(FD_BOUNDARY), boundary))
     return _DiffusionReg.apply(disp, FD_BOUNDARY[boundary])
+
+
+# --------------------------------------------------------------------------- NGF similarity (training term)
+class _Ngf(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, y, eps, boundary):
+        x, (B, D, H, W) = _volume(x, "input")
+        y, _ = _volume(y, "target")
+        sums = torch.empty(B, device=x.device, dtype=torch.float64)
+        with torch.cuda.device(x.device):
+            _native.check(_native.lib().lr_ngf_sum(_ptr(x), _ptr(y), B, D, H, W, boundary, eps, _ptr(sums), _stream()),
+                          "lr_ngf_sum")
+        ctx.save_for_backward(x, y)
+        ctx.cfg = (eps, boundary)
+        return (1.0 - sums.sum() / float(B * D * H * W)).to(torch.float32)
+
+    @staticmethod
+    def backward(ctx, grad_loss):
+        x, y = ctx.saved_tensors
+        eps, boundary = ctx.cfg
+        B, D, H, W = x.shape[0], *x.shape[-3:]
+        g = grad_loss.to(device=x.device, dtype=torch.float32).reshape(1).contiguous()
+        gx = torch.empty_like(x)
+        with torch.cuda.device(x.device):
+            _native.check(_native.lib().lr_ngf_backward(_ptr(x), _ptr(y), B, D, H, W, boundary, eps, _ptr(g), _ptr(gx),
+                                                        _stream()), "lr_ngf_backward")
+        return gx, None, None, None
+
+
+def ngf_loss(input, target, eps=1.0, boundary="linear"):
+    """Normalized gradient field similarity: 1 - mean over (B, D, H, W) of (g.h)^2 / ((|g|^2 + eps^2)(|h|^2 + eps^2)),
+    with g and h the regulariser's central differences of input and target (face rule `boundary`, as diffusion_reg);
+    it scores edge alignment only, so an intensity change between the images does not affect it (definition:
+    include/liftreg_b200.h, lr_ngf_sum).  input and target are (B,1,D,H,W) or (B,D,H,W) CUDA float32 with every
+    spatial axis >= 2; eps (finite, > 0) is in the units of g: intensity per unit of the [-1, 1] grid coordinate.
+    Differentiable wrt `input` (the warped image); `target` is data.  A float32 scalar computed without a host
+    synchronisation.  The reference's NGFLoss is not in its tree, so parity is unpinned."""
+    for t, name in ((input, "input"), (target, "target")):
+        if not isinstance(t, torch.Tensor) or not (t.dim() == 4 or (t.dim() == 5 and t.shape[1] == 1)):
+            raise ValueError("%s must be (B,1,D,H,W) or (B,D,H,W), got %s"
+                             % (name, tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__))
+    if input.shape != target.shape:
+        raise ValueError("input %s and target %s must have the same shape" % (tuple(input.shape), tuple(target.shape)))
+    if min(input.shape[-3:]) < 2:
+        raise ValueError("every spatial axis needs >= 2 entries, got %s" % (tuple(input.shape[-3:]),))
+    eps = float(eps)
+    if not (math.isfinite(eps) and eps >= 1e-77):
+        raise ValueError("eps must be finite and > 0 (>= 1e-77), got %r" % eps)
+    if boundary not in FD_BOUNDARY:
+        raise ValueError("boundary must be one of %s, got %r" % (sorted(FD_BOUNDARY), boundary))
+    return _Ngf.apply(input, target, eps, FD_BOUNDARY[boundary])
+
 
 
 # --------------------------------------------------------------------------- validation metrics (not differentiable)

@@ -160,6 +160,23 @@ def main():
         _native.check(lib.lr_local_ncc_backward(vp(s["x8"]), vp(s["y8"]), 8, *VOL, 9, 1e-5, vp(ncc_g), vp(s["g8"]),
                                                 vp(lncc_ws), lncc_ws.numel(), st), "lncc_bwd8")
 
+    ngf_sum = torch.zeros(8, device=dev, dtype=torch.float64)
+
+    def k_ngf(s, st):          # NGF forward: one pass over two volumes (8 B per voxel)
+        _native.check(lib.lr_ngf_sum(vp(s["moving"]), vp(s["mu"]), 1, *VOL, 0, 1.0, vp(ngf_sum), st), "ngf")
+
+    def k_ngf_bwd(s, st):      # NGF adjoint: reads x and y, writes grad_x (12 B per voxel)
+        _native.check(lib.lr_ngf_backward(vp(s["moving"]), vp(s["mu"]), 1, *VOL, 0, 1.0, vp(ncc_g), vp(s["gvol"]), st), "ngf_bwd")
+
+    if "ngf_bwd8" in which and "x8" not in sets[0]:
+        for i, s_ in enumerate(sets):
+            s_["x8"] = torch.from_numpy(rs.uniform(-1, 1, (8, 1) + VOL).astype(np.float32)).to(dev)
+            s_["y8"] = torch.from_numpy(rs.uniform(-1, 1, (8, 1) + VOL).astype(np.float32)).to(dev)
+            s_["g8"] = torch.empty((8, 1) + VOL, device=dev)
+
+    def k_ngf_bwd8(s, st):
+        _native.check(lib.lr_ngf_backward(vp(s["x8"]), vp(s["y8"]), 8, *VOL, 0, 1.0, vp(ncc_g), vp(s["g8"]), st), "ngf_bwd8")
+
     dice_names = ("dice", "dice_bwd", "dice_bwd8")
     if "labels2" in which or "labels6" in which or any(n in which for n in dice_names):
         # label maps as a validation item has them: mostly background, a few organ-sized blobs, target = shifted pred
@@ -207,7 +224,8 @@ def main():
 
     units = {"atten": (k_atten, nv, 8 * nv), "idmap": (k_idmap, nv, 12 * nv), "reg": (k_reg, nv, 12 * nv), "jac": (k_jac, nv, 12 * nv), "jac_map": (k_jac_map, nv, 16 * nv),
              "labels2": (k_labels(2), nv, 8 * nv), "labels6": (k_labels(6), nv, 8 * nv), "reg_bwd": (k_reg_bwd, nv, 24 * nv), "fold_bwd": (k_fold_bwd, nv, 24 * nv), "fold_bwd8": (k_fold_bwd8, 8 * nv, 8 * 24 * nv), "ncc": (k_ncc, nv, 8 * nv), "lncc": (k_lncc, nv, 8 * nv), "lncc_bwd": (k_lncc_bwd, nv, 44 * nv),
-             "lncc_bwd8": (k_lncc_bwd8, 8 * nv, 8 * 44 * nv), "dice": (k_dice, nv, 20 * nv), "dice_bwd": (k_dice_bwd, nv, 32 * nv),
+             "lncc_bwd8": (k_lncc_bwd8, 8 * nv, 8 * 44 * nv), "ngf": (k_ngf, nv, 8 * nv), "ngf_bwd": (k_ngf_bwd, nv, 12 * nv),
+             "ngf_bwd8": (k_ngf_bwd8, 8 * nv, 8 * 12 * nv), "dice": (k_dice, nv, 20 * nv), "dice_bwd": (k_dice_bwd, nv, 32 * nv),
              "dice_bwd8": (k_dice_bwd8, 8 * nv, 8 * 32 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
              "pca_bwd": (k_pca_bwd, 3 * nv, 4 * 3 * nv * 56 + 4 * 3 * nv), "warp_bwd": (k_warp_bwd, nv, 32 * nv),
              "drr_bwd": (k_drr_bwd, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240), "backproject": (k_backproject, batch * P * nv, batch * (4 * P * nv + 4 * P * DET[0] * DET[1])),
