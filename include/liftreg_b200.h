@@ -420,6 +420,43 @@ LR_API int lr_ngf_sum(const float *x, const float *y, int B, int D, int H, int W
 LR_API int lr_ngf_backward(const float *x, const float *y, int B, int D, int H, int W, int boundary, double eps,
                            const float *grad_loss, float *grad_x, lr_stream_t stream);
 
+/* ---- mutual information (MI) similarity, Parzen joint histogram (PARITY UNPINNED) -------------------------------------
+ * Mattes et al. (2003) MI, the default metric of elastix; the reference has no MI, so nothing pins it.
+ * x = warped, y = target, each B items of N float32 (any shape, flattened per item); nb = num_bins in [4, 64];
+ * lo < hi finite fp32 (the value range; ops.mi_loss uses (-1, 1), the range of the unit-normalised CT).  The range is
+ * FIXED rather than each image's own min and max as Mattes uses: no min/max pass, no host synchronisation, and the
+ * gradient has no term through the range.
+ *   s = (float)((nb - 1) / ((double)hi - lo)).  Per voxel v, in fp32 with each op rounded:
+ *     u = (fminf(fmaxf(v, lo), hi) - lo) * s        (NaN -> lo, -inf -> lo, +inf -> hi: no input indexes outside)
+ *     target row   iota = floor(u_y + 0.5)           (in [0, nb-1]; zero-order Parzen window)
+ *     moving taps  k0 = min(floor(u_x), nb - 2),  f = u_x - k0 (exact; in [0, 1] up to the rounding of u near nb-1),
+ *                  kappa = k0 - 1 .. k0 + 2 with the cubic B-spline weights, in fp64 from the fp32 f:
+ *       F = f, G = 1 - F, F2 = F*F, F3 = F2*F, r6 = 1.0/6.0 (the double nearest 1/6);
+ *       w0 = ((G*G)*G)*r6,  w1 = ((4 - 6*F2) + 3*F3)*r6,  w2 = (((1 + 3*F) + 3*F2) - 3*F3)*r6,  w3 = F3*r6.
+ *   hist (B, nb, nb+2) float64: hist[b][iota][kappa + 1] += w_m, so every tap lands inside (kappa in [-1, nb]).
+ *   p = hist/N, p_y = sum over the columns of p, p_x = sum over the rows, MI_b = sum_{p>0} p (log p - log p_y - log p_x),
+ *   loss = -mean_b MI_b (nats).
+ * Gradient wrt x only (p_y does not depend on x, and sum_m dw_m/df = 0):
+ *   d loss / d x_v = -(g/(B N)) * s * sum_m w_m'(f_v) * c(iota_v, k0_v - 1 + m),  c(iota, kappa) = log(p / p_x) (0 where
+ *   p = 0), exactly 0 unless lo <= x_v <= hi (torch.clamp's mask; NaN gets 0).  The cubic B-spline is C^2, so the
+ *   gradient does not jump at bin edges.
+ * lr_mi_hist: hist (B*nb*(nb+2) float64) is zeroed and filled by the call; the fp64 atomic order varies, so the last
+ *   bits may differ between calls.
+ * lr_mi_backward: grad_x (B*N) is OVERWRITTEN with grad_loss[0] * d loss / d x for the given hist (grad_loss: one float
+ *   in device memory).  Per item, the column sums P_x[j] = sum_{r = 0..nb-1} hist[r][j] (fp64, rows in order) and the
+ *   table T = (float)(log(hist / P_x) * k), k = -((double)g * s) / ((double)B * N), are formed in fp64 and T is rounded
+ *   once to fp32 (T = 0 where hist = 0).  Per voxel, in fp32 with each op rounded, the derivative weights are
+ *     w0' = -((1-f)^2 * 0.5),  w1' = -((f * (4 - 3f)) * 0.5),  w2' = ((1-f) * (1 + 3f)) * 0.5,  w3' = (f*f) * 0.5
+ *   (the polynomials -(1-f)^2/2, f(3f-4)/2, (1+2f-3f^2)/2, f^2/2 in product form, free of cancellation), and
+ *   grad = fma(T3, w3', fma(T2, w2', fma(T1, w1', T0 * w0'))) with T_m = T[iota][k0 + m].  Each element is written
+ *   once, without atomics: the same hist gives the same bits.
+ * Arguments: no null pointer; 1 <= B <= 65535, N >= 1; 4 <= nb <= 64; lo, hi finite with lo < hi and s finite and
+ * > 0.  The checks run before any CUDA call. */
+LR_API int lr_mi_hist(const float *x, const float *y, int B, int64_t N, int num_bins, float lo, float hi, double *hist,
+                      lr_stream_t stream);
+LR_API int lr_mi_backward(const float *x, const float *y, int B, int64_t N, int num_bins, float lo, float hi,
+                          const double *hist, const float *grad_loss, float *grad_x, lr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -70,6 +70,8 @@ SIGNATURES = {
     "lr_label_dice_backward": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "lr_ngf_sum": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.c_double, _vp, _vp]),
     "lr_ngf_backward": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.c_double, _vp, _vp, _vp]),
+    "lr_mi_hist": (_i, [_vp, _vp, _i, _i64, _i, _f, _f, _vp, _vp]),
+    "lr_mi_backward": (_i, [_vp, _vp, _i, _i64, _i, _f, _f, _vp, _vp, _vp, _vp]),
 }
 
 _lib = None

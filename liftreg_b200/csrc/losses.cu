@@ -1389,6 +1389,166 @@ __global__ void __launch_bounds__(FOLD_THREADS) ngf_backward_kernel(const float 
     }
 }
 
+// ---- mutual information (MI) similarity, Parzen joint histogram (include/liftreg_b200.h, lr_mi_hist; PARITY UNPINNED) --
+// Per voxel the fp32 chain u = (clamp(v) - lo) * s of x and y gives the target row iota = floor(u_y + 1/2) and the
+// moving cubic B-spline taps k0 - 1 .. k0 + 2 with fraction f = u_x - k0; the histogram row iota gets the four fp64 tap
+// weights in columns k0 .. k0 + 3.  A CT image puts most voxels into very few keys (iota, k0) -- air and bone saturate
+// the [-1, 1] range -- so the forward keeps one run of equal keys per lane and adds a run to the block's fp64 shared
+// histogram only when the key changes (one warp sum and one set of atomics when every flushing lane of the warp holds
+// the same key).  The adjoint needs only c(iota, kappa) = log(p / p_x) per bin: each block derives the item's table
+// c * (-g s / (B N)) in fp64 and rounds it once to fp32, then streams x and y and writes each gradient element once.
+constexpr int MI_THREADS = 256, MI_BWD_THREADS = 512, MI_NBMAX = 64;
+
+struct MiMap {
+    float lo, hi, s;
+    int nb;
+};
+
+// u = (clamp(v, lo, hi) - lo) * s, each op rounded; NaN clamps to lo
+__device__ __forceinline__ float mi_u(float v, const MiMap &m) { return mul_rn(sub_rn(fminf(fmaxf(v, m.lo), m.hi), m.lo), m.s); }
+
+// the voxel's histogram key: bin index of its first tap, row iota and column k0 of the (nb, nb + 2) histogram, and f.
+// u <= (nb-1)(1 + 3 * 2^-24), so iota <= nb - 1 already; the min only guards the index.
+__device__ __forceinline__ int mi_key(float vx, float vy, const MiMap &m, float &f) {
+    const float ux = mi_u(vx, m), uy = mi_u(vy, m);
+    const int row = min((int)floorf(add_rn(uy, 0.5f)), m.nb - 1);
+    const int k0 = min((int)floorf(ux), m.nb - 2);
+    f = sub_rn(ux, (float)k0);                               // exact
+    return row * (m.nb + 2) + k0;
+}
+
+// cubic B-spline weights of the taps k0 - 1 .. k0 + 2 in fp64 from the fp32 f, in the header's order
+__device__ __forceinline__ void mi_weights(float f, double (&w)[4]) {
+    const double F = (double)f, G = 1.0 - F, F2 = F * F, F3 = F2 * F, r6 = 1.0 / 6.0;
+    w[0] = G * G * G * r6;
+    w[1] = ((4.0 - 6.0 * F2) + 3.0 * F3) * r6;
+    w[2] = (((1.0 + 3.0 * F) + 3.0 * F2) - 3.0 * F3) * r6;
+    w[3] = F3 * r6;
+}
+
+// adds the runs of the lanes with `part` set to the block's bins (called by the whole warp)
+__device__ __forceinline__ void mi_flush(double *__restrict__ h, int key, const double (&a)[4], bool part, int lane) {
+    const unsigned m = __ballot_sync(0xffffffffu, part);
+    if (!m) return;
+    const int k0 = __shfl_sync(0xffffffffu, key, __ffs(m) - 1);
+    if (__all_sync(0xffffffffu, !part || key == k0)) {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const double t = warp_sum(part ? a[j] : 0.0);
+            if (lane == 0) atomicAdd(h + k0 + j, t);
+        }
+    } else if (part) {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) atomicAdd(h + key + j, a[j]);
+    }
+}
+
+// one voxel of the forward for every lane of the warp (valid: the lane has a voxel)
+__device__ __forceinline__ void mi_step(bool valid, float vx, float vy, const MiMap &m, double *__restrict__ h, int &key,
+                                        double (&a)[4], int lane) {
+    int k = -1;
+    double w[4] = {0.0, 0.0, 0.0, 0.0};
+    if (valid) {
+        float f;
+        k = mi_key(vx, vy, m, f);
+        mi_weights(f, w);
+    }
+    const bool change = k != key;
+    mi_flush(h, key, a, change && key >= 0, lane);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) a[j] = change ? w[j] : a[j] + w[j];
+    key = k;
+}
+
+// hist[b] += the fp64 tap weights of item b; label_confusion_kernel's traversal (warp-uniform trip counts over float4
+// groups of both images, a scalar loop for the rest or for unaligned items), one fp64 atomic per block and non-empty bin
+__global__ void __launch_bounds__(MI_THREADS) mi_hist_kernel(const float *__restrict__ x, const float *__restrict__ y, int64_t N,
+                                                             MiMap m, double *__restrict__ hist) {
+    extern __shared__ double mi_bins[];
+    const int nbins = m.nb * (m.nb + 2), b = blockIdx.y, lane = threadIdx.x & 31;
+    for (int i = threadIdx.x; i < nbins; i += MI_THREADS) mi_bins[i] = 0.0;
+    __syncthreads();
+    const float *xb = x + (int64_t)b * N, *yb = y + (int64_t)b * N;
+    const int64_t wid = ((int64_t)blockIdx.x * MI_THREADS + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * MI_THREADS) >> 5;
+    const int64_t n4 = (((uintptr_t)xb | (uintptr_t)yb) % 16 == 0) ? N / 4 : 0;
+    int key = -1;
+    double a[4] = {0.0, 0.0, 0.0, 0.0};
+    for (int64_t base = wid * 32; base < n4; base += nwarps * 32) {
+        const int64_t i = base + lane;
+        const bool ok = i < n4;
+        float4 p = make_float4(0.f, 0.f, 0.f, 0.f), t = p;
+        if (ok) {
+            p = ld_stream4(reinterpret_cast<const float4 *>(xb) + i);
+            t = ld_stream4(reinterpret_cast<const float4 *>(yb) + i);
+        }
+        mi_step(ok, p.x, t.x, m, mi_bins, key, a, lane);
+        mi_step(ok, p.y, t.y, m, mi_bins, key, a, lane);
+        mi_step(ok, p.z, t.z, m, mi_bins, key, a, lane);
+        mi_step(ok, p.w, t.w, m, mi_bins, key, a, lane);
+    }
+    for (int64_t base = 4 * n4 + wid * 32; base < N; base += nwarps * 32) {
+        const int64_t i = base + lane;
+        const bool ok = i < N;
+        mi_step(ok, ok ? ld_stream(xb + i) : 0.f, ok ? ld_stream(yb + i) : 0.f, m, mi_bins, key, a, lane);
+    }
+    mi_flush(mi_bins, key, a, key >= 0, lane);
+    __syncthreads();
+    double *hb = hist + (int64_t)b * nbins;
+    for (int i = threadIdx.x; i < nbins; i += MI_THREADS) {
+        const double v = mi_bins[i];
+        if (v != 0.0) atomicAdd(hb + i, v);
+    }
+}
+
+// d w_m / d f in fp32, the header's product forms (no cancellation near f = 0 or 1)
+__device__ __forceinline__ float mi_grad_one(float vx, float vy, const MiMap &m, const float *__restrict__ tab) {
+    float f;
+    const int k = mi_key(vx, vy, m, f);
+    const float g = sub_rn(1.0f, f);
+    const float d0 = -mul_rn(mul_rn(g, g), 0.5f);
+    const float d1 = -mul_rn(mul_rn(f, sub_rn(4.0f, mul_rn(3.0f, f))), 0.5f);
+    const float d2 = mul_rn(mul_rn(g, add_rn(1.0f, mul_rn(3.0f, f))), 0.5f);
+    const float d3 = mul_rn(mul_rn(f, f), 0.5f);
+    const float acc = fma_rn(tab[k + 3], d3, fma_rn(tab[k + 2], d2, fma_rn(tab[k + 1], d1, mul_rn(tab[k], d0))));
+    return vx >= m.lo && vx <= m.hi ? acc : 0.0f;             // torch.clamp's mask: NaN and values outside get 0
+}
+
+// grad_x = grad_loss * d loss / d x for the given histogram; every element written once, no atomics
+__global__ void __launch_bounds__(MI_BWD_THREADS) mi_backward_kernel(const float *__restrict__ x, const float *__restrict__ y,
+                                                                     int64_t N, int B, MiMap m, const double *__restrict__ hist,
+                                                                     const float *__restrict__ grad_loss, float *__restrict__ gx) {
+    extern __shared__ float mi_tab[];
+    __shared__ double col[MI_NBMAX + 2];
+    const int b = blockIdx.y, nc = m.nb + 2, nbins = m.nb * nc;
+    const double *hb = hist + (int64_t)b * nbins;
+    for (int j = threadIdx.x; j < nc; j += MI_BWD_THREADS) {   // p_x * N, summed over the rows in order
+        double s = 0.0;
+        for (int r = 0; r < m.nb; ++r) s += hb[r * nc + j];
+        col[j] = s;
+    }
+    __syncthreads();
+    const double k = -((double)grad_loss[0] * (double)m.s) / ((double)B * (double)N);
+    for (int i = threadIdx.x; i < nbins; i += MI_BWD_THREADS) {
+        const double h = hb[i];
+        mi_tab[i] = h > 0.0 ? (float)(log(h / col[i % nc]) * k) : 0.0f;
+    }
+    __syncthreads();
+    const float *xb = x + (int64_t)b * N, *yb = y + (int64_t)b * N;
+    float *gb = gx + (int64_t)b * N;
+    const int64_t t = (int64_t)blockIdx.x * MI_BWD_THREADS + threadIdx.x, stride = (int64_t)gridDim.x * MI_BWD_THREADS;
+    const int64_t n4 = (((uintptr_t)xb | (uintptr_t)yb | (uintptr_t)gb) % 16 == 0) ? N / 4 : 0;
+    for (int64_t i = t; i < n4; i += stride) {
+        const float4 xv = ld_stream4(reinterpret_cast<const float4 *>(xb) + i), yv = ld_stream4(reinterpret_cast<const float4 *>(yb) + i);
+        float4 o;
+        o.x = mi_grad_one(xv.x, yv.x, m, mi_tab);
+        o.y = mi_grad_one(xv.y, yv.y, m, mi_tab);
+        o.z = mi_grad_one(xv.z, yv.z, m, mi_tab);
+        o.w = mi_grad_one(xv.w, yv.w, m, mi_tab);
+        st_stream4(reinterpret_cast<float4 *>(gb) + i, o);
+    }
+    for (int64_t i = 4 * n4 + t; i < N; i += stride) st_stream(gb + i, mi_grad_one(ld_stream(xb + i), ld_stream(yb + i), m, mi_tab));
+}
+
 }  // namespace lr
 
 using namespace lr;
@@ -1710,4 +1870,58 @@ extern "C" int lr_ngf_backward(const float *x, const float *y, int B, int D, int
     cudaStream_t st = as_stream(stream);
     return boundary == LR_FD_LINEAR ? ngf_backward_launch<0>(x, y, B, D, H, W, eps, grad_loss, grad_x, st)
                                     : ngf_backward_launch<1>(x, y, B, D, H, W, eps, grad_loss, grad_x, st);
+}
+
+// argument rules shared by the MI entries; 0 when they hold, with the map's fp32 s = (nb - 1) / (hi - lo)
+static int mi_check(const char *who, int B, int64_t N, int nb, float lo, float hi, MiMap &m) {
+    LR_REQUIRE(B >= 1 && B <= 65535 && N >= 1, "%s: bad size (B=%d N=%lld; 1 <= B <= 65535, N >= 1)", who, B, (long long)N);
+    LR_REQUIRE(nb >= 4 && nb <= MI_NBMAX, "%s: num_bins=%d must be in [4, %d]", who, nb, MI_NBMAX);
+    LR_REQUIRE(lo >= -FLT_MAX && hi <= FLT_MAX && lo < hi, "%s: value range (%g, %g) must be finite with lo < hi", who, (double)lo, (double)hi);
+    const float s = (float)((double)(nb - 1) / ((double)hi - (double)lo));
+    LR_REQUIRE(s > 0.0f && s <= FLT_MAX, "%s: (num_bins - 1) / (hi - lo) = %g is not a finite positive float", who, (double)s);
+    m.lo = lo; m.hi = hi; m.s = s; m.nb = nb;
+    return 0;
+}
+
+// blocks per item: >= 16 voxels per thread, one wave over the whole grid
+static unsigned mi_blocks(int64_t N, int B, int threads, int per_sm) {
+    int64_t want = (N + threads * 16 - 1) / (threads * 16);
+    const int64_t cap = ((int64_t)sm_count() * per_sm + B - 1) / B;
+    if (want > cap) want = cap;
+    return (unsigned)(want < 1 ? 1 : want);
+}
+
+template <typename K>
+static int mi_per_sm(K kernel, int threads, size_t smem) {
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem) != cudaSuccess || per_sm < 1) {
+        cudaGetLastError();
+        per_sm = 1;
+    }
+    return per_sm;
+}
+
+extern "C" int lr_mi_hist(const float *x, const float *y, int B, int64_t N, int num_bins, float lo, float hi, double *hist,
+                          lr_stream_t stream) {
+    LR_REQUIRE(x && y && hist, "mi_hist: null pointer");
+    MiMap m;
+    if (int e = mi_check("mi_hist", B, N, num_bins, lo, hi, m)) return e;
+    cudaStream_t st = as_stream(stream);
+    const size_t nbins = (size_t)num_bins * (num_bins + 2), smem = sizeof(double) * nbins;
+    cudaError_t ce = cudaMemsetAsync(hist, 0, sizeof(double) * nbins * (size_t)B, st);
+    if (ce != cudaSuccess) { set_error("mi_hist: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    const dim3 grid(mi_blocks(N, B, MI_THREADS, mi_per_sm(mi_hist_kernel, MI_THREADS, smem)), (unsigned)B);
+    mi_hist_kernel<<<grid, MI_THREADS, smem, st>>>(x, y, N, m, hist);
+    return check_launch("mi_hist_kernel");
+}
+
+extern "C" int lr_mi_backward(const float *x, const float *y, int B, int64_t N, int num_bins, float lo, float hi,
+                              const double *hist, const float *grad_loss, float *grad_x, lr_stream_t stream) {
+    LR_REQUIRE(x && y && hist && grad_loss && grad_x, "mi_backward: null pointer");
+    MiMap m;
+    if (int e = mi_check("mi_backward", B, N, num_bins, lo, hi, m)) return e;
+    const size_t smem = sizeof(float) * (size_t)num_bins * (num_bins + 2);
+    const dim3 grid(mi_blocks(N, B, MI_BWD_THREADS, mi_per_sm(mi_backward_kernel, MI_BWD_THREADS, smem)), (unsigned)B);
+    mi_backward_kernel<<<grid, MI_BWD_THREADS, smem, as_stream(stream)>>>(x, y, N, B, m, hist, grad_loss, grad_x);
+    return check_launch("mi_backward_kernel");
 }

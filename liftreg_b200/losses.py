@@ -53,6 +53,23 @@ class NGFLoss(nn.Module):
         return ops.ngf_loss(input, target, self.eps, self.boundary)
 
 
+class MILoss(nn.Module):
+    """-mean_b mutual information of the Parzen joint histogram (ops.mi_loss; Mattes et al. 2003, elastix's default
+    metric) over a fixed value range, so a non-linear intensity relation between the images (saturated HU windows,
+    density change of the lung between breathing phases) is not penalised.  Not in the reference, so parity is
+    unpinned.  Select it with `SubspaceLoss(opt, sim=MILoss())` or by its dotted name
+    (`sim_class = "liftreg_b200.losses.MILoss"`); it needs no arguments.  Inputs are flattened per item, as NCCLoss."""
+
+    def __init__(self, num_bins=32, value_range=(-1.0, 1.0)):
+        super().__init__()
+        self.num_bins = int(num_bins)
+        self.value_range = (float(value_range[0]), float(value_range[1]))
+
+    def forward(self, input, target):
+        return ops.mi_loss(input.reshape(input.shape[0], -1), target.reshape(target.shape[0], -1), self.num_bins,
+                           self.value_range)
+
+
 def sigmoid_decay(ep, static=5, k=5):
     """reference utils/utils.py:93-107: 1 for the first `static` epochs, then k / (k + exp((ep - static) / k))."""
     if ep < static:

@@ -565,6 +565,76 @@ def ngf_loss(input, target, eps=1.0, boundary="linear"):
     return _Ngf.apply(input, target, eps, FD_BOUNDARY[boundary])
 
 
+# --------------------------------------------------------------------------- mutual information similarity (training term)
+def _mi_loss_from_hist(hist, N):
+    """-mean_b MI_b from hist (B, nb, nb+2) float64 of N voxels per item: float64 on the histogram's device, no host
+    synchronisation"""
+    p = hist / float(N)
+    pos = p > 0
+    one = torch.ones((), dtype=p.dtype, device=p.device)
+    py = p.sum(2, keepdim=True).expand_as(p)
+    px = p.sum(1, keepdim=True).expand_as(p)
+    log = lambda t: torch.log(torch.where(pos, t, one))
+    mi = torch.where(pos, p * (log(p) - log(py) - log(px)), 0.0).sum((1, 2))
+    return -mi.mean()
+
+
+class _Mi(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, y, nb, lo, hi):
+        x = _need_cuda_f32(x, "input")
+        y = _need_cuda_f32(y, "target")
+        B, N = x.shape[0], x.numel() // x.shape[0]
+        hist = torch.empty((B, nb, nb + 2), device=x.device, dtype=torch.float64)
+        with torch.cuda.device(x.device):
+            _native.check(_native.lib().lr_mi_hist(_ptr(x), _ptr(y), B, N, nb, lo, hi, _ptr(hist), _stream()), "lr_mi_hist")
+        ctx.save_for_backward(x, y, hist)
+        ctx.cfg = (nb, lo, hi)
+        return _mi_loss_from_hist(hist, N).to(torch.float32)
+
+    @staticmethod
+    def backward(ctx, grad_loss):
+        x, y, hist = ctx.saved_tensors
+        nb, lo, hi = ctx.cfg
+        B, N = x.shape[0], x.numel() // x.shape[0]
+        g = grad_loss.to(device=x.device, dtype=torch.float32).reshape(1).contiguous()
+        gx = torch.empty_like(x)
+        with torch.cuda.device(x.device):
+            _native.check(_native.lib().lr_mi_backward(_ptr(x), _ptr(y), B, N, nb, lo, hi, _ptr(hist), _ptr(g), _ptr(gx),
+                                                       _stream()), "lr_mi_backward")
+        return gx, None, None, None, None
+
+
+def mi_loss(input, target, num_bins=32, value_range=(-1.0, 1.0)):
+    """-mean_b of the mutual information (nats) of the Parzen joint histogram of input_b and target_b (Mattes et al.
+    2003): a cubic B-spline window on the input, a zero-order window on the target, num_bins bins over the FIXED
+    value_range (lo, hi), values outside clamped to it (definition: include/liftreg_b200.h, lr_mi_hist).  input and
+    target are (B, ...) CUDA float32 of one shape, each item flattened.  Differentiable wrt `input` (the warped image);
+    `target` is data.  A float32 scalar computed without a host synchronisation.  The reference has no MI, so parity
+    is unpinned."""
+    for t, name in ((input, "input"), (target, "target")):
+        if not isinstance(t, torch.Tensor) or t.dim() < 1 or t.numel() == 0:
+            raise ValueError("%s must be a non-empty (B, ...) tensor, got %s"
+                             % (name, tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__))
+    if input.shape != target.shape:
+        raise ValueError("input %s and target %s must have the same shape" % (tuple(input.shape), tuple(target.shape)))
+    if input.shape[0] > 65535:
+        raise ValueError("at most 65535 items per call, got %d" % input.shape[0])
+    if isinstance(num_bins, bool) or not isinstance(num_bins, (int, np.integer)) or not 4 <= num_bins <= 64:
+        raise ValueError("num_bins must be an integer in [4, 64], got %r" % (num_bins,))
+    try:
+        lo, hi = (float(v) for v in value_range)
+    except (TypeError, ValueError):
+        raise ValueError("value_range must be a pair (lo, hi) of numbers, got %r" % (value_range,)) from None
+    with np.errstate(over="ignore"):
+        lo32, hi32 = np.float32(lo), np.float32(hi)
+        s = np.float32((int(num_bins) - 1) / (float(hi32) - float(lo32))) if hi32 > lo32 else np.float32(0)
+    if not (np.isfinite(lo32) and np.isfinite(hi32) and lo32 < hi32 and np.isfinite(s) and s > 0):
+        raise ValueError("value_range (%r, %r) must be finite in float32 with lo < hi and (num_bins - 1) / (hi - lo) a "
+                         "finite positive float" % (lo, hi))
+    return _Mi.apply(input, target, int(num_bins), float(lo32), float(hi32))
+
+
 
 # --------------------------------------------------------------------------- validation metrics (not differentiable)
 JACOBIAN_STATS = ("folding_count", "folding_abs_sum", "det_min", "det_max", "det_sum", "det_sum_sq", "nonfinite_count")

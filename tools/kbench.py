@@ -177,6 +177,36 @@ def main():
     def k_ngf_bwd8(s, st):
         _native.check(lib.lr_ngf_backward(vp(s["x8"]), vp(s["y8"]), 8, *VOL, 0, 1.0, vp(ncc_g), vp(s["g8"]), st), "ngf_bwd8")
 
+    mi_names = ("mi", "mi_bwd", "mi_bwd8")
+    if any(n in which for n in mi_names):
+        # the unit-normalised CT phantom pair: the histogram's contention depends on the image content (air and bone
+        # saturate the range), so uniform noise would time a different kernel
+        mi_y = torch.from_numpy(synthetic.hu_to_unit(synthetic.ct_phantom(VOL, seed=0))[None, None]).to(dev)
+        mi_x = ops.warp(mi_y, torch.from_numpy(synthetic.smooth_displacement(VOL, seed=1, max_disp=0.05, coarse=4)).to(dev)[None]
+                        + ops.identity_map(VOL, dev))
+        mi_hist = torch.zeros((8, 32, 34), device=dev, dtype=torch.float64)
+        _native.check(lib.lr_mi_hist(vp(mi_x), vp(mi_y), 1, nv, 32, -1.0, 1.0, vp(mi_hist), None), "mi")
+        for s_ in sets:
+            s_["mi_x"], s_["mi_y"], s_["mi_g"] = mi_x.clone(), mi_y.clone(), torch.empty_like(mi_x)
+        if "mi_bwd8" in which:
+            _native.check(lib.lr_mi_hist(vp(mi_x.repeat(8, 1, 1, 1, 1)), vp(mi_y.repeat(8, 1, 1, 1, 1)), 8, nv, 32, -1.0, 1.0,
+                                         vp(mi_hist), None), "mi8")
+            for s_ in sets:
+                s_["mi_x8"], s_["mi_y8"] = mi_x.repeat(8, 1, 1, 1, 1), mi_y.repeat(8, 1, 1, 1, 1)
+                s_["mi_g8"] = torch.empty_like(s_["mi_x8"])
+        torch.cuda.synchronize()
+
+    def k_mi(s, st):           # MI forward: the joint histogram of warped + target (8 B per voxel), nb = 32
+        _native.check(lib.lr_mi_hist(vp(s["mi_x"]), vp(s["mi_y"]), 1, nv, 32, -1.0, 1.0, vp(mi_hist), st), "mi")
+
+    def k_mi_bwd(s, st):       # MI adjoint: reads x and y, writes grad_x (12 B per voxel)
+        _native.check(lib.lr_mi_backward(vp(s["mi_x"]), vp(s["mi_y"]), 1, nv, 32, -1.0, 1.0, vp(mi_hist), vp(ncc_g),
+                                         vp(s["mi_g"]), st), "mi_bwd")
+
+    def k_mi_bwd8(s, st):
+        _native.check(lib.lr_mi_backward(vp(s["mi_x8"]), vp(s["mi_y8"]), 8, nv, 32, -1.0, 1.0, vp(mi_hist), vp(ncc_g),
+                                         vp(s["mi_g8"]), st), "mi_bwd8")
+
     dice_names = ("dice", "dice_bwd", "dice_bwd8")
     if "labels2" in which or "labels6" in which or any(n in which for n in dice_names):
         # label maps as a validation item has them: mostly background, a few organ-sized blobs, target = shifted pred
@@ -225,7 +255,8 @@ def main():
     units = {"atten": (k_atten, nv, 8 * nv), "idmap": (k_idmap, nv, 12 * nv), "reg": (k_reg, nv, 12 * nv), "jac": (k_jac, nv, 12 * nv), "jac_map": (k_jac_map, nv, 16 * nv),
              "labels2": (k_labels(2), nv, 8 * nv), "labels6": (k_labels(6), nv, 8 * nv), "reg_bwd": (k_reg_bwd, nv, 24 * nv), "fold_bwd": (k_fold_bwd, nv, 24 * nv), "fold_bwd8": (k_fold_bwd8, 8 * nv, 8 * 24 * nv), "ncc": (k_ncc, nv, 8 * nv), "lncc": (k_lncc, nv, 8 * nv), "lncc_bwd": (k_lncc_bwd, nv, 44 * nv),
              "lncc_bwd8": (k_lncc_bwd8, 8 * nv, 8 * 44 * nv), "ngf": (k_ngf, nv, 8 * nv), "ngf_bwd": (k_ngf_bwd, nv, 12 * nv),
-             "ngf_bwd8": (k_ngf_bwd8, 8 * nv, 8 * 12 * nv), "dice": (k_dice, nv, 20 * nv), "dice_bwd": (k_dice_bwd, nv, 32 * nv),
+             "ngf_bwd8": (k_ngf_bwd8, 8 * nv, 8 * 12 * nv), "mi": (k_mi, nv, 8 * nv), "mi_bwd": (k_mi_bwd, nv, 12 * nv),
+             "mi_bwd8": (k_mi_bwd8, 8 * nv, 8 * 12 * nv), "dice": (k_dice, nv, 20 * nv), "dice_bwd": (k_dice_bwd, nv, 32 * nv),
              "dice_bwd8": (k_dice_bwd8, 8 * nv, 8 * 32 * nv), "ncc_bwd": (k_ncc_bwd, nv, 12 * nv), "warp": (k_warp, batch * nv, batch * 20 * nv), "pca": (k_pca, 3 * nv, 4 * 3 * nv * 56 + 8 * 3 * nv),
              "pca_bwd": (k_pca_bwd, 3 * nv, 4 * 3 * nv * 56 + 4 * 3 * nv), "warp_bwd": (k_warp_bwd, nv, 32 * nv),
              "drr_bwd": (k_drr_bwd, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240), "backproject": (k_backproject, batch * P * nv, batch * (4 * P * nv + 4 * P * DET[0] * DET[1])),
