@@ -321,6 +321,43 @@ LR_API int lr_jacobian_det(const float *phi, int B, int D, int H, int W, int bou
 LR_API int lr_label_confusion(const float *pred, const float *target, int B, int64_t N, int L,
                               int64_t *counts, int64_t *invalid, lr_stream_t stream);
 
+/* ---- surface-distance validation metrics (PARITY UNPINNED: the reference scores no surface metric) ------------------
+ * The boundary scores registration papers report next to Dice (Hausdorff, HD95, average symmetric surface distance)
+ * all follow from the directed surface distances below; metrics.surface_distance forms them.  These are voxel-based
+ * distances, not the surfel-area-weighted ones of DeepMind's surface_distance package.
+ *   pred, target / from, to: (B,D,H,W) float32 label maps (what the nearest-mode warp returns); labels 1..L-1 are
+ *   scored, L <= 128; a value that is not an integer in [0, L) is "no label".
+ *   The surface S_M(l) of label l in map M is the set of voxels with M == l that have at least one of their 6 face
+ *   neighbours outside the volume or != l (scipy's m & ~binary_erosion(m, generate_binary_structure(3, 1),
+ *   border_value=0)).
+ * lr_label_surface_counts: counts (B,2,L) int64 = [|S_pred(l)|, |S_target(l)|] for every l in [0, L) (exact), and
+ *   invalid (B) int64 = #voxels where either value is not an integer in [0, L), as lr_label_confusion counts them.
+ *   Both outputs are zeroed by the call.
+ * lr_surface_distances: for every voxel v of S_from(label), the distance from v to the nearest voxel n of S_to(label)
+ *   with spacing (s_d, s_h, s_w), formed from the index offsets as scipy's distance_transform_edt forms it, in fp64:
+ *     d(v) = sqrt(((s_d*(v_d - n_d))^2 + (s_h*(v_h - n_h))^2) + (s_w*(v_w - n_w))^2)    (+inf if S_to is empty)
+ *   The nearest voxel is found by an exact separable transform (Meijster et al. 2000); with integer spacings every
+ *   squared distance is an exact integer in fp64 and d(v) is bit-identical to scipy's whichever voxel a tie picks, and
+ *   otherwise it is within 8*2^-53*d(v) of it (DESIGN.md §3).
+ *   seg_offset (B+1) int64 in device memory, nondecreasing: item b's distances are written, in no particular order, to
+ *   dist[seg_offset[b] .. seg_offset[b+1]); a segment holds |S_from(label)| of the item when the offsets come from
+ *   lr_label_surface_counts of the same maps, and a write past a segment's end is dropped.
+ *   stats (B,3) float64, overwritten by the call: [count, sum, max] of each item's distances (max 0 when the count is
+ *   0).  The sum is reduced in a fixed order (no floating-point atomics), so repeated calls give the same bits.
+ *   The call needs a caller-owned device workspace of lr_surface_distance_workspace_bytes(B, D, H, W) bytes (16 per
+ *   voxel for the nearest-voxel intermediates and the envelope stacks, plus 24 per item and 128 columns for the
+ *   partial statistics; the call never allocates).
+ * Arguments: no null pointer; 1 <= B <= 65535; every axis >= 1; B*D*H*W < 2^31; 1 <= L <= 128; for the distances
+ * 1 <= label <= 127, H and W <= 65535 (the nearest voxel's (h, w) is packed into 32 bits), the spacings finite and > 0
+ * and the workspace large enough.  The checks run before any CUDA call; the workspace query returns 0 for sizes the
+ * call rejects.  Nothing depends on lr_set_numerics. */
+LR_API int lr_label_surface_counts(const float *pred, const float *target, int B, int D, int H, int W, int L,
+                                   int64_t *counts, int64_t *invalid, lr_stream_t stream);
+LR_API size_t lr_surface_distance_workspace_bytes(int B, int D, int H, int W);
+LR_API int lr_surface_distances(const float *from, const float *to, int B, int D, int H, int W, int label, double s_d,
+                                double s_h, double s_w, const int64_t *seg_offset, double *dist, double *stats,
+                                void *workspace, size_t workspace_bytes, lr_stream_t stream);
+
 /* ---- folding penalty (a training term; PARITY UNPINNED: the reference has no such term) ----------------------------
  *   fold(phi) = 1/(B*D*H*W) * sum_b sum_v max(0, -det_b(v))
  * det is, bit for bit, the determinant lr_jacobian_det computes for the same phi and boundary, over every voxel (no

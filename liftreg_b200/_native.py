@@ -63,6 +63,10 @@ SIGNATURES = {
     "lr_jacobian_det": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "lr_jacobian_fold_backward": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "lr_label_confusion": (_i, [_vp, _vp, _i, _i64, _i, _vp, _vp, _vp]),
+    "lr_label_surface_counts": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "lr_surface_distance_workspace_bytes": (_sz, [_i, _i, _i, _i]),
+    "lr_surface_distances": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.c_double, ctypes.c_double, ctypes.c_double, _vp, _vp,
+                                  _vp, _vp, _sz, _vp]),
     "lr_local_ncc_sum": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.c_double, _vp, _vp]),
     "lr_local_ncc_workspace_bytes": (_sz, [_i, _i, _i, _i, _i]),
     "lr_local_ncc_backward": (_i, [_vp, _vp, _i, _i, _i, _i, _i, ctypes.c_double, _vp, _vp, _vp, _sz, _vp]),

@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "_lib")
 LIB_PATH = os.path.join(LIB_DIR, "libliftreg_b200.so")
-SOURCES = ["api.cu", "warp.cu", "backproject.cu", "drr.cu", "pca_decode.cu", "losses.cu", "probe.cu"]
+SOURCES = ["api.cu", "warp.cu", "backproject.cu", "drr.cu", "pca_decode.cu", "losses.cu", "surface.cu", "probe.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(os.path.dirname(HERE), "include", "liftreg_b200.h")]
 
 NVCC_FLAGS = [

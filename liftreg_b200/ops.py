@@ -733,6 +733,79 @@ def label_confusion(pred, target, num_labels):
     return counts, invalid
 
 
+def _label_volumes(pred, target):
+    """Two label maps (B,1,D,H,W) or (B,D,H,W) of equal shape on one CUDA device -> contiguous float32 (B,D,H,W)."""
+    out = []
+    for t, name in ((pred, "pred"), (target, "target")):
+        t = _label_map(t, name)
+        if t.dim() == 5 and t.shape[1] == 1:
+            t = t[:, 0]
+        if t.dim() != 4:
+            raise ValueError("%s must be (B,1,D,H,W) or (B,D,H,W), got %s" % (name, tuple(t.shape)))
+        out.append(t.contiguous())
+    if out[0].shape != out[1].shape:
+        raise ValueError("pred %s and target %s must have the same shape" % (tuple(pred.shape), tuple(target.shape)))
+    if out[0].device != out[1].device:
+        raise ValueError("pred and target must be on the same device")
+    return out
+
+
+def label_surface_counts(pred, target, num_labels):
+    """Surface sizes of every label in two label maps (B,1,D,H,W) or (B,D,H,W) (float32 as the nearest-mode warp returns
+    them, or an integer dtype): counts (B,2,L) int64 = [|S_pred(l)|, |S_target(l)|] and invalid (B,) int64 = #voxels
+    where either value is not an integer in [0, L).  S_M(l) is the set of voxels labelled l with a face neighbour outside
+    the volume or labelled otherwise (include/liftreg_b200.h, lr_label_surface_counts).  1 <= num_labels <= 128."""
+    L = int(num_labels)
+    if not 1 <= L <= 128:
+        raise ValueError("num_labels must be in [1, 128], got %d" % L)
+    pred, target = _label_volumes(pred, target)
+    B, D, H, W = pred.shape
+    counts = torch.empty((B, 2, L), device=pred.device, dtype=torch.int64)
+    invalid = torch.empty((B,), device=pred.device, dtype=torch.int64)
+    with torch.cuda.device(pred.device):
+        _native.check(_native.lib().lr_label_surface_counts(_ptr(pred), _ptr(target), B, D, H, W, L, _ptr(counts),
+                                                            _ptr(invalid), _stream()), "lr_label_surface_counts")
+    return counts, invalid
+
+
+def surface_distances(from_map, to_map, label, spacing=(1.0, 1.0, 1.0), sizes=None):
+    """Directed surface distances of one label: for every voxel of S_from(label), the distance in mm to the nearest voxel
+    of S_to(label) with spacing (s_D, s_H, s_W), formed as scipy's distance_transform_edt forms it (include/liftreg_b200.h,
+    lr_surface_distances; +inf where S_to is empty).  Maps as in label_surface_counts.
+
+    sizes: |S_from(label)| per item (B,) on the host, e.g. label_surface_counts(...)[0][:, k, label] read back; None
+    runs that count pass here (a host synchronisation).  Returns (dist, seg_offset, stats) on the maps' device: dist
+    (sum(sizes),) float64 holds item b's distances, in no particular order, at [seg_offset[b], seg_offset[b+1]);
+    seg_offset (B+1,) int64; stats (B,3) float64 = [count, sum, max]."""
+    label = int(label)
+    if not 1 <= label <= 127:
+        raise ValueError("label must be in [1, 128), got %d" % label)
+    sp = [float(s) for s in spacing]
+    if len(sp) != 3 or not all(math.isfinite(s) and s > 0 for s in sp):
+        raise ValueError("spacing must be 3 finite values > 0, got %r" % (spacing,))
+    src, dst = _label_volumes(from_map, to_map)
+    B, D, H, W = src.shape
+    if sizes is None:
+        sizes = label_surface_counts(src, dst, 128)[0][:, 0, label].cpu().numpy()
+    sizes = np.asarray(sizes, dtype=np.int64).reshape(-1)
+    if sizes.shape != (B,) or (sizes < 0).any():
+        raise ValueError("sizes must hold B=%d counts >= 0, got %r" % (B, sizes))
+    offsets = np.concatenate([[0], np.cumsum(sizes)])
+    seg_offset = torch.from_numpy(offsets).to(src.device)
+    dist = torch.empty((max(int(offsets[-1]), 1),), device=src.device, dtype=torch.float64)
+    stats = torch.empty((B, 3), device=src.device, dtype=torch.float64)
+    lib = _native.lib()
+    nbytes = lib.lr_surface_distance_workspace_bytes(B, D, H, W)
+    if nbytes == 0:
+        raise ValueError("maps of shape %s are too large for lr_surface_distances (B*D*H*W < 2^31, B <= 65535, "
+                         "H and W <= 65535)" % (tuple(src.shape),))
+    ws = torch.empty((nbytes,), device=src.device, dtype=torch.uint8)
+    with torch.cuda.device(src.device):
+        _native.check(lib.lr_surface_distances(_ptr(src), _ptr(dst), B, D, H, W, label, sp[0], sp[1], sp[2], _ptr(seg_offset),
+                                               _ptr(dist), _ptr(stats), _ptr(ws), nbytes, _stream()), "lr_surface_distances")
+    return dist[:int(offsets[-1])], seg_offset, stats
+
+
 # --------------------------------------------------------------------------- soft Dice of the warped labels (training term)
 def _dice_loss_from_sums(sums):
     """1 - mean_b of the mean over S_b = {l >= 1 : P + T > 0} of 2 I / (P + T) (1 where S_b is empty), from sums

@@ -246,6 +246,34 @@ def main():
                                                  vp(conf_invalid), st), "labels%d" % L)
         return k
 
+    if "sdist" in which or "sdist8" in which:
+        # the phantom's two lungs (labels 1, 2) as target, the same map warped (nearest) by a smooth displacement as
+        # pred; B = 8 stacks 8 displacements.  One map pair and one workspace serve every set: the 16 B/voxel workspace
+        # is larger than L2 at B = 8 and about half of it at B = 1.
+        zz, yy, xx = np.meshgrid(*[np.linspace(-1, 1, n) for n in VOL], indexing="ij")
+        lung = np.zeros(VOL, np.float32)
+        for l, cx in ((1, -0.38), (2, 0.38)):
+            lung[(zz / 0.62) ** 2 + (yy / 0.45) ** 2 + ((xx - cx) / 0.30) ** 2 <= 1.0] = l
+        disp8 = torch.from_numpy(np.stack([synthetic.smooth_displacement(VOL, seed=b) for b in range(8)])).to(dev)
+        tgt8 = torch.from_numpy(lung).to(dev)[None, None].repeat(8, 1, 1, 1, 1)
+        pred8 = ops.warp(tgt8, disp8, zero_boundary=True, using_scale=False, mode="nearest", disp_plus_identity=True)
+        sd = {}
+        for nb in (1, 8):
+            cnt = ops.label_surface_counts(pred8[:nb], tgt8[:nb], 3)[0][:, :, 1].cpu().numpy()     # label 1 (one lung)
+            offs = [torch.from_numpy(np.concatenate([[0], np.cumsum(cnt[:, k])])).to(dev) for k in (0, 1)]
+            nbytes = lib.lr_surface_distance_workspace_bytes(nb, *VOL)
+            sd[nb] = (pred8[:nb].contiguous(), tgt8[:nb].contiguous(), offs,
+                      torch.empty(int(cnt.sum(0).max()), device=dev, dtype=torch.float64),
+                      torch.empty((nb, 3), device=dev, dtype=torch.float64), torch.empty(nbytes, device=dev, dtype=torch.uint8), nbytes)
+
+    def k_sdist_b(nb):         # both directed surface distances of one lung label: pred -> target and target -> pred
+        def k(s, st):
+            p, t, offs, dist, stats, ws, nbytes = sd[nb]
+            for a, b, off in ((p, t, offs[0]), (t, p, offs[1])):
+                _native.check(lib.lr_surface_distances(vp(a), vp(b), nb, *VOL, 1, 2.2, 2.2, 2.2, vp(off), vp(dist), vp(stats),
+                                                       vp(ws), nbytes, st), "sdist")
+        return k
+
     def k_atten(s, st):        # HU -> attenuation (sdct:6-13), elementwise
         _native.check(lib.lr_atten_coef(vp(s["moving"]), nv, vp(s["warped"]), st), "atten")
 
@@ -261,7 +289,9 @@ def main():
              "pca_bwd": (k_pca_bwd, 3 * nv, 4 * 3 * nv * 56 + 4 * 3 * nv), "warp_bwd": (k_warp_bwd, nv, 32 * nv),
              "drr_bwd": (k_drr_bwd, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240), "backproject": (k_backproject, batch * P * nv, batch * (4 * P * nv + 4 * P * DET[0] * DET[1])),
              "drr": (k_drr, P * 240 * 240 * VOL[1], 4 * nv + 4 * P * 240 * 240),
-             "drr256": (k_drr256, P * 256 * 256 * VOL[1], 4 * nv + 4 * P * 256 * 256)}
+             "drr256": (k_drr256, P * 256 * 256 * VOL[1], 4 * nv + 4 * P * 256 * 256),
+             # per direction: both maps read once, the two 4-byte intermediates written and read once (24 B per voxel)
+             "sdist": (k_sdist_b(1), 2 * nv, 2 * 24 * nv), "sdist8": (k_sdist_b(8), 2 * 8 * nv, 2 * 8 * 24 * nv)}
     for name in which:
         fn, n_units, nbytes = units[name]
         g = torch.cuda.CUDAGraph()
