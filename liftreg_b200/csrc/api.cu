@@ -72,7 +72,7 @@ static bool zero_copy_enabled() {
     return v != 0;
 }
 
-static int cuda_ok(cudaError_t e, const char *what) {
+int cuda_ok(cudaError_t e, const char *what) {
     if (e == cudaSuccess) return LR_OK;
     set_error("%s: %s", what, cudaGetErrorString(e));
     return LR_ERR_CUDA;

@@ -157,9 +157,36 @@ __device__ __forceinline__ void red_add_if(bool on, float *p, float v) {
 namespace lr {
 void set_error(const char *fmt, ...);
 int check_launch(const char *what);  // cudaGetLastError -> lr_status; bumps the per-thread launch counter
+int cuda_ok(cudaError_t e, const char *what);  // LR_OK, or LR_ERR_CUDA with the error "what: <cuda message>"
 int sm_count();                      // multiprocessors of the current device (cached per device)
 int numerics_mode();                 // LR_NUMERICS_FAST / LR_NUMERICS_EXACT (lr_set_numerics)
 inline cudaStream_t as_stream(lr_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }
+
+// Resident blocks per SM of `kernel`, or `fallback` when the occupancy query fails (its error is cleared, so that the
+// next check_launch does not report it) or finds none.
+template <typename K>
+int blocks_per_sm(K kernel, int threads, size_t smem, int fallback) {
+    int n = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, threads, smem) != cudaSuccess || n < 1) {
+        cudaGetLastError();
+        n = fallback;
+    }
+    return n;
+}
+
+// Raise the dynamic shared-memory limit of `kernel` to `bytes` (the > 48 KB opt-in).  The attribute belongs to the
+// current device, so it is set again whenever the device differs from `done_dev`, the caller's per-thread record of
+// the last device it was set on.
+template <typename K>
+cudaError_t opt_in_smem(K kernel, int bytes, int &done_dev) {
+    int dev = 0;
+    cudaError_t ce = cudaGetDevice(&dev);
+    if (ce == cudaSuccess && dev != done_dev) {
+        ce = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        if (ce == cudaSuccess) done_dev = dev;
+    }
+    return ce;
+}
 
 // ATen grid_sampler_unnormalize(align_corners) then optional clip_coordinates: the sample coordinate of the warp, and
 // of every kernel that samples as the warp does.

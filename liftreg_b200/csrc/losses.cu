@@ -324,14 +324,11 @@ __global__ void __launch_bounds__(NCC_THREADS, LR_REGP_MINB) diffusion_reg_pair_
         const unsigned pl = (unsigned)(g.h * g.w), cs = pl * (unsigned)g.d;
         unsigned i0 = ((unsigned)b * 3u * (unsigned)g.d + (unsigned)z0) * pl + (unsigned)y * (unsigned)g.w + (unsigned)x;
         const f32x2 sd2 = splat2(g.sd), sh2 = splat2(g.sh), sw2 = splat2(g.sw);
-#ifndef LR_REG_WINDOW
-#define LR_REG_WINDOW 1
-#endif
         f32x2 vm[3], vc[3];
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
-            vc[c] = LR_REG_WINDOW ? ldg2(disp + (i0 + c * cs)) : 0ull;
-            vm[c] = LR_REG_WINDOW ? (z0 > 0 ? ldg2(disp + (i0 + c * cs - pl)) : vc[c]) : 0ull;
+            vc[c] = ldg2(disp + (i0 + c * cs));
+            vm[c] = z0 > 0 ? ldg2(disp + (i0 + c * cs - pl)) : vc[c];
         }
         f32x2 part = 0ull;                                               // fp32 partial sums of at most 16 planes
         for (int z = z0; z < z1; ++z, i0 += pl) {
@@ -340,8 +337,7 @@ __global__ void __launch_bounds__(NCC_THREADS, LR_REGP_MINB) diffusion_reg_pair_
 #pragma unroll
             for (int c = 0; c < 3; ++c) {
                 const unsigned ic = i0 + c * cs;
-                const f32x2 cc = LR_REG_WINDOW ? vc[c] : ldg2(disp + ic);
-                if (!LR_REG_WINDOW) vm[c] = zlo ? cc : ldg2(disp + (ic - pl));
+                const f32x2 cc = vc[c];
                 const f32x2 vp = zhi ? cc : ldg2(disp + (ic + pl));      // allocating load: next iteration's row neighbours hit L1
                 if (LR_REG_PF > 0 && z + LR_REG_PF <= z1) prefetch_l2(disp + (ic + LR_REG_PF * pl));
                 const f32x2 yu = ldg2(disp + (ic + oyu)), yd = ldg2(disp + (ic + oyd));
@@ -451,9 +447,7 @@ static int march_dims(K kernel, int threads, int tile_w, int tile_h, int waves, 
     const int64_t tiles = (int64_t)((W + tile_w - 1) / tile_w) * ((H + tile_h - 1) / tile_h) * B;
     // ONE wave of blocks when the tiles allow it (a second, nearly empty wave would double the time of this short
     // kernel): as many chunks of planes as fit the resident-block capacity, chunks of at least 4 planes
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
-    const int64_t capacity = (int64_t)sm_count() * per_sm * waves;
+    const int64_t capacity = (int64_t)sm_count() * blocks_per_sm(kernel, threads, 0, 4) * waves;
     int64_t chunks = capacity / tiles;
     if (chunks < 1) chunks = 1;
     if (chunks > (D + 3) / 4) chunks = (D + 3) / 4;
@@ -1557,8 +1551,7 @@ extern "C" int lr_ncc_sums(const float *x, const float *y, int B, int64_t N, dou
     LR_REQUIRE(x && y && sums, "ncc_sums: null pointer");
     LR_REQUIRE(B > 0 && B <= 65535 && N > 0, "ncc_sums: bad size (B=%d N=%lld)", B, (long long)N);
     cudaStream_t st = as_stream(stream);
-    cudaError_t ce = cudaMemsetAsync(sums, 0, sizeof(double) * NCC_SUMS * (size_t)B, st);
-    if (ce != cudaSuccess) { set_error("ncc_sums: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    if (int e = cuda_ok(cudaMemsetAsync(sums, 0, sizeof(double) * NCC_SUMS * (size_t)B, st), "ncc_sums: memset failed")) return e;
     const dim3 grid(ncc_blocks(N, B), (unsigned)B);
     ncc_shifted_kernel<<<grid, NCC_THREADS, 0, st>>>(x, y, N, sums);
     if (int e = check_launch("ncc_shifted_kernel")) return e;
@@ -1575,51 +1568,68 @@ extern "C" int lr_ncc_backward(const float *x, const float *y, int B, int64_t N,
     return check_launch("ncc_backward_kernel");
 }
 
-extern "C" int lr_diffusion_reg_sum(const float *disp, int B, int D, int H, int W, int boundary, double *sum, lr_stream_t stream) {
-    LR_REQUIRE(disp && sum, "diffusion_reg_sum: null pointer");
-    LR_REQUIRE(B > 0 && D >= 2 && H >= 2 && W >= 2, "diffusion_reg_sum: every axis needs >= 2 entries (B=%d, %dx%dx%d)", B, D, H, W);
-    LR_REQUIRE(boundary == LR_FD_LINEAR || boundary == LR_FD_NEUMANN_ZERO, "diffusion_reg_sum: unknown boundary mode %d", boundary);
+// argument rules shared by the finite-difference entries over `channels` (D,H,W) volumes per item, which the kernels
+// index with 32 bits, of which the `margin` voxels next to every face are left out (only jacobian_det skips any); 0 when
+// they hold
+static int fd_check(const char *who, int B, int D, int H, int W, int boundary, int channels, int margin = 0) {
+    LR_REQUIRE(B > 0 && D >= 2 && H >= 2 && W >= 2, "%s: every axis needs >= 2 entries (B=%d, %dx%dx%d)", who, B, D, H, W);
+    LR_REQUIRE(boundary == LR_FD_LINEAR || boundary == LR_FD_NEUMANN_ZERO, "%s: unknown boundary mode %d", who, boundary);
+    LR_REQUIRE(margin >= 0 && 2 * (int64_t)margin < D && 2 * (int64_t)margin < H && 2 * (int64_t)margin < W,
+               "%s: margin %d leaves no interior voxel of %dx%dx%d (2*margin must be < every axis)", who, margin, D, H, W);
+    LR_REQUIRE((int64_t)B * channels * D * H * W < ((int64_t)1 << 31),
+               channels == 3 ? "%s: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)"
+                             : "%s: too large for one launch (B=%d, %dx%dx%d; B*D*H*W must stay below 2^31)",
+               who, B, D, H, W);
+    return 0;
+}
+
+template <int MODE>
+static int diffusion_reg_launch(const float *disp, int B, int D, int H, int W, double *sum, cudaStream_t st) {
     RegDims g; dim3 grid;
     const bool pairs = reg_use_pairs(disp, nullptr, W);
-    const int rd = pairs ? (boundary == LR_FD_LINEAR ? reg_dims(diffusion_reg_pair_kernel<0>, true, LR_REG_WAVES, B, D, H, W, g, grid)
-                                                     : reg_dims(diffusion_reg_pair_kernel<1>, true, LR_REG_WAVES, B, D, H, W, g, grid))
-                         : (boundary == LR_FD_LINEAR ? reg_dims(diffusion_reg_kernel<0>, false, LR_REG_WAVES, B, D, H, W, g, grid)
-                                                     : reg_dims(diffusion_reg_kernel<1>, false, LR_REG_WAVES, B, D, H, W, g, grid));
+    const int rd = pairs ? reg_dims(diffusion_reg_pair_kernel<MODE>, true, LR_REG_WAVES, B, D, H, W, g, grid)
+                         : reg_dims(diffusion_reg_kernel<MODE>, false, LR_REG_WAVES, B, D, H, W, g, grid);
     LR_REQUIRE(rd == 0, "diffusion_reg_sum: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)", B, D, H, W);
-    cudaStream_t st = as_stream(stream);
-    cudaError_t ce = cudaMemsetAsync(sum, 0, sizeof(double), st);
-    if (ce != cudaSuccess) { set_error("diffusion_reg_sum: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    if (int e = cuda_ok(cudaMemsetAsync(sum, 0, sizeof(double), st), "diffusion_reg_sum: memset failed")) return e;
     if (pairs) {
-        if (boundary == LR_FD_LINEAR) diffusion_reg_pair_kernel<0><<<grid, NCC_THREADS, 0, st>>>(disp, g, sum);
-        else diffusion_reg_pair_kernel<1><<<grid, NCC_THREADS, 0, st>>>(disp, g, sum);
+        diffusion_reg_pair_kernel<MODE><<<grid, NCC_THREADS, 0, st>>>(disp, g, sum);
         return check_launch("diffusion_reg_pair_kernel");
     }
-    if (boundary == LR_FD_LINEAR) diffusion_reg_kernel<0><<<grid, NCC_THREADS, 0, st>>>(disp, g, sum);
-    else diffusion_reg_kernel<1><<<grid, NCC_THREADS, 0, st>>>(disp, g, sum);
+    diffusion_reg_kernel<MODE><<<grid, NCC_THREADS, 0, st>>>(disp, g, sum);
     return check_launch("diffusion_reg_kernel");
+}
+
+extern "C" int lr_diffusion_reg_sum(const float *disp, int B, int D, int H, int W, int boundary, double *sum, lr_stream_t stream) {
+    LR_REQUIRE(disp && sum, "diffusion_reg_sum: null pointer");
+    if (int e = fd_check("diffusion_reg_sum", B, D, H, W, boundary, 3)) return e;
+    cudaStream_t st = as_stream(stream);
+    return boundary == LR_FD_LINEAR ? diffusion_reg_launch<0>(disp, B, D, H, W, sum, st)
+                                    : diffusion_reg_launch<1>(disp, B, D, H, W, sum, st);
+}
+
+template <int MODE>
+static int diffusion_reg_backward_launch(const float *disp, int B, int D, int H, int W, const float *grad_loss, float *grad_disp,
+                                         cudaStream_t st) {
+    RegDims g; dim3 grid;
+    const bool pairs = reg_use_pairs(disp, grad_disp, W);
+    const int rd = pairs ? reg_dims(diffusion_reg_backward_pair_kernel<MODE>, true, LR_REG_BWD_WAVES, B, D, H, W, g, grid)
+                         : reg_dims(diffusion_reg_backward_kernel<MODE>, false, LR_REG_BWD_WAVES, B, D, H, W, g, grid);
+    LR_REQUIRE(rd == 0, "diffusion_reg_backward: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)", B, D, H, W);
+    if (pairs) {
+        diffusion_reg_backward_pair_kernel<MODE><<<grid, NCC_THREADS, 0, st>>>(disp, g, B, grad_loss, grad_disp);
+        return check_launch("diffusion_reg_backward_pair_kernel");
+    }
+    diffusion_reg_backward_kernel<MODE><<<grid, NCC_THREADS, 0, st>>>(disp, g, B, grad_loss, grad_disp);
+    return check_launch("diffusion_reg_backward_kernel");
 }
 
 extern "C" int lr_diffusion_reg_backward(const float *disp, int B, int D, int H, int W, int boundary, const float *grad_loss,
                                          float *grad_disp, lr_stream_t stream) {
     LR_REQUIRE(disp && grad_loss && grad_disp, "diffusion_reg_backward: null pointer");
-    LR_REQUIRE(B > 0 && D >= 2 && H >= 2 && W >= 2, "diffusion_reg_backward: every axis needs >= 2 entries (B=%d, %dx%dx%d)", B, D, H, W);
-    LR_REQUIRE(boundary == LR_FD_LINEAR || boundary == LR_FD_NEUMANN_ZERO, "diffusion_reg_backward: unknown boundary mode %d", boundary);
-    RegDims g; dim3 grid;
-    const bool pairs = reg_use_pairs(disp, grad_disp, W);
-    const int rd = pairs ? (boundary == LR_FD_LINEAR ? reg_dims(diffusion_reg_backward_pair_kernel<0>, true, LR_REG_BWD_WAVES, B, D, H, W, g, grid)
-                                                     : reg_dims(diffusion_reg_backward_pair_kernel<1>, true, LR_REG_BWD_WAVES, B, D, H, W, g, grid))
-                         : (boundary == LR_FD_LINEAR ? reg_dims(diffusion_reg_backward_kernel<0>, false, LR_REG_BWD_WAVES, B, D, H, W, g, grid)
-                                                     : reg_dims(diffusion_reg_backward_kernel<1>, false, LR_REG_BWD_WAVES, B, D, H, W, g, grid));
-    LR_REQUIRE(rd == 0, "diffusion_reg_backward: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)", B, D, H, W);
+    if (int e = fd_check("diffusion_reg_backward", B, D, H, W, boundary, 3)) return e;
     cudaStream_t st = as_stream(stream);
-    if (pairs) {
-        if (boundary == LR_FD_LINEAR) diffusion_reg_backward_pair_kernel<0><<<grid, NCC_THREADS, 0, st>>>(disp, g, B, grad_loss, grad_disp);
-        else diffusion_reg_backward_pair_kernel<1><<<grid, NCC_THREADS, 0, st>>>(disp, g, B, grad_loss, grad_disp);
-        return check_launch("diffusion_reg_backward_pair_kernel");
-    }
-    if (boundary == LR_FD_LINEAR) diffusion_reg_backward_kernel<0><<<grid, NCC_THREADS, 0, st>>>(disp, g, B, grad_loss, grad_disp);
-    else diffusion_reg_backward_kernel<1><<<grid, NCC_THREADS, 0, st>>>(disp, g, B, grad_loss, grad_disp);
-    return check_launch("diffusion_reg_backward_kernel");
+    return boundary == LR_FD_LINEAR ? diffusion_reg_backward_launch<0>(disp, B, D, H, W, grad_loss, grad_disp, st)
+                                    : diffusion_reg_backward_launch<1>(disp, B, D, H, W, grad_loss, grad_disp, st);
 }
 
 template <int MODE>
@@ -1642,12 +1652,7 @@ static int jacobian_launch(const float *phi, int B, int D, int H, int W, int mar
 extern "C" int lr_jacobian_det(const float *phi, int B, int D, int H, int W, int boundary, int margin, float *det, double *stats,
                                lr_stream_t stream) {
     LR_REQUIRE(phi && stats, "jacobian_det: null pointer");
-    LR_REQUIRE(B > 0 && D >= 2 && H >= 2 && W >= 2, "jacobian_det: every axis needs >= 2 entries (B=%d, %dx%dx%d)", B, D, H, W);
-    LR_REQUIRE(boundary == LR_FD_LINEAR || boundary == LR_FD_NEUMANN_ZERO, "jacobian_det: unknown boundary mode %d", boundary);
-    LR_REQUIRE(margin >= 0 && 2 * (int64_t)margin < D && 2 * (int64_t)margin < H && 2 * (int64_t)margin < W,
-               "jacobian_det: margin %d leaves no interior voxel of %dx%dx%d (2*margin must be < every axis)", margin, D, H, W);
-    LR_REQUIRE((int64_t)B * 3 * D * H * W < ((int64_t)1 << 31),
-               "jacobian_det: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)", B, D, H, W);
+    if (int e = fd_check("jacobian_det", B, D, H, W, boundary, 3, margin)) return e;
     cudaStream_t st = as_stream(stream);
     return boundary == LR_FD_LINEAR ? jacobian_launch<0>(phi, B, D, H, W, margin, det, stats, st)
                                     : jacobian_launch<1>(phi, B, D, H, W, margin, det, stats, st);
@@ -1665,10 +1670,7 @@ static int fold_backward_launch(const float *phi, int B, int D, int H, int W, co
 extern "C" int lr_jacobian_fold_backward(const float *phi, int B, int D, int H, int W, int boundary, const float *grad_loss,
                                          float *grad_phi, lr_stream_t stream) {
     LR_REQUIRE(phi && grad_loss && grad_phi, "jacobian_fold_backward: null pointer");
-    LR_REQUIRE(B > 0 && D >= 2 && H >= 2 && W >= 2, "jacobian_fold_backward: every axis needs >= 2 entries (B=%d, %dx%dx%d)", B, D, H, W);
-    LR_REQUIRE(boundary == LR_FD_LINEAR || boundary == LR_FD_NEUMANN_ZERO, "jacobian_fold_backward: unknown boundary mode %d", boundary);
-    LR_REQUIRE((int64_t)B * 3 * D * H * W < ((int64_t)1 << 31),
-               "jacobian_fold_backward: field too large for one launch (B=%d, %dx%dx%d; B*3*D*H*W must stay below 2^31)", B, D, H, W);
+    if (int e = fd_check("jacobian_fold_backward", B, D, H, W, boundary, 3)) return e;
     cudaStream_t st = as_stream(stream);
     return boundary == LR_FD_LINEAR ? fold_backward_launch<0>(phi, B, D, H, W, grad_loss, grad_phi, st)
                                     : fold_backward_launch<1>(phi, B, D, H, W, grad_loss, grad_phi, st);
@@ -1681,21 +1683,11 @@ extern "C" int lr_label_confusion(const float *pred, const float *target, int B,
     LR_REQUIRE(B > 0 && B <= 65535 && N > 0, "label_confusion: bad size (B=%d N=%lld)", B, (long long)N);
     cudaStream_t st = as_stream(stream);
     const size_t smem = sizeof(unsigned) * ((size_t)L * L + 1);
-    static thread_local int attr_dev = -1, per_sm = 0;       // the > 48 KB opt-in is per device
-    int dev = 0;
-    cudaError_t ce = cudaGetDevice(&dev);
-    if (ce == cudaSuccess && dev != attr_dev) {
-        ce = cudaFuncSetAttribute(label_confusion_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(unsigned) * (128 * 128 + 1)));
-        if (ce == cudaSuccess) attr_dev = dev;
-    }
-    if (ce != cudaSuccess) { set_error("label_confusion: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, label_confusion_kernel, CONF_THREADS, smem) != cudaSuccess || per_sm < 1) {
-        cudaGetLastError();
-        per_sm = 1;
-    }
-    ce = cudaMemsetAsync(counts, 0, sizeof(int64_t) * (size_t)B * L * L, st);
-    if (ce == cudaSuccess) ce = cudaMemsetAsync(invalid, 0, sizeof(int64_t) * (size_t)B, st);
-    if (ce != cudaSuccess) { set_error("label_confusion: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    static thread_local int smem_dev = -1;
+    if (int e = cuda_ok(opt_in_smem(label_confusion_kernel, (int)(sizeof(unsigned) * (128 * 128 + 1)), smem_dev), "label_confusion")) return e;
+    const int per_sm = blocks_per_sm(label_confusion_kernel, CONF_THREADS, smem, 1);
+    if (int e = cuda_ok(cudaMemsetAsync(counts, 0, sizeof(int64_t) * (size_t)B * L * L, st), "label_confusion: memset failed")) return e;
+    if (int e = cuda_ok(cudaMemsetAsync(invalid, 0, sizeof(int64_t) * (size_t)B, st), "label_confusion: memset failed")) return e;
     const dim3 grid(conf_blocks(N, B, L, per_sm), (unsigned)B);
     label_confusion_kernel<<<grid, CONF_THREADS, smem, st>>>(pred, target, N, L, reinterpret_cast<unsigned long long *>(counts),
                                                               reinterpret_cast<unsigned long long *>(invalid));
@@ -1717,20 +1709,10 @@ static int lncc_check(const char *who, int B, int D, int H, int W, int win, doub
 template <int KIND>
 static int lncc_launch(const float *x, const float *y, const float *coef, int B, int D, int H, int W, int win, double eps,
                        const float *grad_loss, double *sum, float *out, cudaStream_t st, const char *name) {
-    static thread_local int attr_dev = -1;          // the > 48 KB opt-in is per device
-    int dev = 0;
-    cudaError_t ce = cudaGetDevice(&dev);
-    if (ce == cudaSuccess && dev != attr_dev) {
-        ce = cudaFuncSetAttribute(local_ncc_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lncc_smem_bytes<KIND>(LNCC_WMAX));
-        if (ce == cudaSuccess) attr_dev = dev;
-    }
-    if (ce != cudaSuccess) { set_error("%s: %s", name, cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    static thread_local int smem_dev = -1;
+    if (int e = cuda_ok(opt_in_smem(local_ncc_kernel<KIND>, (int)lncc_smem_bytes<KIND>(LNCC_WMAX), smem_dev), name)) return e;
     const size_t smem = lncc_smem_bytes<KIND>(win);
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, local_ncc_kernel<KIND>, LNCC_THREADS, smem) != cudaSuccess || per_sm < 1) {
-        cudaGetLastError();
-        per_sm = 1;
-    }
+    const int per_sm = blocks_per_sm(local_ncc_kernel<KIND>, LNCC_THREADS, smem, 1);
     LnccDims g;
     g.D = D; g.H = H; g.W = W; g.w = win;
     g.N = (unsigned)D * (unsigned)H * (unsigned)W;
@@ -1755,8 +1737,7 @@ extern "C" int lr_local_ncc_sum(const float *x, const float *y, int B, int D, in
     LR_REQUIRE(x && y && sum, "local_ncc_sum: null pointer");
     if (int e = lncc_check("local_ncc_sum", B, D, H, W, win, eps)) return e;
     cudaStream_t st = as_stream(stream);
-    cudaError_t ce = cudaMemsetAsync(sum, 0, sizeof(double) * (size_t)B, st);
-    if (ce != cudaSuccess) { set_error("local_ncc_sum: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    if (int e = cuda_ok(cudaMemsetAsync(sum, 0, sizeof(double) * (size_t)B, st), "local_ncc_sum: memset failed")) return e;
     return lncc_launch<LNCC_FWD>(x, y, nullptr, B, D, H, W, win, eps, nullptr, sum, nullptr, st, "local_ncc_kernel<fwd>");
 }
 
@@ -1807,8 +1788,7 @@ extern "C" int lr_label_dice_sums(const float *phi, const float *src, const floa
     DiceDims g; dim3 grid;
     if (int e = dice_dims(label_dice_sums_kernel, "label_dice_sums", B, D, H, W, L, g, grid)) return e;
     cudaStream_t st = as_stream(stream);
-    cudaError_t ce = cudaMemsetAsync(sums, 0, sizeof(double) * 3 * (size_t)B * L, st);
-    if (ce != cudaSuccess) { set_error("label_dice_sums: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    if (int e = cuda_ok(cudaMemsetAsync(sums, 0, sizeof(double) * 3 * (size_t)B * L, st), "label_dice_sums: memset failed")) return e;
     label_dice_sums_kernel<<<grid, DICE_THREADS, 0, st>>>(phi, src, tgt, g, sums);
     return check_launch("label_dice_sums_kernel");
 }
@@ -1826,11 +1806,7 @@ extern "C" int lr_label_dice_backward(const float *phi, const float *src, const 
 // argument rules shared by the NGF entries; 0 when they hold.  eps >= 1e-77 keeps p*q >= eps^4 > 0 in fp64.
 static int ngf_check(const char *who, int B, int D, int H, int W, int boundary, double eps) {
     LR_REQUIRE(eps >= 1e-77 && eps <= DBL_MAX, "%s: eps must be finite and > 0 (>= 1e-77; got %g)", who, eps);
-    LR_REQUIRE(B >= 1 && D >= 2 && H >= 2 && W >= 2, "%s: every axis needs >= 2 entries (B=%d, %dx%dx%d)", who, B, D, H, W);
-    LR_REQUIRE(boundary == LR_FD_LINEAR || boundary == LR_FD_NEUMANN_ZERO, "%s: unknown boundary mode %d", who, boundary);
-    LR_REQUIRE((int64_t)B * D * H * W < ((int64_t)1 << 31), "%s: too large for one launch (B=%d, %dx%dx%d; B*D*H*W must stay below 2^31)",
-               who, B, D, H, W);
-    return 0;
+    return fd_check(who, B, D, H, W, boundary, 1);
 }
 
 template <int MODE>
@@ -1838,8 +1814,7 @@ static int ngf_sum_launch(const float *x, const float *y, int B, int D, int H, i
     RegDims g; dim3 grid;
     LR_REQUIRE(march_dims(ngf_sum_kernel<MODE>, NCC_THREADS, REG_TX, REG_TY, LR_REG_WAVES, B, D, H, W, g, grid, 1) == 0,
                "ngf_sum: too many blocks for one launch (B=%d, %dx%dx%d)", B, D, H, W);
-    cudaError_t ce = cudaMemsetAsync(sum, 0, sizeof(double) * (size_t)B, st);
-    if (ce != cudaSuccess) { set_error("ngf_sum: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    if (int e = cuda_ok(cudaMemsetAsync(sum, 0, sizeof(double) * (size_t)B, st), "ngf_sum: memset failed")) return e;
     ngf_sum_kernel<MODE><<<grid, NCC_THREADS, 0, st>>>(x, y, g, eps * eps, sum);
     return check_launch("ngf_sum_kernel");
 }
@@ -1891,16 +1866,6 @@ static unsigned mi_blocks(int64_t N, int B, int threads, int per_sm) {
     return (unsigned)(want < 1 ? 1 : want);
 }
 
-template <typename K>
-static int mi_per_sm(K kernel, int threads, size_t smem) {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem) != cudaSuccess || per_sm < 1) {
-        cudaGetLastError();
-        per_sm = 1;
-    }
-    return per_sm;
-}
-
 extern "C" int lr_mi_hist(const float *x, const float *y, int B, int64_t N, int num_bins, float lo, float hi, double *hist,
                           lr_stream_t stream) {
     LR_REQUIRE(x && y && hist, "mi_hist: null pointer");
@@ -1908,9 +1873,8 @@ extern "C" int lr_mi_hist(const float *x, const float *y, int B, int64_t N, int 
     if (int e = mi_check("mi_hist", B, N, num_bins, lo, hi, m)) return e;
     cudaStream_t st = as_stream(stream);
     const size_t nbins = (size_t)num_bins * (num_bins + 2), smem = sizeof(double) * nbins;
-    cudaError_t ce = cudaMemsetAsync(hist, 0, sizeof(double) * nbins * (size_t)B, st);
-    if (ce != cudaSuccess) { set_error("mi_hist: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
-    const dim3 grid(mi_blocks(N, B, MI_THREADS, mi_per_sm(mi_hist_kernel, MI_THREADS, smem)), (unsigned)B);
+    if (int e = cuda_ok(cudaMemsetAsync(hist, 0, sizeof(double) * nbins * (size_t)B, st), "mi_hist: memset failed")) return e;
+    const dim3 grid(mi_blocks(N, B, MI_THREADS, blocks_per_sm(mi_hist_kernel, MI_THREADS, smem, 1)), (unsigned)B);
     mi_hist_kernel<<<grid, MI_THREADS, smem, st>>>(x, y, N, m, hist);
     return check_launch("mi_hist_kernel");
 }
@@ -1921,7 +1885,7 @@ extern "C" int lr_mi_backward(const float *x, const float *y, int B, int64_t N, 
     MiMap m;
     if (int e = mi_check("mi_backward", B, N, num_bins, lo, hi, m)) return e;
     const size_t smem = sizeof(float) * (size_t)num_bins * (num_bins + 2);
-    const dim3 grid(mi_blocks(N, B, MI_BWD_THREADS, mi_per_sm(mi_backward_kernel, MI_BWD_THREADS, smem)), (unsigned)B);
+    const dim3 grid(mi_blocks(N, B, MI_BWD_THREADS, blocks_per_sm(mi_backward_kernel, MI_BWD_THREADS, smem, 1)), (unsigned)B);
     mi_backward_kernel<<<grid, MI_BWD_THREADS, smem, as_stream(stream)>>>(x, y, N, B, m, hist, grad_loss, grad_x);
     return check_launch("mi_backward_kernel");
 }

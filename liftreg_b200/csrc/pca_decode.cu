@@ -405,11 +405,10 @@ static int launch_pca(const float *coefs, const float *basis, const float *mean,
         // + 4 floats: the compiler reads the coefficient table four at a time in the k-loop's remainder iterations
         const size_t smem_t = sizeof(float) * ((size_t)PT_STAGES * PT_ROWS * g.K + (size_t)g.K * BT + 4);
         if (smem_t <= 110 * 1024) {
-            static thread_local bool attr_done = false;
-            if (smem_t > 48 * 1024 && !attr_done) {
-                cudaError_t e = cudaFuncSetAttribute(pca_decode_tma_kernel<BT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
-                if (e != cudaSuccess) { set_error("pca_decode: cannot raise shared memory limit: %s", cudaGetErrorString(e)); return LR_ERR_CUDA; }
-                attr_done = true;
+            if (smem_t > 48 * 1024) {
+                static thread_local int smem_dev = -1;
+                const cudaError_t ce = opt_in_smem(pca_decode_tma_kernel<BT>, 110 * 1024, smem_dev);
+                if (int e = cuda_ok(ce, "pca_decode: cannot raise shared memory limit")) return e;
             }
             const int64_t n_tiles = (g.N + PT_ROWS - 1) / PT_ROWS;
             int per_sm = (int)((224 * 1024) / (smem_t + 1024));
@@ -424,15 +423,16 @@ static int launch_pca(const float *coefs, const float *basis, const float *mean,
     // + 4 floats: the compiler reads the coefficient table four at a time in the k-loop's remainder iterations
     const size_t smem = sizeof(float) * ((size_t)PD_ROWS * pitch + (size_t)g.K * BT + 4);
     if (smem > 200 * 1024) { set_error("pca_decode: K=%d needs %zu bytes of shared memory", g.K, smem); return LR_ERR_BAD_ARGUMENT; }
-    if (smem > 48 * 1024) {       // opt in to large dynamic shared memory (idempotent, cheap)
-        cudaError_t e = vec ? cudaFuncSetAttribute(pca_decode_kernel<BT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024)
-                            : cudaFuncSetAttribute(pca_decode_scalar_kernel<BT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) { set_error("pca_decode: cannot raise shared memory limit: %s", cudaGetErrorString(e)); return LR_ERR_CUDA; }
+    if (smem > 48 * 1024) {
+        static thread_local int vec_dev = -1, scalar_dev = -1;
+        const cudaError_t ce = vec ? opt_in_smem(pca_decode_kernel<BT>, 200 * 1024, vec_dev)
+                                   : opt_in_smem(pca_decode_scalar_kernel<BT>, 200 * 1024, scalar_dev);
+        if (int e = cuda_ok(ce, "pca_decode: cannot raise shared memory limit")) return e;
     }
-    int blocks_per_sm = (int)((220 * 1024) / (smem + 1024));
-    if (blocks_per_sm > 8) blocks_per_sm = 8;
-    if (blocks_per_sm < 1) blocks_per_sm = 1;
-    int64_t grid = (int64_t)148 * blocks_per_sm;
+    int per_sm = (int)((220 * 1024) / (smem + 1024));
+    if (per_sm > 8) per_sm = 8;
+    if (per_sm < 1) per_sm = 1;
+    int64_t grid = (int64_t)148 * per_sm;
     if (grid > g.n_tiles) grid = g.n_tiles;
     if (vec) pca_decode_kernel<BT><<<(unsigned)grid, PD_ROWS, smem, st>>>(coefs, basis, mean, out, g);
     else pca_decode_scalar_kernel<BT><<<(unsigned)grid, PD_ROWS, smem, st>>>(coefs, basis, mean, out, g);
@@ -517,11 +517,10 @@ static int launch_pca_bwd(const float *gout, const float *basis, float *gcoefs, 
     if (g.K % 4 == 0 && ((uintptr_t)basis & 15) == 0 && g.N % 4 == 0 && ((uintptr_t)gout & 15) == 0 && g.K <= PT_ROWS) {
         const size_t smem_t = sizeof(float) * (size_t)PT_STAGES * ((size_t)PT_ROWS * g.K + (size_t)BT * PT_ROWS);
         if (smem_t <= 110 * 1024) {
-            static thread_local bool attr_done = false;
-            if (smem_t > 48 * 1024 && !attr_done) {
-                cudaError_t e = cudaFuncSetAttribute(pca_decode_backward_tma_kernel<BT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
-                if (e != cudaSuccess) { set_error("pca_decode_backward: cannot raise shared memory limit: %s", cudaGetErrorString(e)); return LR_ERR_CUDA; }
-                attr_done = true;
+            if (smem_t > 48 * 1024) {
+                static thread_local int smem_dev = -1;
+                const cudaError_t ce = opt_in_smem(pca_decode_backward_tma_kernel<BT>, 110 * 1024, smem_dev);
+                if (int e = cuda_ok(ce, "pca_decode_backward: cannot raise shared memory limit")) return e;
             }
             const int64_t n_tiles = (g.N + PT_ROWS - 1) / PT_ROWS;
             int per_sm = (int)((224 * 1024) / (smem_t + 1024));
@@ -540,14 +539,15 @@ static int launch_pca_bwd(const float *gout, const float *basis, float *gcoefs, 
     const size_t smem = sizeof(float) * smem_f;
     if (smem > 200 * 1024) { set_error("pca_decode_backward: needs %zu bytes of shared memory", smem); return LR_ERR_BAD_ARGUMENT; }
     if (smem > 48 * 1024) {
-        cudaError_t e = vec ? cudaFuncSetAttribute(pca_decode_backward_kernel<BT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024)
-                            : cudaFuncSetAttribute(pca_decode_backward_kernel<BT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) { set_error("pca_decode_backward: cannot raise shared memory limit: %s", cudaGetErrorString(e)); return LR_ERR_CUDA; }
+        static thread_local int vec_dev = -1, scalar_dev = -1;
+        const cudaError_t ce = vec ? opt_in_smem(pca_decode_backward_kernel<BT, true>, 200 * 1024, vec_dev)
+                                   : opt_in_smem(pca_decode_backward_kernel<BT, false>, 200 * 1024, scalar_dev);
+        if (int e = cuda_ok(ce, "pca_decode_backward: cannot raise shared memory limit")) return e;
     }
-    int blocks_per_sm = (int)((220 * 1024) / (smem + 1024));
-    if (blocks_per_sm > 8) blocks_per_sm = 8;
-    if (blocks_per_sm < 1) blocks_per_sm = 1;
-    int64_t grid = (int64_t)148 * blocks_per_sm;
+    int per_sm = (int)((220 * 1024) / (smem + 1024));
+    if (per_sm > 8) per_sm = 8;
+    if (per_sm < 1) per_sm = 1;
+    int64_t grid = (int64_t)148 * per_sm;
     if (grid > g.n_tiles) grid = g.n_tiles;
     if (vec) pca_decode_backward_kernel<BT, true><<<(unsigned)grid, PD_ROWS, smem, st>>>(gout, basis, gcoefs, g);
     else pca_decode_backward_kernel<BT, false><<<(unsigned)grid, PD_ROWS, smem, st>>>(gout, basis, gcoefs, g);

@@ -330,9 +330,8 @@ extern "C" int lr_label_surface_counts(const float *pred, const float *target, i
     LR_REQUIRE(L >= 1 && L <= 128, "label_surface_counts: number of labels L=%d must be in [1, 128]", L);
     if (int e = surface_check("label_surface_counts", B, D, H, W)) return e;
     cudaStream_t st = as_stream(stream);
-    cudaError_t ce = cudaMemsetAsync(counts, 0, sizeof(int64_t) * (size_t)B * 2 * L, st);
-    if (ce == cudaSuccess) ce = cudaMemsetAsync(invalid, 0, sizeof(int64_t) * (size_t)B, st);
-    if (ce != cudaSuccess) { set_error("label_surface_counts: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    if (int e = cuda_ok(cudaMemsetAsync(counts, 0, sizeof(int64_t) * (size_t)B * 2 * L, st), "label_surface_counts: memset failed")) return e;
+    if (int e = cuda_ok(cudaMemsetAsync(invalid, 0, sizeof(int64_t) * (size_t)B, st), "label_surface_counts: memset failed")) return e;
     const int N = D * H * W;
     int64_t per_item = (N + SCOUNT_THREADS * 16 - 1) / (SCOUNT_THREADS * 16);      // >= 16 voxels per thread
     const int64_t cap = ((int64_t)sm_count() * 8 + B - 1) / B;
@@ -374,8 +373,8 @@ extern "C" int lr_surface_distances(const float *from, const float *to, int B, i
     ws += align_up(3 * sizeof(double) * (size_t)B * nbx);
     int *near = reinterpret_cast<int *>(ws), *S = reinterpret_cast<int *>(ws + vol), *T = reinterpret_cast<int *>(ws + 2 * vol);
     auto *packed = reinterpret_cast<unsigned *>(ws + 3 * vol);
-    cudaError_t ce = cudaMemsetAsync(fill, 0, (sizeof(unsigned long long) + sizeof(unsigned)) * (size_t)B, st);
-    if (ce != cudaSuccess) { set_error("surface_distances: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
+    if (int e = cuda_ok(cudaMemsetAsync(fill, 0, (sizeof(unsigned long long) + sizeof(unsigned)) * (size_t)B, st), "surface_distances: memset failed"))
+        return e;
     const float fl = (float)label;
     const int rows = B * D * H;
     sdist_row_kernel<<<(rows + SD_ROW_WARPS - 1) / SD_ROW_WARPS, SD_ROW_WARPS * 32, 0, st>>>(to, rows, D, H, W, fl, near);

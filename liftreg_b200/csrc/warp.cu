@@ -866,9 +866,7 @@ extern "C" int lr_warp_backward_slab(const float *grad_out, const float *img, co
         // gradient is a pure scatter, which the linear kernel cannot express -> not needed by the reference
         // (evaluate_dir_lab.py:221 warps label maps without autograd).
         LR_REQUIRE(!grad_img, "warp_backward: grad_img is not supported for nearest mode");
-        cudaError_t ce = cudaMemsetAsync(grad_phi, 0, sizeof(float) * 3 * (size_t)B * g.nvox_o, st);
-        if (ce != cudaSuccess) { set_error("warp_backward: memset failed: %s", cudaGetErrorString(ce)); return LR_ERR_CUDA; }
-        return LR_OK;
+        return cuda_ok(cudaMemsetAsync(grad_phi, 0, sizeof(float) * 3 * (size_t)B * g.nvox_o, st), "warp_backward: memset failed");
     }
     const bool sc = using_scale != 0, id = disp_plus_identity != 0;
     const int chunk = batch_chunk(g.Do);

@@ -24,6 +24,17 @@ def _ptr(t):
     return ctypes.c_void_p(t.data_ptr()) if t is not None else None
 
 
+def _call(name, device, *args):
+    """Call the C-ABI entry `name` on `device` with args and that device's current stream; RuntimeError if it fails."""
+    with torch.cuda.device(device):
+        _native.check(getattr(_native.lib(), name)(*args, _stream()), name)
+
+
+def _grad_scalar(grad_loss, device):
+    """The incoming gradient of a scalar loss as the one-element float32 tensor on `device` that the adjoints read."""
+    return grad_loss.to(device=device, dtype=torch.float32).reshape(1).contiguous()
+
+
 def _need_cuda_f32(t, name):
     if not isinstance(t, torch.Tensor):
         raise TypeError("%s must be a torch.Tensor, got %s" % (name, type(t).__name__))
@@ -88,10 +99,8 @@ class _DRR(torch.autograd.Function):
                 raise ValueError("out must be a contiguous CUDA float32 tensor of %d elements" % (B * P * rd * rh))
             proj = out
             ctx.mark_dirty(out)
-        with torch.cuda.device(vol.device):
-            _native.check(_native.lib().lr_drr_forward(_ptr(vol), B, d, w, h, _dp(poses), n_sets, P, rd, rh,
-                                                       _fp(spacing), y_norm_mode, out_scale, _ptr(proj), _stream()),
-                          "lr_drr_forward")
+        _call("lr_drr_forward", vol.device, _ptr(vol), B, d, w, h, _dp(poses), n_sets, P, rd, rh, _fp(spacing), y_norm_mode,
+              out_scale, _ptr(proj))
         ctx.geom = (poses, rd, rh, spacing, y_norm_mode, out_scale, (B, d, w, h))
         return proj
 
@@ -101,10 +110,8 @@ class _DRR(torch.autograd.Function):
         grad_proj = _need_cuda_f32(grad_proj, "grad_proj")
         n_sets, P, _ = poses.shape
         grad_vol = torch.zeros((B, d, w, h), device=grad_proj.device, dtype=torch.float32)
-        with torch.cuda.device(grad_proj.device):
-            _native.check(_native.lib().lr_drr_backward(_ptr(grad_proj), B, d, w, h, _dp(poses), n_sets, P, rd, rh,
-                                                        _fp(spacing), y_norm_mode, out_scale, _ptr(grad_vol), _stream()),
-                          "lr_drr_backward")
+        _call("lr_drr_backward", grad_proj.device, _ptr(grad_proj), B, d, w, h, _dp(poses), n_sets, P, rd, rh, _fp(spacing),
+              y_norm_mode, out_scale, _ptr(grad_vol))
         return grad_vol, None, None, None, None, None, None, None
 
 
@@ -129,7 +136,6 @@ def drr_project_peers(vol, poses, resolution, spacing, out_ptrs, view_stride, y_
     """Multi-GPU sweep form of drr_project (no autograd): the kernel stores the images into every buffer of `out_ptrs`
     (raw device addresses: this rank's gather buffer and the peers', see sharding.PeerGather), view k of the call at
     k * view_stride images from each address.  Nothing is returned; the caller orders the ranks with a barrier."""
-    import ctypes
     poses = _poses64(poses)
     vol = _need_cuda_f32(vol, "vol")
     if vol.dim() != 4 or poses.shape[0] not in (1, vol.shape[0]):
@@ -137,11 +143,9 @@ def drr_project_peers(vol, poses, resolution, spacing, out_ptrs, view_stride, y_
     B, d, w, h = vol.shape
     n_sets, P, _ = poses.shape
     ptrs = (ctypes.c_void_p * len(out_ptrs))(*[int(a) for a in out_ptrs])
-    with torch.cuda.device(vol.device):
-        _native.check(_native.lib().lr_drr_forward_peers(_ptr(vol), B, d, w, h, _dp(poses), n_sets, P, int(resolution[0]),
-                                                         int(resolution[1]), _fp(_spacing3(spacing)), int(y_norm_mode),
-                                                         float(out_scale), ptrs, len(out_ptrs), int(view_stride), _stream()),
-                      "lr_drr_forward_peers")
+    _call("lr_drr_forward_peers", vol.device, _ptr(vol), B, d, w, h, _dp(poses), n_sets, P, int(resolution[0]),
+          int(resolution[1]), _fp(_spacing3(spacing)), int(y_norm_mode), float(out_scale), ptrs, len(out_ptrs),
+          int(view_stride))
 
 
 def project_grid(poses, resolution, obj_shape, spacing, device, y_norm_mode=YNORM_WM1, flip=False, want_grid=True):
@@ -155,10 +159,8 @@ def project_grid(poses, resolution, obj_shape, spacing, device, y_norm_mode=YNOR
         raise RuntimeError("project_grid needs a CUDA device: liftreg_b200 has no CPU path")
     grid = torch.empty((P, rd, rh, w, 3), device=dev, dtype=torch.float32) if want_grid else None
     dx = torch.empty((P, rd, rh), device=dev, dtype=torch.float32)
-    with torch.cuda.device(dev):
-        _native.check(_native.lib().lr_project_grid(_dp(poses), P, rd, rh, d, w, h, _fp(_spacing3(spacing)),
-                                                    int(y_norm_mode), int(bool(flip)), _ptr(grid), _ptr(dx), _stream()),
-                      "lr_project_grid")
+    _call("lr_project_grid", dev, _dp(poses), P, rd, rh, d, w, h, _fp(_spacing3(spacing)), int(y_norm_mode), int(bool(flip)),
+          _ptr(grid), _ptr(dx))
     return grid, dx
 
 
@@ -181,11 +183,8 @@ class _Backproject(torch.autograd.Function):
                 raise ValueError("out must be (B,>=%d,%d,%d,%d), got %s" % (channel_offset + P, d, w, h, tuple(out.shape)))
             view, bs, cs = out[:, channel_offset:channel_offset + P], out.shape[1] * nv, nv
             ctx.mark_dirty(out)
-        with torch.cuda.device(proj.device):
-            _native.check(_native.lib().lr_backproject_forward_slab(_ptr(proj), _fp(poses), B, P, pw, ph, d_total, w, h,
-                                                                    i_begin, i_count, ctypes.c_void_p(view.data_ptr()),
-                                                                    bs, cs, _stream()),
-                          "lr_backproject_forward_slab")
+        _call("lr_backproject_forward_slab", proj.device, _ptr(proj), _fp(poses), B, P, pw, ph, d_total, w, h, i_begin, i_count,
+              ctypes.c_void_p(view.data_ptr()), bs, cs)
         ctx.geom = (poses, B, P, pw, ph, d, w, h, channel_offset, out.shape[1], d_total, i_begin)
         return out
 
@@ -199,10 +198,8 @@ class _Backproject(torch.autograd.Function):
         nv = d * w * h
         gview = grad_out[:, off:off + P]
         grad_proj = torch.zeros((B, P, pw, ph), device=grad_out.device, dtype=torch.float32)
-        with torch.cuda.device(grad_out.device):
-            _native.check(_native.lib().lr_backproject_backward(ctypes.c_void_p(gview.data_ptr()), nchan * nv, nv, _fp(poses),
-                                                                B, P, pw, ph, d, w, h, _ptr(grad_proj), _stream()),
-                          "lr_backproject_backward")
+        _call("lr_backproject_backward", grad_out.device, ctypes.c_void_p(gview.data_ptr()), nchan * nv, nv, _fp(poses), B, P,
+              pw, ph, d, w, h, _ptr(grad_proj))
         # `out` was overwritten in channels [off, off+P): the gradient wrt its previous content passes through elsewhere
         grad_buf = None
         if ctx.needs_input_grad[5]:
@@ -242,9 +239,7 @@ def backproj_grid(poses, img_shape, proj_shape, device):
     if dev.type != "cuda":
         raise RuntimeError("backproj_grid needs a CUDA device: liftreg_b200 has no CPU path")
     grid = torch.empty((poses.shape[0], 2, d, w, h), device=dev, dtype=torch.float32)
-    with torch.cuda.device(dev):
-        _native.check(_native.lib().lr_backproj_grid(_fp(poses), poses.shape[0], d, w, h, pw, ph, _ptr(grid), _stream()),
-                      "lr_backproj_grid")
+    _call("lr_backproj_grid", dev, _fp(poses), poses.shape[0], d, w, h, pw, ph, _ptr(grid))
     return grid
 
 
@@ -257,11 +252,8 @@ class _Warp(torch.autograd.Function):
         B, C, D, H, W = img.shape
         z_count = phi.shape[2]
         out = torch.empty((B, C, z_count, H, W), device=img.device, dtype=torch.float32)
-        with torch.cuda.device(img.device):
-            _native.check(_native.lib().lr_warp_forward_slab(_ptr(img), _ptr(phi), B, C, D, H, W, z_begin, z_count, padding,
-                                                             mode, int(using_scale), int(disp_plus_identity), _ptr(out),
-                                                             _stream()),
-                          "lr_warp_forward_slab")
+        _call("lr_warp_forward_slab", img.device, _ptr(img), _ptr(phi), B, C, D, H, W, z_begin, z_count, padding, mode,
+              int(using_scale), int(disp_plus_identity), _ptr(out))
         ctx.save_for_backward(img, phi)
         ctx.cfg = (padding, mode, using_scale, disp_plus_identity, z_begin)
         return out
@@ -278,11 +270,8 @@ class _Warp(torch.autograd.Function):
             raise NotImplementedError("gradient wrt the image is not implemented for nearest-mode warps")
         gimg = torch.zeros_like(img) if need_img else None
         gphi = torch.empty_like(phi) if need_phi else None
-        with torch.cuda.device(img.device):
-            _native.check(_native.lib().lr_warp_backward_slab(_ptr(grad_out), _ptr(img), _ptr(phi), B, C, D, H, W, z_begin,
-                                                              z_count, padding, mode, int(using_scale), int(ident),
-                                                              _ptr(gimg), _ptr(gphi), _stream()),
-                          "lr_warp_backward_slab")
+        _call("lr_warp_backward_slab", img.device, _ptr(grad_out), _ptr(img), _ptr(phi), B, C, D, H, W, z_begin, z_count,
+              padding, mode, int(using_scale), int(ident), _ptr(gimg), _ptr(gphi))
         return gimg, gphi, None, None, None, None, None
 
 
@@ -318,8 +307,7 @@ def identity_map(sz, device):
     if dev.type != "cuda":
         raise RuntimeError("identity_map needs a CUDA device: liftreg_b200 has no CPU path")
     out = torch.empty((3, D, H, W), device=dev, dtype=torch.float32)
-    with torch.cuda.device(dev):
-        _native.check(_native.lib().lr_identity_map(D, H, W, _ptr(out), _stream()), "lr_identity_map")
+    _call("lr_identity_map", dev, D, H, W, _ptr(out))
     return out
 
 
@@ -328,8 +316,7 @@ def atten_coef_(img):
     t = _need_cuda_f32(img, "img")
     if t.data_ptr() != img.data_ptr():
         raise ValueError("atten_coef_ needs a contiguous tensor")
-    with torch.cuda.device(t.device):
-        _native.check(_native.lib().lr_atten_coef(_ptr(t), t.numel(), _ptr(t), _stream()), "lr_atten_coef")
+    _call("lr_atten_coef", t.device, _ptr(t), t.numel(), _ptr(t))
     return img
 
 
@@ -343,9 +330,8 @@ class _PcaDecode(torch.autograd.Function):
         B, K = coefs.shape
         N = basis.shape[0]
         out = torch.empty((B, N), device=coefs.device, dtype=torch.float32)
-        with torch.cuda.device(coefs.device):
-            _native.check(_native.lib().lr_pca_decode(_ptr(coefs), _ptr(basis), _ptr(mean_c), B, K, N, int(add_identity),
-                                                      D, H, W, _ptr(out), _stream()), "lr_pca_decode")
+        _call("lr_pca_decode", coefs.device, _ptr(coefs), _ptr(basis), _ptr(mean_c), B, K, N, int(add_identity), D, H, W,
+              _ptr(out))
         ctx.save_for_backward(basis)
         return out
 
@@ -357,9 +343,7 @@ class _PcaDecode(torch.autograd.Function):
         B, N = grad_out.shape
         K = basis.shape[1]
         gcoefs = torch.zeros((B, K), device=grad_out.device, dtype=torch.float32)
-        with torch.cuda.device(grad_out.device):
-            _native.check(_native.lib().lr_pca_decode_backward(_ptr(grad_out), _ptr(basis), B, K, N, _ptr(gcoefs), _stream()),
-                          "lr_pca_decode_backward")
+        _call("lr_pca_decode_backward", grad_out.device, _ptr(grad_out), _ptr(basis), B, K, N, _ptr(gcoefs))
         return gcoefs, None, None, None, None, None, None
 
 
@@ -396,8 +380,7 @@ class _Ncc(torch.autograd.Function):
         B = x.shape[0]
         N = x.numel() // B
         sums = torch.empty((B, 7), device=x.device, dtype=torch.float64)
-        with torch.cuda.device(x.device):
-            _native.check(_native.lib().lr_ncc_sums(_ptr(x), _ptr(y), B, N, _ptr(sums), _stream()), "lr_ncc_sums")
+        _call("lr_ncc_sums", x.device, _ptr(x), _ptr(y), B, N, _ptr(sums))
         ncc = sums[:, 2] / torch.sqrt(sums[:, 3] * sums[:, 4])           # the 1/N of the three means cancels
         ctx.save_for_backward(x, y, sums)
         return (1.0 - ncc.mean()).to(torch.float32)
@@ -407,11 +390,9 @@ class _Ncc(torch.autograd.Function):
         x, y, sums = ctx.saved_tensors
         B = x.shape[0]
         N = x.numel() // B
-        g = grad_loss.to(device=x.device, dtype=torch.float32).reshape(1).contiguous()
+        g = _grad_scalar(grad_loss, x.device)
         gx = torch.empty_like(x)
-        with torch.cuda.device(x.device):
-            _native.check(_native.lib().lr_ncc_backward(_ptr(x), _ptr(y), B, N, _ptr(sums), _ptr(g), _ptr(gx), _stream()),
-                          "lr_ncc_backward")
+        _call("lr_ncc_backward", x.device, _ptr(x), _ptr(y), B, N, _ptr(sums), _ptr(g), _ptr(gx))
         return gx, None
 
 
@@ -424,24 +405,27 @@ def ncc_loss(input, target):
 
 
 # --------------------------------------------------------------------------- local NCC similarity (training term)
-def _volume(t, name):
-    """(B,1,D,H,W) or (B,D,H,W) CUDA float32 -> contiguous tensor and (B, D, H, W)"""
-    if not isinstance(t, torch.Tensor) or not (t.dim() == 4 or (t.dim() == 5 and t.shape[1] == 1)):
-        raise ValueError("%s must be (B,1,D,H,W) or (B,D,H,W), got %s"
-                         % (name, tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__))
-    t = _need_cuda_f32(t, name)
-    return t, (t.shape[0],) + tuple(t.shape[-3:])
+def _volume_shape(t, name, want=None):
+    """(B, D, H, W) of a (B,1,D,H,W) or (B,D,H,W) tensor t, which must equal `want` when given; ValueError otherwise.
+    Checks the shape only, so that callers raise every ValueError before their device and dtype checks."""
+    if isinstance(t, torch.Tensor) and (t.dim() == 4 or (t.dim() == 5 and t.shape[1] == 1)):
+        got = (t.shape[0],) + tuple(t.shape[-3:])
+        if want is None or got == want:
+            return got
+    else:
+        got = tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__
+    raise ValueError("%s must be (B,1,D,H,W) or (B,D,H,W)%s, got %s"
+                     % (name, "" if want is None else " with (B,D,H,W) = %s" % (want,), got))
 
 
 class _LocalNcc(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, y, window, eps):
-        x, (B, D, H, W) = _volume(x, "input")
-        y, _ = _volume(y, "target")
+        x = _need_cuda_f32(x, "input")
+        y = _need_cuda_f32(y, "target")
+        B, D, H, W = x.shape[0], *x.shape[-3:]
         sums = torch.empty(B, device=x.device, dtype=torch.float64)
-        with torch.cuda.device(x.device):
-            _native.check(_native.lib().lr_local_ncc_sum(_ptr(x), _ptr(y), B, D, H, W, window, eps, _ptr(sums), _stream()),
-                          "lr_local_ncc_sum")
+        _call("lr_local_ncc_sum", x.device, _ptr(x), _ptr(y), B, D, H, W, window, eps, _ptr(sums))
         ctx.save_for_backward(x, y)
         ctx.cfg = (window, eps)
         return (1.0 - sums.sum() / float(B * D * H * W)).to(torch.float32)
@@ -451,13 +435,11 @@ class _LocalNcc(torch.autograd.Function):
         x, y = ctx.saved_tensors
         window, eps = ctx.cfg
         B, D, H, W = x.shape[0], *x.shape[-3:]
-        g = grad_loss.to(device=x.device, dtype=torch.float32).reshape(1).contiguous()
+        g = _grad_scalar(grad_loss, x.device)
         gx = torch.empty_like(x)
-        lib = _native.lib()
-        ws = torch.empty(lib.lr_local_ncc_workspace_bytes(B, D, H, W, window), device=x.device, dtype=torch.uint8)
-        with torch.cuda.device(x.device):
-            _native.check(lib.lr_local_ncc_backward(_ptr(x), _ptr(y), B, D, H, W, window, eps, _ptr(g), _ptr(gx), _ptr(ws),
-                                                    ws.numel(), _stream()), "lr_local_ncc_backward")
+        ws = torch.empty(_native.lib().lr_local_ncc_workspace_bytes(B, D, H, W, window), device=x.device, dtype=torch.uint8)
+        _call("lr_local_ncc_backward", x.device, _ptr(x), _ptr(y), B, D, H, W, window, eps, _ptr(g), _ptr(gx), _ptr(ws),
+              ws.numel())
         return gx, None, None, None
 
 
@@ -469,11 +451,19 @@ def local_ncc_loss(input, target, window=9, eps=1e-5):
     has no such term, so parity is unpinned."""
     if input.shape != target.shape:
         raise ValueError("input %s and target %s must have the same shape" % (tuple(input.shape), tuple(target.shape)))
+    _volume_shape(input, "input")
     return _LocalNcc.apply(input, target, int(window), float(eps))
 
 
 # --------------------------------------------------------------------------- displacement regulariser (row f4)
 FD_BOUNDARY = {"linear": 0, "neumann_zero": 1}       # LR_FD_LINEAR / LR_FD_NEUMANN_ZERO (mermaid FD modes)
+
+
+def _fd_boundary(boundary):
+    """The C-ABI code of the face rule named `boundary`; ValueError for a name not in FD_BOUNDARY."""
+    if boundary not in FD_BOUNDARY:
+        raise ValueError("boundary must be one of %s, got %r" % (sorted(FD_BOUNDARY), boundary))
+    return FD_BOUNDARY[boundary]
 
 
 class _DiffusionReg(torch.autograd.Function):
@@ -482,9 +472,7 @@ class _DiffusionReg(torch.autograd.Function):
         disp = _need_cuda_f32(disp, "disp")
         B, _, D, H, W = disp.shape
         total = torch.empty(1, device=disp.device, dtype=torch.float64)
-        with torch.cuda.device(disp.device):
-            _native.check(_native.lib().lr_diffusion_reg_sum(_ptr(disp), B, D, H, W, boundary, _ptr(total), _stream()),
-                          "lr_diffusion_reg_sum")
+        _call("lr_diffusion_reg_sum", disp.device, _ptr(disp), B, D, H, W, boundary, _ptr(total))
         ctx.save_for_backward(disp)
         ctx.boundary = boundary
         return (total[0] / float(B * D * H * W)).to(torch.float32)
@@ -493,11 +481,9 @@ class _DiffusionReg(torch.autograd.Function):
     def backward(ctx, grad_loss):
         disp, = ctx.saved_tensors
         B, _, D, H, W = disp.shape
-        g = grad_loss.to(device=disp.device, dtype=torch.float32).reshape(1).contiguous()
+        g = _grad_scalar(grad_loss, disp.device)
         gd = torch.empty_like(disp)
-        with torch.cuda.device(disp.device):
-            _native.check(_native.lib().lr_diffusion_reg_backward(_ptr(disp), B, D, H, W, ctx.boundary, _ptr(g), _ptr(gd),
-                                                                  _stream()), "lr_diffusion_reg_backward")
+        _call("lr_diffusion_reg_backward", disp.device, _ptr(disp), B, D, H, W, ctx.boundary, _ptr(g), _ptr(gd))
         return gd, None
 
 
@@ -509,21 +495,18 @@ def diffusion_reg(disp, boundary="linear"):
     the missing neighbour is extrapolated linearly) or "neumann_zero" (zero difference on the faces)."""
     if disp.dim() != 5 or disp.shape[1] != 3:
         raise ValueError("disp must be (B,3,D,H,W), got %s" % (tuple(disp.shape),))
-    if boundary not in FD_BOUNDARY:
-        raise ValueError("boundary must be one of %s, got %r" % (sorted(FD_BOUNDARY), boundary))
-    return _DiffusionReg.apply(disp, FD_BOUNDARY[boundary])
+    return _DiffusionReg.apply(disp, _fd_boundary(boundary))
 
 
 # --------------------------------------------------------------------------- NGF similarity (training term)
 class _Ngf(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, y, eps, boundary):
-        x, (B, D, H, W) = _volume(x, "input")
-        y, _ = _volume(y, "target")
+        x = _need_cuda_f32(x, "input")
+        y = _need_cuda_f32(y, "target")
+        B, D, H, W = x.shape[0], *x.shape[-3:]
         sums = torch.empty(B, device=x.device, dtype=torch.float64)
-        with torch.cuda.device(x.device):
-            _native.check(_native.lib().lr_ngf_sum(_ptr(x), _ptr(y), B, D, H, W, boundary, eps, _ptr(sums), _stream()),
-                          "lr_ngf_sum")
+        _call("lr_ngf_sum", x.device, _ptr(x), _ptr(y), B, D, H, W, boundary, eps, _ptr(sums))
         ctx.save_for_backward(x, y)
         ctx.cfg = (eps, boundary)
         return (1.0 - sums.sum() / float(B * D * H * W)).to(torch.float32)
@@ -533,11 +516,9 @@ class _Ngf(torch.autograd.Function):
         x, y = ctx.saved_tensors
         eps, boundary = ctx.cfg
         B, D, H, W = x.shape[0], *x.shape[-3:]
-        g = grad_loss.to(device=x.device, dtype=torch.float32).reshape(1).contiguous()
+        g = _grad_scalar(grad_loss, x.device)
         gx = torch.empty_like(x)
-        with torch.cuda.device(x.device):
-            _native.check(_native.lib().lr_ngf_backward(_ptr(x), _ptr(y), B, D, H, W, boundary, eps, _ptr(g), _ptr(gx),
-                                                        _stream()), "lr_ngf_backward")
+        _call("lr_ngf_backward", x.device, _ptr(x), _ptr(y), B, D, H, W, boundary, eps, _ptr(g), _ptr(gx))
         return gx, None, None, None
 
 
@@ -549,10 +530,8 @@ def ngf_loss(input, target, eps=1.0, boundary="linear"):
     spatial axis >= 2; eps (finite, > 0) is in the units of g: intensity per unit of the [-1, 1] grid coordinate.
     Differentiable wrt `input` (the warped image); `target` is data.  A float32 scalar computed without a host
     synchronisation.  The reference's NGFLoss is not in its tree, so parity is unpinned."""
-    for t, name in ((input, "input"), (target, "target")):
-        if not isinstance(t, torch.Tensor) or not (t.dim() == 4 or (t.dim() == 5 and t.shape[1] == 1)):
-            raise ValueError("%s must be (B,1,D,H,W) or (B,D,H,W), got %s"
-                             % (name, tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__))
+    _volume_shape(input, "input")
+    _volume_shape(target, "target")
     if input.shape != target.shape:
         raise ValueError("input %s and target %s must have the same shape" % (tuple(input.shape), tuple(target.shape)))
     if min(input.shape[-3:]) < 2:
@@ -560,9 +539,7 @@ def ngf_loss(input, target, eps=1.0, boundary="linear"):
     eps = float(eps)
     if not (math.isfinite(eps) and eps >= 1e-77):
         raise ValueError("eps must be finite and > 0 (>= 1e-77), got %r" % eps)
-    if boundary not in FD_BOUNDARY:
-        raise ValueError("boundary must be one of %s, got %r" % (sorted(FD_BOUNDARY), boundary))
-    return _Ngf.apply(input, target, eps, FD_BOUNDARY[boundary])
+    return _Ngf.apply(input, target, eps, _fd_boundary(boundary))
 
 
 # --------------------------------------------------------------------------- mutual information similarity (training term)
@@ -586,8 +563,7 @@ class _Mi(torch.autograd.Function):
         y = _need_cuda_f32(y, "target")
         B, N = x.shape[0], x.numel() // x.shape[0]
         hist = torch.empty((B, nb, nb + 2), device=x.device, dtype=torch.float64)
-        with torch.cuda.device(x.device):
-            _native.check(_native.lib().lr_mi_hist(_ptr(x), _ptr(y), B, N, nb, lo, hi, _ptr(hist), _stream()), "lr_mi_hist")
+        _call("lr_mi_hist", x.device, _ptr(x), _ptr(y), B, N, nb, lo, hi, _ptr(hist))
         ctx.save_for_backward(x, y, hist)
         ctx.cfg = (nb, lo, hi)
         return _mi_loss_from_hist(hist, N).to(torch.float32)
@@ -597,11 +573,9 @@ class _Mi(torch.autograd.Function):
         x, y, hist = ctx.saved_tensors
         nb, lo, hi = ctx.cfg
         B, N = x.shape[0], x.numel() // x.shape[0]
-        g = grad_loss.to(device=x.device, dtype=torch.float32).reshape(1).contiguous()
+        g = _grad_scalar(grad_loss, x.device)
         gx = torch.empty_like(x)
-        with torch.cuda.device(x.device):
-            _native.check(_native.lib().lr_mi_backward(_ptr(x), _ptr(y), B, N, nb, lo, hi, _ptr(hist), _ptr(g), _ptr(gx),
-                                                       _stream()), "lr_mi_backward")
+        _call("lr_mi_backward", x.device, _ptr(x), _ptr(y), B, N, nb, lo, hi, _ptr(hist), _ptr(g), _ptr(gx))
         return gx, None, None, None, None
 
 
@@ -640,12 +614,10 @@ def mi_loss(input, target, num_bins=32, value_range=(-1.0, 1.0)):
 JACOBIAN_STATS = ("folding_count", "folding_abs_sum", "det_min", "det_max", "det_sum", "det_sum_sq", "nonfinite_count")
 
 
-def _need_map(phi, boundary):
+def _need_map(phi):
+    """ValueError unless phi is a (B,3,D,H,W) tensor (shape only: the device and dtype are checked after it)."""
     if not isinstance(phi, torch.Tensor) or phi.dim() != 5 or phi.shape[1] != 3:
         raise ValueError("phi must be a (B,3,D,H,W) tensor, got %s" % (tuple(phi.shape) if isinstance(phi, torch.Tensor) else type(phi).__name__,))
-    if boundary not in FD_BOUNDARY:
-        raise ValueError("boundary must be one of %s, got %r" % (sorted(FD_BOUNDARY), boundary))
-    return _need_cuda_f32(phi, "phi")
 
 
 def jacobian_det(phi, boundary="linear", margin=0, want_map=False):
@@ -655,13 +627,13 @@ def jacobian_det(phi, boundary="linear", margin=0, want_map=False):
     Returns (stats, det): stats is a (B,7) float64 CUDA tensor ordered as JACOBIAN_STATS, over the voxels at least
     `margin` from every face (sums and min / max over finite values only); det is the (B,D,H,W) float32 map when
     want_map, else None.  Parity with the reference's utils.py:20-55 is unpinned (include/liftreg_b200.h)."""
-    phi = _need_map(phi, boundary)
+    _need_map(phi)
+    code = _fd_boundary(boundary)
+    phi = _need_cuda_f32(phi, "phi")
     B, _, D, H, W = phi.shape
     stats = torch.empty((B, 7), device=phi.device, dtype=torch.float64)
     det = torch.empty((B, D, H, W), device=phi.device, dtype=torch.float32) if want_map else None
-    with torch.cuda.device(phi.device):
-        _native.check(_native.lib().lr_jacobian_det(_ptr(phi), B, D, H, W, FD_BOUNDARY[boundary], int(margin), _ptr(det),
-                                                    _ptr(stats), _stream()), "lr_jacobian_det")
+    _call("lr_jacobian_det", phi.device, _ptr(phi), B, D, H, W, code, int(margin), _ptr(det), _ptr(stats))
     return stats, det
 
 
@@ -669,12 +641,10 @@ def jacobian_det(phi, boundary="linear", margin=0, want_map=False):
 class _FoldPenalty(torch.autograd.Function):
     @staticmethod
     def forward(ctx, phi, boundary):
-        phi = _need_map(phi, boundary)
+        phi = _need_cuda_f32(phi, "phi")
         B, _, D, H, W = phi.shape
         stats = torch.empty((B, 7), device=phi.device, dtype=torch.float64)
-        with torch.cuda.device(phi.device):
-            _native.check(_native.lib().lr_jacobian_det(_ptr(phi), B, D, H, W, FD_BOUNDARY[boundary], 0, None, _ptr(stats),
-                                                        _stream()), "lr_jacobian_det")
+        _call("lr_jacobian_det", phi.device, _ptr(phi), B, D, H, W, boundary, 0, None, _ptr(stats))
         ctx.save_for_backward(phi)
         ctx.boundary = boundary
         return (stats[:, 1].sum() / float(B * D * H * W)).to(torch.float32)
@@ -683,11 +653,9 @@ class _FoldPenalty(torch.autograd.Function):
     def backward(ctx, grad_loss):
         phi, = ctx.saved_tensors
         B, _, D, H, W = phi.shape
-        g = grad_loss.to(device=phi.device, dtype=torch.float32).reshape(1).contiguous()
+        g = _grad_scalar(grad_loss, phi.device)
         gphi = torch.empty_like(phi)
-        with torch.cuda.device(phi.device):
-            _native.check(_native.lib().lr_jacobian_fold_backward(_ptr(phi), B, D, H, W, FD_BOUNDARY[ctx.boundary], _ptr(g),
-                                                                  _ptr(gphi), _stream()), "lr_jacobian_fold_backward")
+        _call("lr_jacobian_fold_backward", phi.device, _ptr(phi), B, D, H, W, ctx.boundary, _ptr(g), _ptr(gphi))
         return gphi, None
 
 
@@ -697,7 +665,8 @@ def fold_penalty(phi, boundary="linear"):
     device, computed without a host synchronisation; differentiable wrt phi (subgradient over the strict fold set
     det < 0).  The reference has no such term, so parity is unpinned (include/liftreg_b200.h,
     lr_jacobian_fold_backward)."""
-    return _FoldPenalty.apply(phi, boundary)
+    _need_map(phi)
+    return _FoldPenalty.apply(phi, _fd_boundary(boundary))
 
 
 def _label_map(t, name):
@@ -727,9 +696,7 @@ def label_confusion(pred, target, num_labels):
     N = pred.numel() // B if B else 0
     counts = torch.empty((B, L, L), device=pred.device, dtype=torch.int64)
     invalid = torch.empty((B,), device=pred.device, dtype=torch.int64)
-    with torch.cuda.device(pred.device):
-        _native.check(_native.lib().lr_label_confusion(_ptr(pred), _ptr(target), B, N, L, _ptr(counts), _ptr(invalid),
-                                                       _stream()), "lr_label_confusion")
+    _call("lr_label_confusion", pred.device, _ptr(pred), _ptr(target), B, N, L, _ptr(counts), _ptr(invalid))
     return counts, invalid
 
 
@@ -738,11 +705,8 @@ def _label_volumes(pred, target):
     out = []
     for t, name in ((pred, "pred"), (target, "target")):
         t = _label_map(t, name)
-        if t.dim() == 5 and t.shape[1] == 1:
-            t = t[:, 0]
-        if t.dim() != 4:
-            raise ValueError("%s must be (B,1,D,H,W) or (B,D,H,W), got %s" % (name, tuple(t.shape)))
-        out.append(t.contiguous())
+        _volume_shape(t, name)
+        out.append((t[:, 0] if t.dim() == 5 else t).contiguous())
     if out[0].shape != out[1].shape:
         raise ValueError("pred %s and target %s must have the same shape" % (tuple(pred.shape), tuple(target.shape)))
     if out[0].device != out[1].device:
@@ -762,9 +726,7 @@ def label_surface_counts(pred, target, num_labels):
     B, D, H, W = pred.shape
     counts = torch.empty((B, 2, L), device=pred.device, dtype=torch.int64)
     invalid = torch.empty((B,), device=pred.device, dtype=torch.int64)
-    with torch.cuda.device(pred.device):
-        _native.check(_native.lib().lr_label_surface_counts(_ptr(pred), _ptr(target), B, D, H, W, L, _ptr(counts),
-                                                            _ptr(invalid), _stream()), "lr_label_surface_counts")
+    _call("lr_label_surface_counts", pred.device, _ptr(pred), _ptr(target), B, D, H, W, L, _ptr(counts), _ptr(invalid))
     return counts, invalid
 
 
@@ -794,15 +756,13 @@ def surface_distances(from_map, to_map, label, spacing=(1.0, 1.0, 1.0), sizes=No
     seg_offset = torch.from_numpy(offsets).to(src.device)
     dist = torch.empty((max(int(offsets[-1]), 1),), device=src.device, dtype=torch.float64)
     stats = torch.empty((B, 3), device=src.device, dtype=torch.float64)
-    lib = _native.lib()
-    nbytes = lib.lr_surface_distance_workspace_bytes(B, D, H, W)
+    nbytes = _native.lib().lr_surface_distance_workspace_bytes(B, D, H, W)
     if nbytes == 0:
         raise ValueError("maps of shape %s are too large for lr_surface_distances (B*D*H*W < 2^31, B <= 65535, "
                          "H and W <= 65535)" % (tuple(src.shape),))
     ws = torch.empty((nbytes,), device=src.device, dtype=torch.uint8)
-    with torch.cuda.device(src.device):
-        _native.check(lib.lr_surface_distances(_ptr(src), _ptr(dst), B, D, H, W, label, sp[0], sp[1], sp[2], _ptr(seg_offset),
-                                               _ptr(dist), _ptr(stats), _ptr(ws), nbytes, _stream()), "lr_surface_distances")
+    _call("lr_surface_distances", src.device, _ptr(src), _ptr(dst), B, D, H, W, label, sp[0], sp[1], sp[2], _ptr(seg_offset),
+          _ptr(dist), _ptr(stats), _ptr(ws), nbytes)
     return dist[:int(offsets[-1])], seg_offset, stats
 
 
@@ -826,9 +786,7 @@ class _LabelDice(torch.autograd.Function):
         phi = _need_cuda_f32(phi, "phi")
         B, _, D, H, W = phi.shape
         sums = torch.empty((B, num_labels, 3), device=phi.device, dtype=torch.float64)
-        with torch.cuda.device(phi.device):
-            _native.check(_native.lib().lr_label_dice_sums(_ptr(phi), _ptr(src), _ptr(tgt), B, D, H, W, num_labels, _ptr(sums),
-                                                           _stream()), "lr_label_dice_sums")
+        _call("lr_label_dice_sums", phi.device, _ptr(phi), _ptr(src), _ptr(tgt), B, D, H, W, num_labels, _ptr(sums))
         ctx.save_for_backward(phi, src, tgt, sums)
         return _dice_loss_from_sums(sums).to(torch.float32)
 
@@ -836,12 +794,10 @@ class _LabelDice(torch.autograd.Function):
     def backward(ctx, grad_loss):
         phi, src, tgt, sums = ctx.saved_tensors
         B, _, D, H, W = phi.shape
-        g = grad_loss.to(device=phi.device, dtype=torch.float32).reshape(1).contiguous()
+        g = _grad_scalar(grad_loss, phi.device)
         gphi = torch.empty_like(phi)
-        with torch.cuda.device(phi.device):
-            _native.check(_native.lib().lr_label_dice_backward(_ptr(phi), _ptr(src), _ptr(tgt), B, D, H, W, sums.shape[1],
-                                                               _ptr(sums), _ptr(g), _ptr(gphi), _stream()),
-                          "lr_label_dice_backward")
+        _call("lr_label_dice_backward", phi.device, _ptr(phi), _ptr(src), _ptr(tgt), B, D, H, W, sums.shape[1], _ptr(sums),
+              _ptr(g), _ptr(gphi))
         return gphi, None, None, None
 
 
@@ -856,9 +812,7 @@ def label_dice_loss(phi, source_labels, target_labels, num_labels):
     [0, num_labels) counts as no label.  2 <= num_labels <= 128.  A float32 scalar on phi's device, computed without a
     host synchronisation; differentiable wrt phi (the labels are data).  The reference has no such term, so parity is
     unpinned."""
-    if not isinstance(phi, torch.Tensor) or phi.dim() != 5 or phi.shape[1] != 3:
-        raise ValueError("phi must be a (B,3,D,H,W) tensor, got %s"
-                         % (tuple(phi.shape) if isinstance(phi, torch.Tensor) else type(phi).__name__,))
+    _need_map(phi)
     L = int(num_labels)
     if not 2 <= L <= 128:
         raise ValueError("num_labels must be in [2, 128], got %d" % L)
@@ -866,11 +820,8 @@ def label_dice_loss(phi, source_labels, target_labels, num_labels):
     maps = []
     for t, name in ((source_labels, "source_labels"), (target_labels, "target_labels")):
         t = _label_map(t, name)
-        if t.dim() == 5 and t.shape[1] == 1:
-            t = t[:, 0]
-        if tuple(t.shape) != want:
-            raise ValueError("%s must be (B,1,D,H,W) or (B,D,H,W) with (B,D,H,W) = %s, got %s" % (name, want, tuple(t.shape)))
+        _volume_shape(t, name, want)
         if t.device != phi.device:
             raise ValueError("%s must be on phi's device %s (got %s)" % (name, phi.device, t.device))
-        maps.append(t.contiguous())
+        maps.append((t[:, 0] if t.dim() == 5 else t).contiguous())
     return _LabelDice.apply(phi, maps[0], maps[1], L)

@@ -154,3 +154,29 @@ def test_fold_backward_rejects_bad_arguments_before_any_cuda_call(lib):
     for args, msg in cases:
         assert lib.lr_jacobian_fold_backward(*args) == -1, args
         assert msg in lib.lr_last_error(), (args, lib.lr_last_error())
+
+
+def test_diffusion_reg_rejects_bad_arguments_before_any_cuda_call(lib):
+    fake = ctypes.c_void_p(256)          # never dereferenced: every call below fails validation first
+    g = ctypes.c_void_p(512)
+    out = ctypes.c_void_p(1024)
+    cases = [
+        (lib.lr_diffusion_reg_sum, (None, 1, 4, 4, 4, 0, out, None), b"null"),
+        (lib.lr_diffusion_reg_sum, (fake, 1, 4, 4, 4, 0, None, None), b"null"),
+        (lib.lr_diffusion_reg_backward, (None, 1, 4, 4, 4, 0, g, out, None), b"null"),
+        (lib.lr_diffusion_reg_backward, (fake, 1, 4, 4, 4, 0, None, out, None), b"null"),
+        (lib.lr_diffusion_reg_backward, (fake, 1, 4, 4, 4, 0, g, None, None), b"null"),
+    ]
+    # (B, D, H, W, boundary): the rules both entries share
+    for dims, msg in [((0, 4, 4, 4, 0), b">= 2"),
+                      ((1, 1, 4, 4, 0), b">= 2"),
+                      ((1, 4, 4, 1, 1), b">= 2"),
+                      ((1, 4, 4, 4, 2), b"boundary"),
+                      ((1, 4, 4, 4, -1), b"boundary"),
+                      ((1, 1024, 1024, 1024, 0), b"2^31"),
+                      ((3, 512, 512, 1024, 1), b"2^31")]:
+        cases.append((lib.lr_diffusion_reg_sum, (fake, *dims, out, None), msg))
+        cases.append((lib.lr_diffusion_reg_backward, (fake, *dims, g, out, None), msg))
+    for fn, args, msg in cases:
+        assert fn(*args) == -1, (fn.__name__, args)
+        assert msg in lib.lr_last_error(), (fn.__name__, args, lib.lr_last_error())

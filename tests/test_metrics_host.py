@@ -112,6 +112,7 @@ def test_validation_metric_entries_reject_bad_arguments_before_any_cuda_call(lib
         (lib.lr_jacobian_det, (fake, 1, 4, 9, 9, 0, 2, None, stats, None), b"margin"),
         (lib.lr_jacobian_det, (fake, 1, 9, 9, 9, 0, -1, None, stats, None), b"margin"),
         (lib.lr_jacobian_det, (fake, 1, 1024, 1024, 1024, 0, 0, None, stats, None), b"2^31"),
+        (lib.lr_jacobian_det, (fake, 1, 1024, 1024, 1024, 0, 600, None, stats, None), b"margin"),   # margin first
         (lib.lr_label_confusion, (None, fake, 1, 10, 2, stats, stats, None), b"null"),
         (lib.lr_label_confusion, (fake, fake, 1, 10, 2, None, stats, None), b"null"),
         (lib.lr_label_confusion, (fake, fake, 1, 10, 0, stats, stats, None), b"[1, 128]"),
